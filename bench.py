@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: env-steps/s of the fused LMaze step at 1M envs per B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch: the fused kernel (action
 decode, wall lookup, move, reward, done, auto-reset, full f32 observation render,
@@ -42,6 +42,10 @@ V0_STEP_BYTES = V0_OBS_BYTES + 1 + 4 + 4 + 4 + 1
 V3_OBS_BYTES = 3 * 72 * 72 * 4
 V3_STEP_BYTES = V3_OBS_BYTES + 1 + 4 + 4 + 4 + 1
 FALLBACK_HBM_GBS = 6650.0      # B200_PROFILING.md fallback when MEASURED_PEAKS.json is absent
+# --dump-outputs keeps at most 256 observation rows (v0: 28.9 MB) and 2^20 values of each per-env output, which holds
+# every variant's dump under 64 MB
+DUMP_OBS_ROWS = 256
+DUMP_ENV_VALUES = 1 << 20
 
 
 def parse_args():
@@ -63,7 +67,15 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the rollout / obs-to-host side measurements")
     ap.add_argument("--cpu-budget", type=float, default=12.0, help="seconds of CPU-oracle timing")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned to its caller as DIR/<name>.npy (float32; per-env "
+                         "values of up to %d envs and %d observation rows, larger batches as a fixed seeded sample "
+                         "whose env indices are written beside them), so that two builds can be compared output for "
+                         "output"
+                         % (DUMP_ENV_VALUES, DUMP_OBS_ROWS))
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records the GPU path (--impl ours)")
     if args.warmup is None:
         args.warmup = 1000 if (args.impl == "ours" and args.variant in ("v2", "v4", "v5")) else 5
     return args
@@ -146,31 +158,44 @@ def recorded_traffic(variant, render_mode, n_envs):
 
 
 # --------------------------------------------------------------------------- CPU legs (oracle = checker / baseline only)
-def cpu_oracle_throughput_v5(n_envs, threads, budget_s, min_steps=2):
+def cpu_oracle_throughput_v5(n_envs, threads, budget_s, min_steps=2, warmup=0):
     """lmaze-v5: plannerStep (where the local episode ended) + step + reset on globalDone, both observations
-    rendered, on `threads` host threads (one OracleHier slice per thread; ctypes releases the GIL)."""
+    rendered, on `threads` host threads (one OracleHier slice per thread; ctypes releases the GIL).  The clock
+    starts once every thread has built its slice and run `warmup` untimed steps."""
     import numpy as np
     from oracle import oracle as O
     per = max(1, n_envs // threads)
     counts = [0] * threads
+    ready = threading.Barrier(threads + 1)
 
     def worker(k):
         rng = np.random.RandomState(k)
-        o = O.OracleHier(per, seed=1, env_id0=k * per)
-        o.reset(want_obs=False)
-        mask = np.ones(per, np.uint8)
-        t0 = time.perf_counter()
-        while counts[k] < min_steps or time.perf_counter() - t0 < budget_s:
+
+        def step(mask):
             o.planner_step(rng.randint(0, 25, size=per), mask=mask)
             _, _, _, _, gd, ld, _ = o.step(rng.randint(0, 4, size=per))
             if gd.any():
                 o.reset(mask=gd, want_obs=False)
-            mask = (gd | ld).astype(np.uint8)
+            return (gd | ld).astype(np.uint8)
+        try:
+            o = O.OracleHier(per, seed=1, env_id0=k * per)
+            o.reset(want_obs=False)
+            mask = np.ones(per, np.uint8)
+            for _ in range(warmup):
+                mask = step(mask)
+        except BaseException:
+            ready.abort()          # the main thread's wait raises instead of waiting for this thread forever
+            raise
+        ready.wait()
+        t0 = time.perf_counter()
+        while counts[k] < min_steps or time.perf_counter() - t0 < budget_s:
+            mask = step(mask)
             counts[k] += 1
     ths = [threading.Thread(target=worker, args=(k,)) for k in range(threads)]
-    t0 = time.perf_counter()
     for t in ths:
         t.start()
+    ready.wait()
+    t0 = time.perf_counter()
     for t in ths:
         t.join()
     dt = time.perf_counter() - t0
@@ -234,9 +259,10 @@ def run_reference(args):
     threads = os.cpu_count() or 1
     sample_envs = 32768
     if args.variant == "v5":
-        value, k, dt = cpu_oracle_throughput_v5(sample_envs, threads, 0.0, min_steps=args.warmup + args.steps)
+        value, k, dt = cpu_oracle_throughput_v5(sample_envs, threads, 0.0, min_steps=args.steps, warmup=args.warmup)
         sample = ("%d-env slice of the %d-env workload per step (plannerStep where due + step + both f32 obs renders), "
-                  "C oracle port, %d threads; %d steps incl. warm-up" % (sample_envs, args.envs, threads, k))
+                  "C oracle port, %d threads; %d timed steps after %d warm-up steps"
+                  % (sample_envs, args.envs, threads, k, args.warmup))
         print(json.dumps({
             "impl": "reference", "metric": "env_steps_per_sec", "value": value, "unit": "env-steps/s",
             "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup, "ms_per_step": dt / max(1, k) * 1e3,
@@ -442,6 +468,13 @@ def run_ours(args):
     gpu_launches = env.launch_count - launches0
     per_step = sorted(evs[i].elapsed_time(evs[i + 1]) / max(1, len(windows)) for i in range(args.steps))
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        # step() hands its caller the env's own output buffers: read them before anything steps the env again
+        outputs = {"obs": env.obs, "reward": env.reward, "done": env.done}
+        if hier:
+            outputs.update(local_obs=env.loc_obs, local_reward=env.local_reward, local_done=env.local_done,
+                           foveal_goal=env.foveal_goal)
+        dump_outputs(args.dump_outputs, outputs, windows[-1], "_rank%d" % rank if world > 1 else "")
     value = world * N * args.steps / (total_ms * 1e-3)
     step_ms = total_ms / args.steps
     launches_per_step = max(1, gpu_launches // args.steps)
@@ -594,6 +627,28 @@ def run_ours(args):
 
 
 VISIT_HIST_BYTES = 64          # one env's visit history (v4 / v5): the window centre of each averaging since the reset
+
+
+def dump_outputs(out_dir, outputs, obs_env0, suffix=""):
+    """--dump-outputs: every output as out_dir/<name><suffix>.npy in float32.  Per-env values are kept for up to
+    DUMP_ENV_VALUES envs and observation rows (tensors of more than one dimension) for DUMP_OBS_ROWS envs; a larger
+    batch is sampled at indices drawn from a fixed seed, so the same arguments always keep the same envs.  The kept
+    env indices (within this rank's batch) are written as env_index / obs_env_index (float64); obs_env0 is the env
+    of the observation tensor's first row (the last render window's start)."""
+    import numpy as np
+    import torch
+
+    def keep(n, k):
+        return np.arange(n) if n <= k else np.sort(np.random.RandomState(0).choice(n, k, replace=False))
+    env_rows = keep(outputs["reward"].shape[0], DUMP_ENV_VALUES)
+    obs_rows = keep(outputs["obs"].shape[0], DUMP_OBS_ROWS)
+    arrays = {"env_index": env_rows.astype(np.float64), "obs_env_index": (obs_env0 + obs_rows).astype(np.float64)}
+    for name, t in outputs.items():
+        rows = torch.from_numpy(obs_rows if t.dim() > 1 else env_rows).to(t.device)
+        arrays[name] = t[rows].to(torch.float32).cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), a)
 
 
 def main_workload_checks(rk, lmz, env, args, hier, seed, N, W, R, action_ring, steps_done, K=1024, KO=32):

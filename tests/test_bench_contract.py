@@ -32,6 +32,37 @@ def test_reference_arm_other_ranks_stay_silent():
     assert res.returncode == 0 and res.stdout.strip() == ""
 
 
+@pytest.mark.gpu
+@pytest.mark.parametrize("variant", ["v0", "v5"])
+def test_dump_outputs_repeat_exactly(variant, tmp_path):
+    """--dump-outputs writes the last timed step's outputs; two runs with the same arguments write the same bits, and
+    --steps is the number of timed steps."""
+    import numpy as np
+    names = ["obs", "reward", "done", "env_index", "obs_env_index"]
+    if variant == "v5":
+        names += ["local_obs", "local_reward", "local_done", "foveal_goal"]
+    runs = []
+    for k in range(2):
+        out = tmp_path / ("run%d" % k)
+        res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--variant", variant, "--envs", "3000",
+                              "--steps", "4", "--warmup", "3", "--no-extras", "--no-cpu-baseline", "--dump-outputs", str(out)],
+                             stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=600)
+        assert res.returncode == 0, res.stderr[-2000:]
+        d = json.loads(res.stdout)
+        assert d["steps"] == 4 and d["warmup"] == 3
+        if variant == "v0":
+            assert d["gpu_launches"] == 4                       # one fused launch per timed step
+        assert sorted(p.name for p in out.iterdir()) == sorted(n + ".npy" for n in names)
+        runs.append({n: np.load(str(out / (n + ".npy"))) for n in names})
+    a, b = runs
+    assert sum(x.nbytes for x in a.values()) <= 64 << 20
+    assert a["reward"].shape == (3000,) and a["obs"].shape[0] == 256 and a["obs_env_index"].shape == (256,)
+    for n in names:
+        assert a[n].dtype in (np.float32, np.float64)
+        assert np.array_equal(a[n].view(np.uint8), b[n].view(np.uint8)), n
+    assert set(np.unique(a["reward"].view(np.uint32)).tolist()) <= {0x80000000, 0xBF800000, 0xBC23D70A, 0x42C80000}
+
+
 def test_default_warmup_puts_the_foveal_variants_in_steady_state(monkeypatch):
     """bench.py's own arm warms v2 / v4 / v5 for 1,000 steps unless told otherwise (their episodes start together and need
     that long to de-synchronise, DESIGN.md 3.5); everything else, and the CPU arm, keeps the short default."""
