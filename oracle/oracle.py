@@ -169,13 +169,17 @@ class OracleVec(object):
     drive both with the same calls.
     """
 
-    def __init__(self, variant, n, seed=0, env_id0=0, autoreset=True, threads=1, random_ball=True, random_goal=True):
+    def __init__(self, variant, n, seed=0, env_id0=0, autoreset=True, threads=1, random_ball=True, random_goal=True,
+                 lazy_init=False):
+        """lazy_init: leave the envs zeroed for the first reset() to initialise (on all threads): for large batches,
+        whose env-by-env initialisation from Python takes seconds.  Call reset() before anything else then."""
         self.L = lib()
         self.variant, self.n, self.seed, self.env_id0 = variant, int(n), int(seed), int(env_id0)
         self.autoreset, self.threads = bool(autoreset), int(threads)
         self.env_bytes = self.L.lmzo_sizeof_env()
         self._mem = np.zeros(self.n * self.env_bytes, dtype=np.uint8)  # zero => lazily lmzo_init'ed
-        for i in range(self.n):
+        assert not lazy_init or (random_ball and random_goal)
+        for i in range(0 if lazy_init else self.n):
             self.L.lmzo_init(self._env(i), variant)
             if not (random_ball and random_goal):
                 self.L.lmzo_env_set_flags(self._env(i), int(random_ball), int(random_goal))
@@ -231,6 +235,13 @@ class OracleVec(object):
         rc = self.L.lmzo_env_force_v2(self._env(i), layout, sx, sy, gx, gy, px, py, step_count)
         if rc != 0:
             raise ValueError("oracle rejected forced v2 state")
+
+    def reset_masked(self, mask):
+        """Device-RNG reset of the envs where mask is true (lmz_reset with a mask and no spawn cells)."""
+        for i in np.nonzero(np.asarray(mask))[0]:
+            i = int(i)
+            self.L.lmzo_vec_reset(self._env(i), 1, self.variant, None, self.seed, self.env_id0 + i,
+                                  self.episode.ctypes.data + 4 * i, None, 1)
 
     def export_visit(self):
         """v4 visit layer state[2] of every env, float32 [N, 18, 18]."""

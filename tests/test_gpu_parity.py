@@ -9,6 +9,8 @@ import numpy as np
 import pytest
 import torch
 
+from philox_np import _rng_actions
+
 pytestmark = pytest.mark.gpu
 
 INVALID = 7
@@ -891,23 +893,3 @@ def test_soak_rollout_65k_envs_1000_steps(lmz, oracle_mod, variant):
     assert [s[k] for k in oracle_mod.STAT_NAMES] == ora.stats.tolist() and s["steps"] == N * T * calls
     env.close()
 
-
-def _philox_np(c0, c1, c2, c3, k0, k1):
-    """numpy Philox-4x32-10 over arrays of counters (same spec as DESIGN.md section 4)."""
-    M0, M1 = np.uint64(0xD2511F53), np.uint64(0xCD9E8D57)
-    c0, c1, c2, c3 = (np.asarray(x, dtype=np.uint64) for x in (c0, c1, c2, c3))
-    k0, k1 = np.uint64(k0), np.uint64(k1)
-    mask = np.uint64(0xFFFFFFFF)
-    for _ in range(10):
-        p0, p1 = M0 * c0, M1 * c2
-        hi0, lo0, hi1, lo1 = p0 >> np.uint64(32), p0 & mask, p1 >> np.uint64(32), p1 & mask
-        c0, c1, c2, c3 = (hi1 ^ c1 ^ k0) & mask, lo1, (hi0 ^ c3 ^ k1) & mask, lo0
-        k0, k1 = (k0 + np.uint64(0x9E3779B9)) & mask, (k1 + np.uint64(0xBB67AE85)) & mask
-    return c0, c1, c2, c3
-
-
-def _rng_actions(seed, ids, t):
-    blk, slot = t >> 6, t & 63
-    w = _philox_np(ids & np.uint64(0xFFFFFFFF), ids >> np.uint64(32), np.full(len(ids), blk & 0xFFFFFFFF, np.uint64),
-                   np.full(len(ids), ((blk >> 32) << 8) | 0x41, np.uint64), seed & 0xFFFFFFFF, seed >> 32)
-    return ((w[slot >> 4] >> np.uint64(2 * (slot & 15))) & np.uint64(3)).astype(np.int64)
