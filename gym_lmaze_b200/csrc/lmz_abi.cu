@@ -69,12 +69,6 @@ void v2_cells(int layout, char *cells) {     // layout 1..5 -> 324 letters
   for (int x = 0; x < 10; ++x) memcpy(cells + (x + 4) * 18 + 4, V2_ACTIVE[layout - 1] + 10 * x, 10);
 }
 
-const char *cells_of(int variant) {
-  if (variant == LMZ_V0) return V0_CELLS;
-  if (variant == LMZ_V3) return V3_CELLS;
-  return nullptr;
-}
-
 int cls_of(char c) {
   switch (c) {
     case 'W': return lmz::CLS_W;
@@ -155,8 +149,9 @@ void build_f4_lut(uint32_t *lut, uint32_t floats_per_env, uint32_t n_entries, Sl
 }
 
 template <class V>
-void build_blob_fov(std::vector<unsigned char> &blob) {
+void build_blob_fov(const char *, std::vector<unsigned char> &blob, int &, int &s_cell, int &x_cell) {
   blob.assign(V::BLOB_BYTES, 0);
+  s_cell = 4 * 18 + 4; x_cell = 8 * 18 + 8;        // maze 1's 'S' and 'X'; spawn candidates are per maze in the blob
   // the obs channels ARE the first C value planes (v2: free, goal, action, prev free, prev goal; v4/v5:
   // crop(free, goal, visit), action / fovealGoal, retStatelast(free, goal, visit)); a group of 4 envs = OBS_FLOATS float4s
   build_f4_lut<V>(reinterpret_cast<uint32_t *>(blob.data() + V::LUT_OFF), V::OBS_FLOATS, V::OBS_FLOATS,
@@ -188,22 +183,60 @@ void build_blob_fov(std::vector<unsigned char> &blob) {
 }
 
 // v5/v6: v4's foveal tables + the local observation's LUT (lmaze_env_v5.py:356-380) + each maze's 'X' cell
-void build_blob_v5(std::vector<unsigned char> &blob) {
+void build_blob_v5(const char *cells, std::vector<unsigned char> &blob, int &n_cand, int &s_cell, int &x_cell) {
   using V = lmz::V5;
-  build_blob_fov<V>(blob);
+  build_blob_fov<V>(cells, blob, n_cand, s_cell, x_cell);
   // local obs channels (lmaze_env_v5.py:360-368): free crop (value plane 9), ball rel. fovea_x1 (7), previous ball (8),
   // fovealGoal (10) -- the local copies are all zero on an IndexError row; one env row = 1,225 float4s exactly
   build_f4_lut<V>(reinterpret_cast<uint32_t *>(blob.data() + V::LOCLUT_OFF), V::LOC_FLOATS, V::LOC_FLOATS / 4,
                   [](int c) { static const int plane[4] = {9, 7, 8, 10}; return plane[c]; });
 }
 
+// ------------------------------------------------------------------ variants
+// What the host needs to know of each built variant.  Byte counts are per env.
+struct VariantInfo {
+  int32_t id;
+  int G, C, S, CL;               // maze side, obs channels, obs side, local obs channels (0: no local observation)
+  uint32_t obs_bytes;            // full f32 observation
+  uint32_t compact_bytes;        // compact observation: u8 [C][G][G], or f32 [C][5][5] for the foveal variants
+  uint32_t bits_bytes;           // bit-packed observation (0: not built)
+  int num_actions, num_layouts, state_cols;
+  bool foveal;                   // the observation is a crop around the ball (v2, v4, v5)
+  bool hier;                     // planner / actor levels and the local observation (v5)
+  bool has_visit;                // float visit layer (v4, v5)
+  const char *cells;             // the one maze of the full-view variants (null: five mazes, v2_cells)
+  void (*build_blob)(const char *cells, std::vector<unsigned char> &blob, int &n_cand, int &s_cell, int &x_cell);
+};
+
+// actions: lmaze_env.py:16, lmaze_env_v3.py:92; v2 lmaze_env_v2.py:39 (commented out in v4, :43-44); v5's step()
+// moves by one cell (lmaze_env_v5.py:205-217), plannerStep takes 25.  Layouts: lmaze_env_v2.py:306, lmaze_env_v4.py:351.
+const VariantInfo VARIANTS[] = {
+    {LMZ_V0, lmz::V0::G, lmz::V0::C, lmz::V0::S, 0, lmz::V0::OBS_BYTES, lmz::V0::COMPACT_BYTES,
+     lmz::V0::BITS_WORDS * 4, 4, 1, LMZ_ST_COLS, false, false, false, V0_CELLS, build_blob<lmz::V0>},
+    {LMZ_V2, lmz::V2::G, lmz::V2::C, lmz::V2::S, 0, lmz::V2::OBS_BYTES, lmz::V2::C * 25 * 4,
+     0, 25, 5, LMZ_ST_COLS, true, false, false, nullptr, build_blob_fov<lmz::V2>},
+    {LMZ_V3, lmz::V3::G, lmz::V3::C, lmz::V3::S, 0, lmz::V3::OBS_BYTES, lmz::V3::COMPACT_BYTES,
+     lmz::V3::BITS_WORDS * 4, 4, 1, LMZ_ST_COLS, false, false, false, V3_CELLS, build_blob<lmz::V3>},
+    {LMZ_V4, lmz::V4::G, lmz::V4::C, lmz::V4::S, 0, lmz::V4::OBS_BYTES, lmz::V4::C * 25 * 4,
+     0, 25, 5, LMZ_ST_COLS, true, false, true, nullptr, build_blob_fov<lmz::V4>},
+    {LMZ_V5, lmz::V5::G, lmz::V5::C, lmz::V5::S, lmz::V5::CL, lmz::V5::OBS_BYTES, lmz::V5::C * 25 * 4,   // CL: lmaze_env_v5.py:357-358
+     0, 4, 5, LMZ_ST_COLS_HIER, true, true, true, nullptr, build_blob_v5},
+};
+
+const VariantInfo *variant_info(int32_t variant) {   // null for a variant that is not built
+  for (const VariantInfo &v : VARIANTS)
+    if (v.id == variant) return &v;
+  return nullptr;
+}
+
+int unknown_variant(int32_t variant) { return fail(LMZ_ERR_UNSUPPORTED, "unknown variant %d", variant); }
+
 }  // namespace
 
 // ------------------------------------------------------------------ handle
 struct lmz_env {
   lmz_config cfg;
-  int G, C, S;
-  size_t obs_bytes_per_env;
+  const VariantInfo *var;        // cfg.variant's entry of VARIANTS
   int num_sms;
   // device memory owned by the handle
   uint32_t *state, *goal_count, *episode;
@@ -223,7 +256,6 @@ struct lmz_env {
   uint8_t *done;
   bool bound;
   int64_t win_lo, win_n;         // obs rows hold envs [win_lo, win_lo + win_n)
-  size_t compact_bytes_per_env;
   bool obs_synced;               // incremental render: obs currently holds a full render of the window
   int n_cand, s_cell, x_cell;
   uint64_t rollout_t;            // rollout steps taken so far (keys the action RNG)
@@ -280,9 +312,48 @@ lmz::KParams base_params(lmz_env *h) {
 
 // bytes of one env's row in the bound obs tensor
 size_t obs_row_bytes(const lmz_env *h) {
-  if (h->cfg.obs_mode == LMZ_OBS_COMPACT) return h->compact_bytes_per_env;
-  if (h->cfg.obs_mode == LMZ_OBS_BITS) return h->cfg.variant == LMZ_V0 ? lmz::V0::BITS_WORDS * 4 : lmz::V3::BITS_WORDS * 4;
-  return h->obs_bytes_per_env;
+  if (h->cfg.obs_mode == LMZ_OBS_COMPACT) return h->var->compact_bytes;
+  if (h->cfg.obs_mode == LMZ_OBS_BITS) return h->var->bits_bytes;
+  return h->var->obs_bytes;
+}
+
+// Resident CTAs per SM of KERN with `threads` threads and `smem` bytes of dynamic shared memory (>= 1), or an LMZ_ERR
+// code.  Queried once per device and thread; `raise_smem` first lifts the kernel's dynamic shared memory limit to `smem`.
+template <auto KERN>
+int resident_ctas(lmz_env *h, int threads, int smem, bool raise_smem, const char *what) {
+  static thread_local int configured_dev = -1;
+  static thread_local int ctas_per_sm = 1;
+  if (configured_dev != h->cfg.device) {
+    if (raise_smem) LMZ_CUDA(cudaFuncSetAttribute(KERN, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    LMZ_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas_per_sm, KERN, threads, smem));
+    if (ctas_per_sm < 1) return fail(LMZ_ERR_CUDA, "%s does not fit on an SM", what);
+    configured_dev = h->cfg.device;
+  }
+  return ctas_per_sm;
+}
+
+// CTAs per SM of a persistent launch: the tune[2] cap when set, else `dflt`; never more than `fit`
+int ctas_per_sm(const lmz_env *h, int dflt, int fit) {
+  const int per_sm = h->cfg.tune[2] > 0 ? h->cfg.tune[2] : dflt;
+  return per_sm < fit ? per_sm : fit;
+}
+
+// `per_sm` CTAs on every SM, but no more CTAs than `work` units
+int64_t persistent_grid(const lmz_env *h, int per_sm, int64_t work) {
+  const int64_t grid = (int64_t)h->num_sms * per_sm;
+  return grid < work ? grid : work;
+}
+
+int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
+
+// Every kernel launch of the handle: at least one CTA, the launch error checked, the launch counted.
+template <class Kern, class... Args>
+int launch(lmz_env *h, Kern kern, int64_t grid, int threads, int smem, cudaStream_t s, Args... args) {
+  if (grid < 1) grid = 1;
+  kern<<<(unsigned)grid, threads, smem, s>>>(args...);
+  LMZ_CUDA(cudaGetLastError());
+  h->launches += 1;
+  return LMZ_OK;
 }
 
 constexpr int TMA_THREADS = 32;      // one warp per SM issues the bulk copies: the TMA engine does the moving
@@ -290,80 +361,38 @@ constexpr int ST_THREADS = 1024;     // 32 warps of vector stores per SM
 
 template <class V, int RENDER, int THREADS>
 int launch_env_t(lmz_env *h, const lmz::KParams &p, cudaStream_t s) {
-  auto kern = (RENDER == lmz::RENDER_TMA) ? lmz::lmz_env_tma_kernel<V, THREADS> : lmz::lmz_env_st_kernel<V, THREADS>;
-  static thread_local int configured_dev = -1;
-  static thread_local int ctas_per_sm = 1;
-  if (configured_dev != h->cfg.device) {
-    LMZ_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)V::BLOB_BYTES));
-    LMZ_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas_per_sm, kern, THREADS, V::BLOB_BYTES));
-    if (ctas_per_sm < 1) return fail(LMZ_ERR_CUDA, "env kernel does not fit on an SM");
-    configured_dev = h->cfg.device;
-  }
+  constexpr auto kern = (RENDER == lmz::RENDER_TMA) ? lmz::lmz_env_tma_kernel<V, THREADS> : lmz::lmz_env_st_kernel<V, THREADS>;
+  const int fit = resident_ctas<kern>(h, THREADS, V::BLOB_BYTES, true, "env kernel");
+  if (fit < 0) return fit;
   // persistent grid: a whole number of CTAs per SM, never more CTAs than tiles
-  const int64_t units = p.tile_end - p.tile_begin;
   // TMA render: ONE issuing CTA per SM even where two fit (v3: 7,528 vs 7,481 GB/s, tools/v3_sweep.py)
-  int per_sm = h->cfg.tune[2] > 0 ? h->cfg.tune[2] : (RENDER == lmz::RENDER_TMA ? 1 : ctas_per_sm);
-  if (per_sm > ctas_per_sm) per_sm = ctas_per_sm;
-  int64_t grid = (int64_t)h->num_sms * per_sm;
-  if (grid > units) grid = units;
-  if (grid < 1) grid = 1;
-  kern<<<(unsigned)grid, THREADS, V::BLOB_BYTES, s>>>(p);
-  LMZ_CUDA(cudaGetLastError());
-  h->launches += 1;
-  return LMZ_OK;
+  const int per_sm = ctas_per_sm(h, RENDER == lmz::RENDER_TMA ? 1 : fit, fit);
+  return launch(h, kern, persistent_grid(h, per_sm, p.tile_end - p.tile_begin), THREADS, V::BLOB_BYTES, s, p);
 }
 
 // transition-only (no obs bound) and compact-obs launches: persistent 128-thread CTAs, dynamic tiles
 template <class V>
 int launch_compact(lmz_env *h, const lmz::KParams &p, cudaStream_t s) {
   constexpr int THREADS = 128;
-  auto kern = lmz::lmz_env_compact_kernel<V, THREADS>;
-  static thread_local int configured_dev = -1;
-  static thread_local int ctas_per_sm = 1;
-  if (configured_dev != h->cfg.device) {
-    LMZ_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas_per_sm, kern, THREADS, 0));
-    if (ctas_per_sm < 1) return fail(LMZ_ERR_CUDA, "compact env kernel does not fit on an SM");
-    configured_dev = h->cfg.device;
-  }
-  const int64_t units = p.tile_end - p.tile_begin;
+  constexpr auto kern = lmz::lmz_env_compact_kernel<V, THREADS>;
+  const int fit = resident_ctas<kern>(h, THREADS, 0, false, "compact env kernel");
+  if (fit < 0) return fit;
   // resident CTAs per SM (tools/small_bench.py): with observations to write, TWO 4-warp CTAs per SM stream more
   // (10.9 vs 9.9 G env-steps/s on v0) than the 8 that fit -- fewer storing warps, higher write bandwidth; the
   // transition-only launch (14 B per env, latency-bound) wants them all
-  int per_sm = h->cfg.tune[2] > 0 ? h->cfg.tune[2] : (p.obs != nullptr ? 2 : ctas_per_sm);
-  if (per_sm > ctas_per_sm) per_sm = ctas_per_sm;
-  int64_t grid = (int64_t)h->num_sms * per_sm;
-  const int64_t need = (units + THREADS / 32 - 1) / (THREADS / 32);
-  if (grid > need) grid = need;
-  if (grid < 1) grid = 1;
-  kern<<<(unsigned)grid, THREADS, 0, s>>>(p);
-  LMZ_CUDA(cudaGetLastError());
-  h->launches += 1;
-  return LMZ_OK;
+  const int per_sm = ctas_per_sm(h, p.obs != nullptr ? 2 : fit, fit);
+  return launch(h, kern, persistent_grid(h, per_sm, ceil_div(p.tile_end - p.tile_begin, THREADS / 32)), THREADS, 0, s, p);
 }
 
 // incremental render (LMZ_RENDER_INCREMENTAL): only the ball / goal blocks that moved are rewritten
 template <class V>
 int launch_incremental(lmz_env *h, const lmz::KParams &p, cudaStream_t s) {
   constexpr int THREADS = 128;
-  auto kern = lmz::lmz_env_incr_kernel<V, THREADS>;
-  static thread_local int configured_dev = -1;
-  static thread_local int ctas_per_sm = 1;
-  if (configured_dev != h->cfg.device) {
-    LMZ_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas_per_sm, kern, THREADS, 0));
-    if (ctas_per_sm < 1) return fail(LMZ_ERR_CUDA, "incremental env kernel does not fit on an SM");
-    configured_dev = h->cfg.device;
-  }
-  const int64_t units = p.tile_end - p.tile_begin;
-  int per_sm = h->cfg.tune[2] > 0 ? h->cfg.tune[2] : (V::ID == 0 ? 4 : 6);      // tools/small_bench.py: +10 % over full occupancy
-  if (per_sm > ctas_per_sm) per_sm = ctas_per_sm;
-  int64_t grid = (int64_t)h->num_sms * per_sm;
-  const int64_t need = (units + THREADS / 32 - 1) / (THREADS / 32);
-  if (grid > need) grid = need;
-  if (grid < 1) grid = 1;
-  kern<<<(unsigned)grid, THREADS, 0, s>>>(p);
-  LMZ_CUDA(cudaGetLastError());
-  h->launches += 1;
-  return LMZ_OK;
+  constexpr auto kern = lmz::lmz_env_incr_kernel<V, THREADS>;
+  const int fit = resident_ctas<kern>(h, THREADS, 0, false, "incremental env kernel");
+  if (fit < 0) return fit;
+  const int per_sm = ctas_per_sm(h, V::ID == 0 ? 4 : 6, fit);      // tools/small_bench.py: +10 % over full occupancy
+  return launch(h, kern, persistent_grid(h, per_sm, ceil_div(p.tile_end - p.tile_begin, THREADS / 32)), THREADS, 0, s, p);
 }
 
 template <class V>
@@ -398,25 +427,11 @@ int launch_env_v(lmz_env *h, const lmz::KParams &p, cudaStream_t s) {
 
 template <class W, int THREADS>
 int launch_fov_t(lmz_env *h, const lmz::KParams &p, cudaStream_t s) {
-  auto kern = lmz::lmz_env_fov_kernel<W, THREADS>;
-  static thread_local int configured_dev = -1;
-  static thread_local int ctas_per_sm = 1;
-  if (configured_dev != h->cfg.device) {
-    LMZ_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)W::SMEM_BYTES));
-    LMZ_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas_per_sm, kern, THREADS, W::SMEM_BYTES));
-    if (ctas_per_sm < 1) return fail(LMZ_ERR_CUDA, "foveal env kernel does not fit on an SM");
-    configured_dev = h->cfg.device;
-  }
-  const int64_t units = p.tile_end - p.tile_begin;
-  int per_sm = h->cfg.tune[2] > 0 ? h->cfg.tune[2] : 1;          // default: ONE persistent CTA per SM
-  if (per_sm > ctas_per_sm) per_sm = ctas_per_sm;
-  int64_t grid = (int64_t)h->num_sms * per_sm;
-  if (grid > units) grid = units;
-  if (grid < 1) grid = 1;
-  kern<<<(unsigned)grid, THREADS, W::SMEM_BYTES, s>>>(p);
-  LMZ_CUDA(cudaGetLastError());
-  h->launches += 1;
-  return LMZ_OK;
+  constexpr auto kern = lmz::lmz_env_fov_kernel<W, THREADS>;
+  const int fit = resident_ctas<kern>(h, THREADS, W::SMEM_BYTES, true, "foveal env kernel");
+  if (fit < 0) return fit;
+  const int per_sm = ctas_per_sm(h, 1, fit);          // default: ONE persistent CTA per SM
+  return launch(h, kern, persistent_grid(h, per_sm, p.tile_end - p.tile_begin), THREADS, W::SMEM_BYTES, s, p);
 }
 
 template <class W>
@@ -446,30 +461,15 @@ template <class W, int THREADS>
 int launch_fov_small_t(lmz_env *h, const lmz::KParams &p, cudaStream_t s) {
   if (W::HAS_LOC && !h->local_bound)
     return fail(LMZ_ERR_STATE, "lmaze-v5/v6: local outputs not bound: call lmz_bind_local first");
-  auto kern = lmz::lmz_fov_small_kernel<W, THREADS>;
+  constexpr auto kern = lmz::lmz_fov_small_kernel<W, THREADS>;
   constexpr int SMEM = (int)lmz::FovSmall<W>::smem_bytes(THREADS);      // tables + one 32-env tile of rows per warp
-  static thread_local int configured_dev = -1;
-  static thread_local int ctas_per_sm = 1;
-  if (configured_dev != h->cfg.device) {
-    LMZ_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
-    LMZ_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas_per_sm, kern, THREADS, SMEM));
-    if (ctas_per_sm < 1) return fail(LMZ_ERR_CUDA, "foveal compact kernel does not fit on an SM");
-    configured_dev = h->cfg.device;
-  }
-  const int64_t units = p.tile_end - p.tile_begin;
+  const int fit = resident_ctas<kern>(h, THREADS, SMEM, true, "foveal compact kernel");
+  if (fit < 0) return fit;
   // resident CTAs per SM (tools/fov_compact_sweep.py): v2 writes through the TMA engine only, and ONE 4-warp CTA per
   // SM streams more (11.5 G env-steps/s) than the three that fit (9.2 G) -- fewer writers, higher write bandwidth;
   // the visit variants and the launches that write nothing are latency-bound and want every CTA that fits
-  int per_sm = h->cfg.tune[2] > 0 ? h->cfg.tune[2] : ((W::NVIS == 0 && p.obs != nullptr) ? 1 : ctas_per_sm);
-  if (per_sm > ctas_per_sm) per_sm = ctas_per_sm;
-  int64_t grid = (int64_t)h->num_sms * per_sm;
-  const int64_t need = (units + THREADS / 32 - 1) / (THREADS / 32);
-  if (grid > need) grid = need;
-  if (grid < 1) grid = 1;
-  kern<<<(unsigned)grid, THREADS, SMEM, s>>>(p);
-  LMZ_CUDA(cudaGetLastError());
-  h->launches += 1;
-  return LMZ_OK;
+  const int per_sm = ctas_per_sm(h, (W::NVIS == 0 && p.obs != nullptr) ? 1 : fit, fit);
+  return launch(h, kern, persistent_grid(h, per_sm, ceil_div(p.tile_end - p.tile_begin, THREADS / 32)), THREADS, SMEM, s, p);
 }
 
 template <class W>
@@ -491,24 +491,11 @@ int launch_planner(lmz_env *h, const lmz::KParams &p, cudaStream_t s) {
   using W = lmz::V5;
   constexpr int THREADS = 128;
   if (!h->local_bound) return fail(LMZ_ERR_STATE, "lmaze-v5/v6: local outputs not bound: call lmz_bind_local first");
-  auto kern = lmz::lmz_planner_kernel<W, THREADS>;
-  static thread_local int configured_dev = -1;
-  static thread_local int ctas_per_sm = 1;
-  if (configured_dev != h->cfg.device) {
-    LMZ_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)W::BLOB_BYTES));
-    LMZ_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas_per_sm, kern, THREADS, W::BLOB_BYTES));
-    if (ctas_per_sm < 1) return fail(LMZ_ERR_CUDA, "planner kernel does not fit on an SM");
-    configured_dev = h->cfg.device;
-  }
-  const int64_t units = p.tile_end - p.tile_begin;
-  int64_t grid = (int64_t)h->num_sms * ctas_per_sm;
-  const int64_t need = (units + THREADS / 32 - 1) / (THREADS / 32);
-  if (grid > need) grid = need;
-  if (grid < 1) grid = 1;
-  kern<<<(unsigned)grid, THREADS, W::BLOB_BYTES, s>>>(p);
-  LMZ_CUDA(cudaGetLastError());
-  h->launches += 1;
-  return LMZ_OK;
+  constexpr auto kern = lmz::lmz_planner_kernel<W, THREADS>;
+  const int fit = resident_ctas<kern>(h, THREADS, W::BLOB_BYTES, true, "planner kernel");
+  if (fit < 0) return fit;
+  // every CTA that fits, whatever tune[2] says
+  return launch(h, kern, persistent_grid(h, fit, ceil_div(p.tile_end - p.tile_begin, THREADS / 32)), THREADS, W::BLOB_BYTES, s, p);
 }
 
 int launch_env(lmz_env *h, const lmz::KParams &p, cudaStream_t s) {
@@ -524,14 +511,8 @@ int launch_env(lmz_env *h, const lmz::KParams &p, cudaStream_t s) {
 template <class V>
 int launch_rollout_v(lmz_env *h, const lmz::KParams &p, cudaStream_t s) {
   constexpr int THREADS = 256;
-  int64_t blocks = (p.n + THREADS - 1) / THREADS;
-  const int64_t cap = (int64_t)h->num_sms * 8;            // 8 resident CTAs of 256 threads per SM
-  if (blocks > cap) blocks = cap;
-  if (blocks < 1) blocks = 1;
-  lmz::lmz_rollout_kernel<V, THREADS><<<(unsigned)blocks, THREADS, 0, s>>>(p);
-  LMZ_CUDA(cudaGetLastError());
-  h->launches += 1;
-  return LMZ_OK;
+  // 8 resident CTAs of 256 threads per SM
+  return launch(h, lmz::lmz_rollout_kernel<V, THREADS>, persistent_grid(h, 8, ceil_div(p.n, THREADS)), THREADS, 0, s, p);
 }
 
 template <class W>
@@ -539,22 +520,10 @@ int launch_fov_rollout(lmz_env *h, const lmz::KParams &p, cudaStream_t s) {
   constexpr int THREADS = 128;
   constexpr int TAB = (int)((W::BLOB_BYTES - W::ROWBITS_OFF + 15u) & ~15u);
   constexpr int SMEM = TAB + THREADS * lmz::HIST_STRIDE;               // tables + one visit-history row per thread
-  auto kern = lmz::lmz_fov_rollout_kernel<W, THREADS>;
-  static thread_local int configured_dev = -1;
-  static thread_local int ctas_per_sm = 1;
-  if (configured_dev != h->cfg.device) {
-    LMZ_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas_per_sm, kern, THREADS, SMEM));
-    if (ctas_per_sm < 1) return fail(LMZ_ERR_CUDA, "foveal rollout kernel does not fit on an SM");
-    configured_dev = h->cfg.device;
-  }
-  int64_t blocks = (p.n + THREADS - 1) / THREADS;
-  const int64_t cap = (int64_t)h->num_sms * ctas_per_sm;
-  if (blocks > cap) blocks = cap;
-  if (blocks < 1) blocks = 1;
-  kern<<<(unsigned)blocks, THREADS, SMEM, s>>>(p);
-  LMZ_CUDA(cudaGetLastError());
-  h->launches += 1;
-  return LMZ_OK;
+  constexpr auto kern = lmz::lmz_fov_rollout_kernel<W, THREADS>;
+  const int fit = resident_ctas<kern>(h, THREADS, SMEM, false, "foveal rollout kernel");
+  if (fit < 0) return fit;
+  return launch(h, kern, persistent_grid(h, fit, ceil_div(p.n, THREADS)), THREADS, SMEM, s, p);
 }
 
 int check_handle(lmz_env *h) {
@@ -567,30 +536,46 @@ int check_bound(lmz_env *h) {
   return LMZ_OK;
 }
 
+// bytes of one action (goal) of LMZ_ACT_* dtype `d`; 0 for an unknown dtype
+size_t action_bytes(int32_t d) { return d == LMZ_ACT_U8 ? 1 : d == LMZ_ACT_I32 ? 4 : d == LMZ_ACT_I64 ? 8 : 0; }
+
+int check_action_dtype(int32_t d, const char *what) {
+  if (!action_bytes(d)) return fail(LMZ_ERR_INVALID, "unknown %s %d", what, d);
+  return LMZ_OK;
+}
+
 // ---- DLPack validation -----------------------------------------------------
+constexpr uint8_t ANY_INT = 255;   // Want::code of an action-like tensor: uint8, int32 or int64
+
 struct Want {
   const char *name;
-  uint8_t code;      // DLDataTypeCode, or 255 = any integer action type
+  uint8_t code;      // DLDataTypeCode, or ANY_INT
   uint8_t bits;
   int ndim;
   int64_t shape[4];
-  bool host_ok;
   int align;        // required alignment of the data pointer in bytes
 };
 
-int check_dl(const lmz_env *h, const DLManagedTensor *mt, const Want &w, void **data, int *action_dtype) {
+// a per-env vector [n] and a per-step matrix [T, n], aligned to their element
+Want per_env(const lmz_env *h, const char *name, uint8_t code, uint8_t bits = 0) {
+  return Want{name, code, bits, 1, {h->cfg.num_envs, 0, 0, 0}, code == ANY_INT ? 1 : bits / 8};
+}
+
+Want per_step(const lmz_env *h, const char *name, int32_t T, uint8_t code, uint8_t bits = 0) {
+  return Want{name, code, bits, 2, {T, h->cfg.num_envs, 0, 0}, code == ANY_INT ? 1 : bits / 8};
+}
+
+int check_dl(const lmz_env *h, const DLManagedTensor *mt, const Want &w, void **data, int *action_dtype = nullptr) {
   if (!mt) return fail(LMZ_ERR_INVALID, "%s: DLManagedTensor is NULL", w.name);
   const DLTensor &t = mt->dl_tensor;
-  if (t.device.device_type == kDLCUDA || t.device.device_type == kDLCUDAManaged) {
-    if (t.device.device_id != h->cfg.device)
-      return fail(LMZ_ERR_INVALID, "%s: tensor is on cuda:%d, env is on cuda:%d", w.name, t.device.device_id,
-                  h->cfg.device);
-  } else if (!(w.host_ok && (t.device.device_type == kDLCUDAHost || t.device.device_type == kDLCPU))) {
+  if (t.device.device_type != kDLCUDA && t.device.device_type != kDLCUDAManaged)
     return fail(LMZ_ERR_INVALID, "%s: tensor must live on the CUDA device (device_type %d)", w.name,
                 t.device.device_type);
-  }
+  if (t.device.device_id != h->cfg.device)
+    return fail(LMZ_ERR_INVALID, "%s: tensor is on cuda:%d, env is on cuda:%d", w.name, t.device.device_id,
+                h->cfg.device);
   if (t.dtype.lanes != 1) return fail(LMZ_ERR_INVALID, "%s: vector dtypes not supported", w.name);
-  if (w.code == 255) {
+  if (w.code == ANY_INT) {
     int ad = -1;
     if ((t.dtype.code == kDLUInt || t.dtype.code == kDLBool) && t.dtype.bits == 8) ad = LMZ_ACT_U8;
     else if (t.dtype.code == kDLInt && t.dtype.bits == 32) ad = LMZ_ACT_I32;
@@ -624,6 +609,47 @@ int check_dl(const lmz_env *h, const DLManagedTensor *mt, const Want &w, void **
   return LMZ_OK;
 }
 
+// Frees whatever the host pipeline holds -- all of it, or what a failed set-up got to create -- and marks it
+// not set up.
+void release_pipe(lmz_env *h) {
+  auto &pp = h->pipe;
+  if (pp.copy) cudaStreamSynchronize(pp.copy);
+  for (int i = 0; i < 2; ++i) {
+    if (pp.ready[i]) cudaEventDestroy(pp.ready[i]);
+    if (pp.drained[i]) cudaEventDestroy(pp.drained[i]);
+    cudaFree(pp.act[i]); cudaFree(pp.obs[i]); cudaFree(pp.reward[i]); cudaFree(pp.done[i]);
+  }
+  if (pp.copy) cudaStreamDestroy(pp.copy);
+  memset(&pp, 0, sizeof(pp));
+}
+
+// Creates the host pipeline's copy stream, events and staging buffers for n envs.  On failure the caller releases
+// what was created.
+int setup_pipe(lmz_env *h, size_t n) {
+  auto &pp = h->pipe;
+  LMZ_CUDA(cudaStreamCreateWithFlags(&pp.copy, cudaStreamNonBlocking));
+  for (int i = 0; i < 2; ++i) {
+    LMZ_CUDA(cudaEventCreateWithFlags(&pp.ready[i], cudaEventDisableTiming));
+    LMZ_CUDA(cudaEventCreateWithFlags(&pp.drained[i], cudaEventDisableTiming));
+    LMZ_CUDA(cudaMalloc(&pp.act[i], n * 8));
+    LMZ_CUDA(cudaMalloc(&pp.reward[i], n * sizeof(float)));
+    LMZ_CUDA(cudaMalloc(&pp.done[i], n));
+  }
+  pp.init = true;
+  return LMZ_OK;
+}
+
+// n copies of `value` to device memory, through a host buffer of at most 2^20 words
+cudaError_t fill_u32(uint32_t *dst, size_t n, uint32_t value) {
+  const std::vector<uint32_t> chunk(n < (1u << 20) ? n : (1u << 20), value);
+  cudaError_t e = cudaSuccess;
+  for (size_t off = 0; off < n && e == cudaSuccess; off += chunk.size()) {
+    const size_t cnt = (n - off < chunk.size()) ? n - off : chunk.size();
+    e = cudaMemcpy(dst + off, chunk.data(), cnt * sizeof(uint32_t), cudaMemcpyHostToDevice);
+  }
+  return e;
+}
+
 }  // namespace
 
 // ================================================================== exports
@@ -647,38 +673,33 @@ void lmz_default_config(lmz_config *cfg) {
 
 int lmz_obs_shape(int32_t variant, int64_t shape[3]) {
   if (!shape) return fail(LMZ_ERR_INVALID, "shape is NULL");
-  if (variant == LMZ_V0) { shape[0] = lmz::V0::C; shape[1] = shape[2] = lmz::V0::S; return LMZ_OK; }
-  if (variant == LMZ_V3) { shape[0] = lmz::V3::C; shape[1] = shape[2] = lmz::V3::S; return LMZ_OK; }
-  if (variant == LMZ_V2) { shape[0] = lmz::V2::C; shape[1] = shape[2] = lmz::V2::S; return LMZ_OK; }
-  if (variant == LMZ_V4) { shape[0] = lmz::V4::C; shape[1] = shape[2] = lmz::V4::S; return LMZ_OK; }
-  if (variant == LMZ_V5) { shape[0] = lmz::V5::C; shape[1] = shape[2] = lmz::V5::S; return LMZ_OK; }
-  return fail(LMZ_ERR_UNSUPPORTED, "unknown variant %d", variant);
+  const VariantInfo *v = variant_info(variant);
+  if (!v) return unknown_variant(variant);
+  shape[0] = v->C; shape[1] = shape[2] = v->S;
+  return LMZ_OK;
 }
 
 int lmz_local_obs_shape(int32_t variant, int64_t shape[3]) {
   if (!shape) return fail(LMZ_ERR_INVALID, "shape is NULL");
-  if (variant != LMZ_V5) return fail(LMZ_ERR_UNSUPPORTED, "only lmaze-v5/v6 have a local observation");
-  shape[0] = lmz::V5::CL; shape[1] = shape[2] = lmz::V5::S;       // lmaze_env_v5.py:357-358
+  const VariantInfo *v = variant_info(variant);
+  if (!v || !v->CL) return fail(LMZ_ERR_UNSUPPORTED, "only lmaze-v5/v6 have a local observation");
+  shape[0] = v->CL; shape[1] = shape[2] = v->S;
   return LMZ_OK;
 }
 
 int lmz_state_cols(int32_t variant) {
-  if (variant == LMZ_V5) return LMZ_ST_COLS_HIER;
-  if (variant == LMZ_V0 || variant == LMZ_V2 || variant == LMZ_V3 || variant == LMZ_V4) return LMZ_ST_COLS;
-  return fail(LMZ_ERR_UNSUPPORTED, "unknown variant %d", variant);
+  const VariantInfo *v = variant_info(variant);
+  return v ? v->state_cols : unknown_variant(variant);
 }
 
 int lmz_num_actions(int32_t variant) {
-  if (variant == LMZ_V0 || variant == LMZ_V3) return 4;      // lmaze_env.py:16, lmaze_env_v3.py:92
-  if (variant == LMZ_V2 || variant == LMZ_V4) return 25;     // lmaze_env_v2.py:39 (commented out in v4, :43-44)
-  if (variant == LMZ_V5) return 4;                           // step() moves by one cell (lmaze_env_v5.py:205-217); plannerStep takes 25
-  return fail(LMZ_ERR_UNSUPPORTED, "unknown variant %d", variant);
+  const VariantInfo *v = variant_info(variant);
+  return v ? v->num_actions : unknown_variant(variant);
 }
 
 int lmz_num_layouts(int32_t variant) {
-  if (variant == LMZ_V0 || variant == LMZ_V3) return 1;
-  if (variant == LMZ_V2 || variant == LMZ_V4 || variant == LMZ_V5) return 5;      // lmaze_env_v2.py:306, lmaze_env_v4.py:351
-  return fail(LMZ_ERR_UNSUPPORTED, "unknown variant %d", variant);
+  const VariantInfo *v = variant_info(variant);
+  return v ? v->num_layouts : unknown_variant(variant);
 }
 
 int lmz_layout_ex(int32_t variant, int32_t index, char *cells) {
@@ -686,21 +707,21 @@ int lmz_layout_ex(int32_t variant, int32_t index, char *cells) {
   const int nl = lmz_num_layouts(variant);
   if (nl < 0) return nl;
   if (index < 1 || index > nl) return fail(LMZ_ERR_INVALID, "layout index %d outside 1..%d", index, nl);
-  if (variant == LMZ_V2 || variant == LMZ_V4 || variant == LMZ_V5) { v2_cells(index, cells); return LMZ_OK; }
+  if (!variant_info(variant)->cells) { v2_cells(index, cells); return LMZ_OK; }
   return lmz_layout(variant, cells);
 }
 
 int lmz_obs_desc(int32_t variant, int32_t obs_mode, int64_t shape[3], int32_t *elem_bytes) {
   if (!shape) return fail(LMZ_ERR_INVALID, "shape is NULL");
   if (int rc = lmz_obs_shape(variant, shape)) return rc;
+  const VariantInfo *v = variant_info(variant);
   if (obs_mode == LMZ_OBS_COMPACT) {
-    const bool fov = variant == LMZ_V2 || variant == LMZ_V4 || variant == LMZ_V5;
-    shape[1] = shape[2] = fov ? 5 : lmz_grid_size(variant);        // foveal variants: the 5x5 crops, as float32
-    if (elem_bytes) *elem_bytes = fov ? 4 : 1;
+    shape[1] = shape[2] = v->foveal ? 5 : v->G;        // foveal variants: the 5x5 crops, as float32
+    if (elem_bytes) *elem_bytes = v->foveal ? 4 : 1;
   } else if (obs_mode == LMZ_OBS_BITS) {
-    if (variant != LMZ_V0 && variant != LMZ_V3)
+    if (!v->bits_bytes)
       return fail(LMZ_ERR_UNSUPPORTED, "bit-packed observations exist for the full-view variants (v0, v3) only");
-    shape[0] = variant == LMZ_V0 ? lmz::V0::BITS_WORDS * 4 : lmz::V3::BITS_WORDS * 4;   // one row of bytes per env
+    shape[0] = v->bits_bytes;                          // one row of bytes per env
     shape[1] = shape[2] = 1;
     if (elem_bytes) *elem_bytes = 1;
   } else if (obs_mode == LMZ_OBS_FULL) {
@@ -712,18 +733,16 @@ int lmz_obs_desc(int32_t variant, int32_t obs_mode, int64_t shape[3], int32_t *e
 }
 
 int lmz_grid_size(int32_t variant) {
-  if (variant == LMZ_V0) return lmz::V0::G;
-  if (variant == LMZ_V3 || variant == LMZ_V2 || variant == LMZ_V4 || variant == LMZ_V5) return lmz::V3::G;
-  return fail(LMZ_ERR_UNSUPPORTED, "unknown variant %d", variant);
+  const VariantInfo *v = variant_info(variant);
+  return v ? v->G : unknown_variant(variant);
 }
 
 int lmz_layout(int32_t variant, char *cells) {
-  if (variant == LMZ_V2 || variant == LMZ_V4 || variant == LMZ_V5) return lmz_layout_ex(variant, 1, cells);
-  const char *c = cells_of(variant);
-  if (!c) return fail(LMZ_ERR_UNSUPPORTED, "unknown variant %d", variant);
+  const VariantInfo *v = variant_info(variant);
+  if (!v) return unknown_variant(variant);
+  if (!v->cells) return lmz_layout_ex(variant, 1, cells);
   if (!cells) return fail(LMZ_ERR_INVALID, "cells is NULL");
-  const int G = lmz_grid_size(variant);
-  memcpy(cells, c, (size_t)G * G);
+  memcpy(cells, v->cells, (size_t)v->G * v->G);
   return LMZ_OK;
 }
 
@@ -733,25 +752,23 @@ int lmz_create(const lmz_config *cfg, lmz_env **out) {
   if (cfg->struct_size != (int32_t)sizeof(lmz_config))
     return fail(LMZ_ERR_INVALID, "lmz_config.struct_size %d != %d: header/library mismatch", cfg->struct_size,
                 (int)sizeof(lmz_config));
-  if (cfg->variant != LMZ_V0 && cfg->variant != LMZ_V3 && cfg->variant != LMZ_V2 && cfg->variant != LMZ_V4 &&
-      cfg->variant != LMZ_V5)
+  const VariantInfo *v = variant_info(cfg->variant);
+  if (!v)
     return fail(LMZ_ERR_UNSUPPORTED,
                 "variant %d is not built (supported: 0 = lmaze-v0, 2 = lmaze-v2, 3 = lmaze-v3, 4 = lmaze-v4, "
                 "5 = lmaze-v5/v6)", cfg->variant);
-  const bool hier = cfg->variant == LMZ_V5;
-  const bool foveal = cfg->variant == LMZ_V2 || cfg->variant == LMZ_V4;
   if (cfg->num_envs < 1) return fail(LMZ_ERR_INVALID, "num_envs must be >= 1 (got %lld)", (long long)cfg->num_envs);
   if (cfg->env_id0 < 0) return fail(LMZ_ERR_INVALID, "env_id0 must be >= 0");
   if (cfg->render_mode != LMZ_RENDER_TMA && cfg->render_mode != LMZ_RENDER_ST128 &&
       cfg->render_mode != LMZ_RENDER_INCREMENTAL)
     return fail(LMZ_ERR_INVALID, "unknown render_mode %d", cfg->render_mode);
-  if (cfg->render_mode == LMZ_RENDER_INCREMENTAL && (foveal || hier))
+  if (cfg->render_mode == LMZ_RENDER_INCREMENTAL && v->foveal)
     return fail(LMZ_ERR_UNSUPPORTED, "incremental render needs a full-view variant (v0, v3): a foveal crop changes entirely every step");
   for (int i = 0; i < 2; ++i)
     if (cfg->reserved[i] != 0) return fail(LMZ_ERR_INVALID, "lmz_config.reserved must be zero");
   if (cfg->obs_mode != LMZ_OBS_FULL && cfg->obs_mode != LMZ_OBS_COMPACT && cfg->obs_mode != LMZ_OBS_BITS)
     return fail(LMZ_ERR_INVALID, "unknown obs_mode %d", cfg->obs_mode);
-  if (cfg->obs_mode == LMZ_OBS_BITS && (foveal || hier))
+  if (cfg->obs_mode == LMZ_OBS_BITS && !v->bits_bytes)
     return fail(LMZ_ERR_UNSUPPORTED, "bit-packed observations exist for the full-view variants (v0, v3) only");
   {
     const int t = cfg->tune[0];
@@ -780,92 +797,52 @@ int lmz_create(const lmz_config *cfg, lmz_env **out) {
   h->cfg = *cfg;
   h->num_sms = prop.multiProcessorCount;
   h->win_lo = 0; h->win_n = cfg->num_envs;
+  h->var = v;
   std::vector<unsigned char> blob;
-  if (cfg->variant == LMZ_V0) {
-    h->G = lmz::V0::G; h->C = lmz::V0::C; h->S = lmz::V0::S; h->obs_bytes_per_env = lmz::V0::OBS_BYTES;
-    h->compact_bytes_per_env = lmz::V0::COMPACT_BYTES;
-    build_blob<lmz::V0>(V0_CELLS, blob, h->n_cand, h->s_cell, h->x_cell);
-  } else if (cfg->variant == LMZ_V2) {
-    h->G = lmz::V2::G; h->C = lmz::V2::C; h->S = lmz::V2::S; h->obs_bytes_per_env = lmz::V2::OBS_BYTES;
-    h->compact_bytes_per_env = lmz::V2::C * 25 * 4;
-    build_blob_fov<lmz::V2>(blob);
-    h->s_cell = 4 * 18 + 4; h->x_cell = 8 * 18 + 8;
-  } else if (cfg->variant == LMZ_V4) {
-    h->G = lmz::V4::G; h->C = lmz::V4::C; h->S = lmz::V4::S; h->obs_bytes_per_env = lmz::V4::OBS_BYTES;
-    h->compact_bytes_per_env = lmz::V4::C * 25 * 4;
-    build_blob_fov<lmz::V4>(blob);
-    h->s_cell = 4 * 18 + 4; h->x_cell = 8 * 18 + 8;
-  } else if (cfg->variant == LMZ_V5) {
-    h->G = lmz::V5::G; h->C = lmz::V5::C; h->S = lmz::V5::S; h->obs_bytes_per_env = lmz::V5::OBS_BYTES;
-    h->compact_bytes_per_env = lmz::V5::C * 25 * 4;
-    build_blob_v5(blob);
-    h->s_cell = 4 * 18 + 4; h->x_cell = 8 * 18 + 8;
-  } else {
-    h->G = lmz::V3::G; h->C = lmz::V3::C; h->S = lmz::V3::S; h->obs_bytes_per_env = lmz::V3::OBS_BYTES;
-    h->compact_bytes_per_env = lmz::V3::COMPACT_BYTES;
-    build_blob<lmz::V3>(V3_CELLS, blob, h->n_cand, h->s_cell, h->x_cell);
-  }
+  v->build_blob(v->cells, blob, h->n_cand, h->s_cell, h->x_cell);
   const size_t n = (size_t)cfg->num_envs;
+  // The per-env state arrays are padded to whole 32-env tiles: the compact foveal kernel fetches a tile's words as
+  // fixed-size bulk copies (lmz_fov.cuh).  The padding is zeroed so that those copies read defined words.
+  const size_t n32 = (n + 31) & ~(size_t)31;
   cudaError_t e = cudaSuccess;
-  // (the per-env state arrays are padded to whole 32-env tiles: the compact foveal kernel fetches a tile's words as
-  // fixed-size bulk copies, lmz_fov.cuh)
-  const size_t n32 = ((size_t)n + 31) & ~(size_t)31;
-  if (e == cudaSuccess) e = cudaMalloc(&h->state, n32 * sizeof(uint32_t));
-  if (e == cudaSuccess) e = cudaMalloc(&h->goal_count, n32 * sizeof(uint32_t));
-  if (e == cudaSuccess) e = cudaMalloc(&h->episode, n * sizeof(uint32_t));
-  if (e == cudaSuccess) e = cudaMalloc(&h->blob, blob.size());
-  if (e == cudaSuccess && hier) e = cudaMalloc(&h->aux2, n32 * sizeof(uint32_t));
-  if (e == cudaSuccess && (cfg->variant == LMZ_V4 || hier)) {      // state[2], the float visit layer (lmaze_env_v4.py:106-113)
-    e = cudaMalloc(&h->visit, n * 324 * sizeof(float));
-    if (e == cudaSuccess) e = cudaMemset(h->visit, 0, n * 324 * sizeof(float));
-    if (e == cudaSuccess) e = cudaMalloc(&h->hist, n32 * 64);           // the visit history (lmz_v2.cuh): empty = an all-zero layer
-    if (e == cudaSuccess) e = cudaMemset(h->hist, 0, n * 64);
+  auto alloc_zero = [&](auto **ptr, size_t bytes) {
+    if (e == cudaSuccess) e = cudaMalloc(ptr, bytes);
+    if (e == cudaSuccess) e = cudaMemset(*ptr, 0, bytes);
+  };
+  alloc_zero(&h->state, n32 * sizeof(uint32_t));
+  alloc_zero(&h->goal_count, n32 * sizeof(uint32_t));
+  alloc_zero(&h->episode, n * sizeof(uint32_t));
+  alloc_zero(&h->stats, (lmz::NUM_STATS + 3) * sizeof(unsigned long long));
+  if (v->hier) alloc_zero(&h->aux2, n32 * sizeof(uint32_t));
+  if (v->has_visit) {
+    alloc_zero(&h->visit, n * 324 * sizeof(float));     // state[2], the float visit layer (lmaze_env_v4.py:106-113)
+    alloc_zero(&h->hist, n32 * 64);                     // the visit history (lmz_v2.cuh): empty = an all-zero layer
   }
-  if (e == cudaSuccess) e = cudaMalloc(&h->stats, (lmz::NUM_STATS + 3) * sizeof(unsigned long long));
-  if (e == cudaSuccess) e = cudaMemset(h->goal_count, 0, n * sizeof(uint32_t));
-  if (e == cudaSuccess) e = cudaMemset(h->episode, 0, n * sizeof(uint32_t));
-  if (e == cudaSuccess) e = cudaMemset(h->stats, 0, (lmz::NUM_STATS + 3) * sizeof(unsigned long long));
+  if (e == cudaSuccess) e = cudaMalloc(&h->blob, blob.size());
   if (e == cudaSuccess) e = cudaMemcpy(h->blob, blob.data(), blob.size(), cudaMemcpyHostToDevice);
   if (e == cudaSuccess) {
     // Before the first reset every env sits on the 'S' cell with the goal on 'X'
     // (lmaze_env_v3.py:119-123 starts at 0,0; any in-range cell keeps the kernels' +-1 lookups in the table).
     lmz::EnvRegs r;
-    r.x = h->s_cell / h->G; r.y = h->s_cell % h->G; r.gx = h->x_cell / h->G; r.gy = h->x_cell % h->G;
+    r.x = h->s_cell / v->G; r.y = h->s_cell % v->G; r.gx = h->x_cell / v->G; r.gy = h->x_cell % v->G;
     r.step = 0; r.rcode = lmz::RC_NEG_ZERO;
     uint32_t packed = (cfg->variant == LMZ_V0) ? lmz::V0::pack(r) : lmz::V3::pack(r);
-    if (foveal) {                          // maze 1, ball on 'S', goal on 'X', no previous action
-      lmz::V2Regs v;
-      v.L = 1; v.x = v.px = 4; v.y = v.py = 4; v.gx = 8; v.gy = 8; v.a = -1; v.step = 0; v.vt = 0;
-      uint32_t aux;
-      lmz::v2_pack(v, packed, aux);
-      std::vector<uint32_t> auxv(n < (1u << 20) ? n : (1u << 20), aux);
-      for (size_t off = 0; off < n && e == cudaSuccess; off += auxv.size()) {
-        const size_t cnt = (n - off < auxv.size()) ? n - off : auxv.size();
-        e = cudaMemcpy(h->goal_count + off, auxv.data(), cnt * sizeof(uint32_t), cudaMemcpyHostToDevice);
-      }
-    }
-    if (hier) {                            // maze 1, everything on 'S', goal on 'X' (the state reset() would leave there)
-      lmz::V5Regs v;
-      v.L = 1; v.x = v.x1 = v.fx1 = v.fgx = v.lx = 4; v.y = v.y1 = v.fy1 = v.fgy = v.ly = 4; v.gx = 8; v.gy = 8;
-      v.fga = 12; v.step = 0; v.fstep = 0; v.ld = 0; v.gd = 0; v.vt = 0;
+    if (v->hier) {                         // maze 1, everything on 'S', goal on 'X' (the state reset() would leave there)
+      lmz::V5Regs r5;
+      r5.L = 1; r5.x = r5.x1 = r5.fx1 = r5.fgx = r5.lx = 4; r5.y = r5.y1 = r5.fy1 = r5.fgy = r5.ly = 4; r5.gx = 8; r5.gy = 8;
+      r5.fga = 12; r5.step = 0; r5.fstep = 0; r5.ld = 0; r5.gd = 0; r5.vt = 0;
       uint32_t w1, w2;
-      lmz::v5_pack(v, packed, w1, w2);
-      std::vector<uint32_t> tmp(n < (1u << 20) ? n : (1u << 20), w1);
-      for (size_t off = 0; off < n && e == cudaSuccess; off += tmp.size()) {
-        const size_t cnt = (n - off < tmp.size()) ? n - off : tmp.size();
-        e = cudaMemcpy(h->goal_count + off, tmp.data(), cnt * sizeof(uint32_t), cudaMemcpyHostToDevice);
-      }
-      tmp.assign(tmp.size(), w2);
-      for (size_t off = 0; off < n && e == cudaSuccess; off += tmp.size()) {
-        const size_t cnt = (n - off < tmp.size()) ? n - off : tmp.size();
-        e = cudaMemcpy(h->aux2 + off, tmp.data(), cnt * sizeof(uint32_t), cudaMemcpyHostToDevice);
-      }
+      lmz::v5_pack(r5, packed, w1, w2);
+      if (e == cudaSuccess) e = fill_u32(h->goal_count, n, w1);
+      if (e == cudaSuccess) e = fill_u32(h->aux2, n, w2);
+    } else if (v->foveal) {                // maze 1, ball on 'S', goal on 'X', no previous action
+      lmz::V2Regs r2;
+      r2.L = 1; r2.x = r2.px = 4; r2.y = r2.py = 4; r2.gx = 8; r2.gy = 8; r2.a = -1; r2.step = 0; r2.vt = 0;
+      uint32_t aux;
+      lmz::v2_pack(r2, packed, aux);
+      if (e == cudaSuccess) e = fill_u32(h->goal_count, n, aux);
     }
-    std::vector<uint32_t> init(n < (1u << 20) ? n : (1u << 20), packed);
-    for (size_t off = 0; off < n && e == cudaSuccess; off += init.size()) {
-      const size_t cnt = (n - off < init.size()) ? n - off : init.size();
-      e = cudaMemcpy(h->state + off, init.data(), cnt * sizeof(uint32_t), cudaMemcpyHostToDevice);
-    }
+    if (e == cudaSuccess) e = fill_u32(h->state, n, packed);
   }
   if (e != cudaSuccess) {
     fail(LMZ_ERR_CUDA, "device allocation/initialisation failed: %s", cudaGetErrorString(e));
@@ -881,14 +858,7 @@ int lmz_destroy(lmz_env *h) {
   DeviceGuard guard(h->cfg.device);
   cudaFree(h->state); cudaFree(h->goal_count); cudaFree(h->episode); cudaFree(h->blob); cudaFree(h->stats);
   cudaFree(h->act_stage); cudaFree(h->visit); cudaFree(h->hist); cudaFree(h->aux2);
-  if (h->pipe.init) {
-    cudaStreamSynchronize(h->pipe.copy);
-    for (int i = 0; i < 2; ++i) {
-      cudaEventDestroy(h->pipe.ready[i]); cudaEventDestroy(h->pipe.drained[i]);
-      cudaFree(h->pipe.act[i]); cudaFree(h->pipe.obs[i]); cudaFree(h->pipe.reward[i]); cudaFree(h->pipe.done[i]);
-    }
-    cudaStreamDestroy(h->pipe.copy);
-  }
+  release_pipe(h);
   delete h;
   return LMZ_OK;
 }
@@ -905,20 +875,14 @@ int lmz_bind(lmz_env *h, void *obs, float *reward, uint8_t *done) {
 }
 
 static int check_obs_dl(lmz_env *h, DLManagedTensor *obs, int64_t rows, void **po) {
-  if (h->cfg.obs_mode == LMZ_OBS_BITS) {
-    Want w{"obs", kDLUInt, 8, 2, {rows, (int64_t)obs_row_bytes(h), 0, 0}, false, 16};
-    return check_dl(h, obs, w, po, nullptr);
-  }
-  if (h->cfg.obs_mode == LMZ_OBS_COMPACT) {
-    if (h->cfg.variant == LMZ_V2 || h->cfg.variant == LMZ_V4 || h->cfg.variant == LMZ_V5) {
-      Want w{"obs", kDLFloat, 32, 4, {rows, h->C, 5, 5}, false, 16};
-      return check_dl(h, obs, w, po, nullptr);
-    }
-    Want w{"obs", kDLUInt, 8, 4, {rows, h->C, h->G, h->G}, false, 16};
-    return check_dl(h, obs, w, po, nullptr);
-  }
-  Want w{"obs", kDLFloat, 32, 4, {rows, h->C, h->S, h->S}, false, 16};
-  return check_dl(h, obs, w, po, nullptr);
+  int64_t shape[3];
+  int32_t elem = 0;
+  if (int rc = lmz_obs_desc(h->cfg.variant, h->cfg.obs_mode, shape, &elem)) return rc;
+  // f32 [rows][C][side][side] or u8 [rows][C][G][G]; bit-packed rows are u8 [rows][bytes]
+  const bool bits = h->cfg.obs_mode == LMZ_OBS_BITS;
+  const Want w{"obs", elem == 4 ? (uint8_t)kDLFloat : (uint8_t)kDLUInt, (uint8_t)(8 * elem), bits ? 2 : 4,
+               {rows, shape[0], shape[1], shape[2]}, 16};
+  return check_dl(h, obs, w, po);
 }
 
 int lmz_bind_dl(lmz_env *h, DLManagedTensor *obs, DLManagedTensor *reward, DLManagedTensor *done) {
@@ -927,17 +891,15 @@ int lmz_bind_dl(lmz_env *h, DLManagedTensor *obs, DLManagedTensor *reward, DLMan
   void *po = nullptr, *pr = nullptr, *pd = nullptr;
   if (obs)
     if (int rc = check_obs_dl(h, obs, n, &po)) return rc;
-  Want wr{"reward", kDLFloat, 32, 1, {n, 0, 0, 0}, false, 4};
-  if (int rc = check_dl(h, reward, wr, &pr, nullptr)) return rc;
-  Want wd{"done", kDLUInt, 8, 1, {n, 0, 0, 0}, false, 1};
-  if (int rc = check_dl(h, done, wd, &pd, nullptr)) return rc;
+  if (int rc = check_dl(h, reward, per_env(h, "reward", kDLFloat, 32), &pr)) return rc;
+  if (int rc = check_dl(h, done, per_env(h, "done", kDLUInt, 8), &pd)) return rc;
   return lmz_bind(h, po, static_cast<float *>(pr), static_cast<uint8_t *>(pd));
 }
 
 int lmz_set_window(lmz_env *h, void *obs, int64_t env_lo, int64_t env_count) {
   if (int rc = check_handle(h)) return rc;
   if (int rc = check_bound(h)) return rc;
-  if (h->cfg.variant == LMZ_V5) return fail(LMZ_ERR_UNSUPPORTED, "lmz_set_window is not built for lmaze-v5/v6");
+  if (h->var->hier) return fail(LMZ_ERR_UNSUPPORTED, "lmz_set_window is not built for lmaze-v5/v6");
   if (!obs) return fail(LMZ_ERR_INVALID, "obs is NULL");
   if ((reinterpret_cast<uintptr_t>(obs) & 15u) != 0) return fail(LMZ_ERR_INVALID, "obs must be 16-byte aligned");
   if (env_lo < 0 || env_count < 1 || env_lo + env_count > h->cfg.num_envs)
@@ -972,13 +934,11 @@ int lmz_reset_dl(lmz_env *h, DLManagedTensor *mask, DLManagedTensor *spawn, void
   if (int rc = check_handle(h)) return rc;
   const int64_t n = h->cfg.num_envs;
   void *pm = nullptr, *ps = nullptr;
-  if (mask) {
-    Want w{"mask", kDLUInt, 8, 1, {n, 0, 0, 0}, false, 1};
-    if (int rc = check_dl(h, mask, w, &pm, nullptr)) return rc;
-  }
+  if (mask)
+    if (int rc = check_dl(h, mask, per_env(h, "mask", kDLUInt, 8), &pm)) return rc;
   if (spawn) {
-    Want w{"spawn", kDLInt, 32, 2, {n, 4, 0, 0}, false, 16};
-    if (int rc = check_dl(h, spawn, w, &ps, nullptr)) return rc;
+    const Want w{"spawn", kDLInt, 32, 2, {n, 4, 0, 0}, 16};
+    if (int rc = check_dl(h, spawn, w, &ps)) return rc;
   }
   return lmz_reset(h, static_cast<const uint8_t *>(pm), static_cast<const int32_t *>(ps), stream);
 }
@@ -987,8 +947,7 @@ int lmz_step(lmz_env *h, const void *actions, int32_t action_dtype, const int32_
   if (int rc = check_handle(h)) return rc;
   if (int rc = check_bound(h)) return rc;
   if (!actions) return fail(LMZ_ERR_INVALID, "actions is NULL");
-  if (action_dtype < LMZ_ACT_U8 || action_dtype > LMZ_ACT_I64)
-    return fail(LMZ_ERR_INVALID, "unknown action dtype %d", action_dtype);
+  if (int rc = check_action_dtype(action_dtype, "action dtype")) return rc;
   if ((reinterpret_cast<uintptr_t>(spawn) & 15u) != 0) return fail(LMZ_ERR_INVALID, "spawn must be 16-byte aligned");
   DeviceGuard guard(h->cfg.device);
   lmz::KParams p = base_params(h);
@@ -1002,11 +961,10 @@ int lmz_step_dl(lmz_env *h, DLManagedTensor *actions, DLManagedTensor *spawn, vo
   const int64_t n = h->cfg.num_envs;
   void *pa = nullptr, *ps = nullptr;
   int ad = 0;
-  Want wa{"actions", 255, 0, 1, {n, 0, 0, 0}, false, 1};
-  if (int rc = check_dl(h, actions, wa, &pa, &ad)) return rc;
+  if (int rc = check_dl(h, actions, per_env(h, "actions", ANY_INT), &pa, &ad)) return rc;
   if (spawn) {
-    Want w{"spawn", kDLInt, 32, 2, {n, 4, 0, 0}, false, 16};
-    if (int rc = check_dl(h, spawn, w, &ps, nullptr)) return rc;
+    const Want w{"spawn", kDLInt, 32, 2, {n, 4, 0, 0}, 16};
+    if (int rc = check_dl(h, spawn, w, &ps)) return rc;
   }
   return lmz_step(h, pa, ad, static_cast<const int32_t *>(ps), stream);
 }
@@ -1016,16 +974,14 @@ int lmz_step_host(lmz_env *h, const void *actions_host, int32_t action_dtype, fl
   if (int rc = check_handle(h)) return rc;
   if (int rc = check_bound(h)) return rc;
   if (!actions_host || !reward_host || !done_host) return fail(LMZ_ERR_INVALID, "host buffers must not be NULL");
-  if (action_dtype < LMZ_ACT_U8 || action_dtype > LMZ_ACT_I64)
-    return fail(LMZ_ERR_INVALID, "unknown action dtype %d", action_dtype);
+  if (int rc = check_action_dtype(action_dtype, "action dtype")) return rc;
   if (obs_host && !h->obs) return fail(LMZ_ERR_STATE, "obs_host given but no device obs buffer is bound");
-  if (h->cfg.variant == LMZ_V5) return fail(LMZ_ERR_UNSUPPORTED, "lmz_step_host is not built for lmaze-v5/v6");
+  if (h->var->hier) return fail(LMZ_ERR_UNSUPPORTED, "lmz_step_host is not built for lmaze-v5/v6");
   DeviceGuard guard(h->cfg.device);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const size_t n = (size_t)h->cfg.num_envs;
   if (!h->act_stage) LMZ_CUDA(cudaMalloc(&h->act_stage, n * 8));
-  const size_t esz = action_dtype == LMZ_ACT_U8 ? 1 : action_dtype == LMZ_ACT_I32 ? 4 : 8;
-  LMZ_CUDA(cudaMemcpyAsync(h->act_stage, actions_host, n * esz, cudaMemcpyHostToDevice, s));
+  LMZ_CUDA(cudaMemcpyAsync(h->act_stage, actions_host, n * action_bytes(action_dtype), cudaMemcpyHostToDevice, s));
   if (int rc = lmz_step(h, h->act_stage, action_dtype, nullptr, stream)) return rc;
   LMZ_CUDA(cudaMemcpyAsync(reward_host, h->reward, n * sizeof(float), cudaMemcpyDeviceToHost, s));
   LMZ_CUDA(cudaMemcpyAsync(done_host, h->done, n, cudaMemcpyDeviceToHost, s));
@@ -1044,36 +1000,27 @@ int lmz_step_host_async(lmz_env *h, const void *actions_host, int32_t action_dty
   if (int rc = check_handle(h)) return rc;
   if (int rc = check_bound(h)) return rc;
   if (!actions_host || !reward_host || !done_host || !ticket) return fail(LMZ_ERR_INVALID, "host buffers / ticket must not be NULL");
-  if (action_dtype < LMZ_ACT_U8 || action_dtype > LMZ_ACT_I64)
-    return fail(LMZ_ERR_INVALID, "unknown action dtype %d", action_dtype);
-  if (h->cfg.variant == LMZ_V5) return fail(LMZ_ERR_UNSUPPORTED, "lmz_step_host_async is not built for lmaze-v5/v6");
+  if (int rc = check_action_dtype(action_dtype, "action dtype")) return rc;
+  if (h->var->hier) return fail(LMZ_ERR_UNSUPPORTED, "lmz_step_host_async is not built for lmaze-v5/v6");
   if (obs_host && h->cfg.obs_mode == LMZ_OBS_FULL)
     return fail(LMZ_ERR_UNSUPPORTED, "the full f32 observation is not double-buffered (2 x N x %zu bytes of HBM): a host "
                 "consumer takes obs_mode compact or bits; pass obs_host = NULL to keep the observation on the device",
-                h->obs_bytes_per_env);
+                (size_t)h->var->obs_bytes);
   if (obs_host && h->win_n != h->cfg.num_envs) return fail(LMZ_ERR_STATE, "obs_host needs the whole batch bound, not a render window");
   DeviceGuard guard(h->cfg.device);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const size_t n = (size_t)h->cfg.num_envs;
   const size_t row = obs_row_bytes(h);
   auto &pp = h->pipe;
-  if (!pp.init) {
-    LMZ_CUDA(cudaStreamCreateWithFlags(&pp.copy, cudaStreamNonBlocking));
-    for (int i = 0; i < 2; ++i) {
-      LMZ_CUDA(cudaEventCreateWithFlags(&pp.ready[i], cudaEventDisableTiming));
-      LMZ_CUDA(cudaEventCreateWithFlags(&pp.drained[i], cudaEventDisableTiming));
-      LMZ_CUDA(cudaMalloc(&pp.act[i], n * 8));
-      LMZ_CUDA(cudaMalloc(&pp.reward[i], n * sizeof(float)));
-      LMZ_CUDA(cudaMalloc(&pp.done[i], n));
-      pp.inflight[i] = false; pp.obs[i] = nullptr;
+  if (!pp.init)
+    if (int rc = setup_pipe(h, n)) {
+      release_pipe(h);
+      return rc;
     }
-    pp.k = 0; pp.init = true;
-  }
   const int slot = (int)(pp.k & 1);
   if (obs_host && !pp.obs[slot]) LMZ_CUDA(cudaMalloc(&pp.obs[slot], n * row));
   if (pp.inflight[slot]) LMZ_CUDA(cudaStreamWaitEvent(s, pp.drained[slot], 0));   // slot's previous copies must be out
-  const size_t esz = action_dtype == LMZ_ACT_U8 ? 1 : action_dtype == LMZ_ACT_I32 ? 4 : 8;
-  LMZ_CUDA(cudaMemcpyAsync(pp.act[slot], actions_host, n * esz, cudaMemcpyHostToDevice, s));
+  LMZ_CUDA(cudaMemcpyAsync(pp.act[slot], actions_host, n * action_bytes(action_dtype), cudaMemcpyHostToDevice, s));
   lmz::KParams p = base_params(h);
   p.mode = lmz::MODE_STEP; p.actions = pp.act[slot]; p.action_dtype = action_dtype;
   p.reward = pp.reward[slot]; p.done = pp.done[slot];
@@ -1131,11 +1078,11 @@ static int rollout_impl(lmz_env *h, int32_t T, const void *actions, int32_t acti
                         uint8_t *reward_codes, uint8_t *dones, void *stream) {
   if (int rc = check_handle(h)) return rc;
   if (T < 1) return fail(LMZ_ERR_INVALID, "T must be >= 1 (got %d)", T);
-  if (h->cfg.variant == LMZ_V5)
+  if (h->var->hier)
     return fail(LMZ_ERR_UNSUPPORTED, "lmaze-v5/v6 roll out through lmz_hier_rollout (planner goals + actor actions)");
   if (!dones) return fail(LMZ_ERR_INVALID, "rewards/dones must not be NULL");
-  if (actions && (action_dtype < LMZ_ACT_U8 || action_dtype > LMZ_ACT_I64))
-    return fail(LMZ_ERR_INVALID, "unknown action dtype %d", action_dtype);
+  if (actions)
+    if (int rc = check_action_dtype(action_dtype, "action dtype")) return rc;
   DeviceGuard guard(h->cfg.device);
   lmz::KParams p = base_params(h);
   p.mode = lmz::MODE_STEP; p.actions = actions; p.action_dtype = action_dtype;
@@ -1152,38 +1099,29 @@ static int rollout_impl(lmz_env *h, int32_t T, const void *actions, int32_t acti
   return rc;
 }
 
-int lmz_rollout_dl(lmz_env *h, int32_t T, DLManagedTensor *actions, DLManagedTensor *rewards, DLManagedTensor *dones,
-                   void *stream) {
+// rewards as f32 [T, n], or (codes) as u8 reward codes [T, n]
+static int rollout_dl(lmz_env *h, int32_t T, DLManagedTensor *actions, DLManagedTensor *rewards, bool codes,
+                      DLManagedTensor *dones, void *stream) {
   if (int rc = check_handle(h)) return rc;
-  const int64_t n = h->cfg.num_envs;
   void *pa = nullptr, *pr = nullptr, *pd = nullptr;
   int ad = 0;
-  if (actions) {
-    Want wa{"actions", 255, 0, 2, {T, n, 0, 0}, false, 1};
-    if (int rc = check_dl(h, actions, wa, &pa, &ad)) return rc;
-  }
-  Want wr{"rewards", kDLFloat, 32, 2, {T, n, 0, 0}, false, 4};
-  if (int rc = check_dl(h, rewards, wr, &pr, nullptr)) return rc;
-  Want wd{"dones", kDLUInt, 8, 2, {T, n, 0, 0}, false, 1};
-  if (int rc = check_dl(h, dones, wd, &pd, nullptr)) return rc;
+  if (actions)
+    if (int rc = check_dl(h, actions, per_step(h, "actions", T, ANY_INT), &pa, &ad)) return rc;
+  const Want wr = codes ? per_step(h, "reward_codes", T, kDLUInt, 8) : per_step(h, "rewards", T, kDLFloat, 32);
+  if (int rc = check_dl(h, rewards, wr, &pr)) return rc;
+  if (int rc = check_dl(h, dones, per_step(h, "dones", T, kDLUInt, 8), &pd)) return rc;
+  if (codes) return lmz_rollout_codes(h, T, pa, ad, static_cast<uint8_t *>(pr), static_cast<uint8_t *>(pd), stream);
   return lmz_rollout(h, T, pa, ad, static_cast<float *>(pr), static_cast<uint8_t *>(pd), stream);
+}
+
+int lmz_rollout_dl(lmz_env *h, int32_t T, DLManagedTensor *actions, DLManagedTensor *rewards, DLManagedTensor *dones,
+                   void *stream) {
+  return rollout_dl(h, T, actions, rewards, false, dones, stream);
 }
 
 int lmz_rollout_codes_dl(lmz_env *h, int32_t T, DLManagedTensor *actions, DLManagedTensor *reward_codes,
                          DLManagedTensor *dones, void *stream) {
-  if (int rc = check_handle(h)) return rc;
-  const int64_t n = h->cfg.num_envs;
-  void *pa = nullptr, *pr = nullptr, *pd = nullptr;
-  int ad = 0;
-  if (actions) {
-    Want wa{"actions", 255, 0, 2, {T, n, 0, 0}, false, 1};
-    if (int rc = check_dl(h, actions, wa, &pa, &ad)) return rc;
-  }
-  Want wr{"reward_codes", kDLUInt, 8, 2, {T, n, 0, 0}, false, 1};
-  if (int rc = check_dl(h, reward_codes, wr, &pr, nullptr)) return rc;
-  Want wd{"dones", kDLUInt, 8, 2, {T, n, 0, 0}, false, 1};
-  if (int rc = check_dl(h, dones, wd, &pd, nullptr)) return rc;
-  return lmz_rollout_codes(h, T, pa, ad, static_cast<uint8_t *>(pr), static_cast<uint8_t *>(pd), stream);
+  return rollout_dl(h, T, actions, reward_codes, true, dones, stream);
 }
 
 static int state_xfer(lmz_env *h, int32_t *io, int set, void *stream) {
@@ -1191,20 +1129,16 @@ static int state_xfer(lmz_env *h, int32_t *io, int set, void *stream) {
   if (!io) return fail(LMZ_ERR_INVALID, "state buffer is NULL");
   DeviceGuard guard(h->cfg.device);
   const int64_t n = h->cfg.num_envs;
-  const unsigned blocks = (unsigned)((n + 255) / 256);
+  const int64_t blocks = ceil_div(n, 256);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   unsigned int *errors = reinterpret_cast<unsigned int *>(h->stats + lmz::NUM_STATS);
-  if (h->cfg.variant == LMZ_V5)
-    lmz::lmz_state_v5_kernel<<<blocks, 256, 0, s>>>(n, h->state, h->goal_count, h->aux2, h->episode, io, set, errors);
-  else if (h->cfg.variant == LMZ_V2 || h->cfg.variant == LMZ_V4)
-    lmz::lmz_state_v2_kernel<<<blocks, 256, 0, s>>>(n, h->state, h->goal_count, h->episode, io, set, errors);
-  else if (h->cfg.variant == LMZ_V0)
-    lmz::lmz_state_kernel<lmz::V0><<<blocks, 256, 0, s>>>(n, h->state, h->goal_count, h->episode, io, set, h->blob, errors);
-  else
-    lmz::lmz_state_kernel<lmz::V3><<<blocks, 256, 0, s>>>(n, h->state, h->goal_count, h->episode, io, set, h->blob, errors);
-  LMZ_CUDA(cudaGetLastError());
-  h->launches += 1;
-  return LMZ_OK;
+  if (h->var->hier)
+    return launch(h, lmz::lmz_state_v5_kernel, blocks, 256, 0, s, n, h->state, h->goal_count, h->aux2, h->episode, io,
+                  set, errors);
+  if (h->var->foveal)
+    return launch(h, lmz::lmz_state_v2_kernel, blocks, 256, 0, s, n, h->state, h->goal_count, h->episode, io, set, errors);
+  return launch(h, h->cfg.variant == LMZ_V0 ? lmz::lmz_state_kernel<lmz::V0> : lmz::lmz_state_kernel<lmz::V3>, blocks,
+                256, 0, s, n, h->state, h->goal_count, h->episode, io, set, h->blob, errors);
 }
 
 int lmz_get_state(lmz_env *h, int32_t *out, void *stream) { return state_xfer(h, out, 0, stream); }
@@ -1216,8 +1150,8 @@ int lmz_set_state(lmz_env *h, const int32_t *in, void *stream) {
 static int state_xfer_dl(lmz_env *h, DLManagedTensor *t, int set, void *stream) {
   if (int rc = check_handle(h)) return rc;
   void *pt = nullptr;
-  Want w{"state", kDLInt, 32, 2, {h->cfg.num_envs, lmz_state_cols(h->cfg.variant), 0, 0}, false, 4};
-  if (int rc = check_dl(h, t, w, &pt, nullptr)) return rc;
+  const Want w{"state", kDLInt, 32, 2, {h->cfg.num_envs, h->var->state_cols, 0, 0}, 4};
+  if (int rc = check_dl(h, t, w, &pt)) return rc;
   return state_xfer(h, static_cast<int32_t *>(pt), set, stream);
 }
 int lmz_get_state_dl(lmz_env *h, DLManagedTensor *out, void *stream) { return state_xfer_dl(h, out, 0, stream); }
@@ -1228,27 +1162,22 @@ int lmz_set_state_dl(lmz_env *h, DLManagedTensor *in, void *stream) {
 
 static int visit_xfer(lmz_env *h, float *buf, int set, void *stream) {
   if (int rc = check_handle(h)) return rc;
-  if (h->cfg.variant != LMZ_V4 && h->cfg.variant != LMZ_V5)
-    return fail(LMZ_ERR_UNSUPPORTED, "only lmaze-v4/v5/v6 have a visit layer");
+  if (!h->var->has_visit) return fail(LMZ_ERR_UNSUPPORTED, "only lmaze-v4/v5/v6 have a visit layer");
   if (!buf) return fail(LMZ_ERR_INVALID, "visit buffer is NULL");
   DeviceGuard guard(h->cfg.device);
   // the handle keeps the layer as its history (lmz_v2.cuh, "visit layer"); it crosses the ABI as values
   const int64_t n = h->cfg.num_envs;
-  const bool v5 = h->cfg.variant == LMZ_V5;
-  const unsigned blocks = (unsigned)((n * 324 + 255) / 256);
-  lmz::lmz_visit_xfer_kernel<<<blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(
-      n, h->visit, h->hist, v5 ? h->state : h->goal_count, v5 ? 25 : 16, buf, set);
-  LMZ_CUDA(cudaGetLastError());
-  h->launches += 1;
-  return LMZ_OK;
+  const bool v5 = h->var->hier;
+  return launch(h, lmz::lmz_visit_xfer_kernel, ceil_div(n * 324, 256), 256, 0, static_cast<cudaStream_t>(stream), n,
+                h->visit, h->hist, v5 ? h->state : h->goal_count, v5 ? 25 : 16, buf, set);
 }
 int lmz_get_visit(lmz_env *h, float *out, void *stream) { return visit_xfer(h, out, 0, stream); }
 int lmz_set_visit(lmz_env *h, const float *in, void *stream) { return visit_xfer(h, const_cast<float *>(in), 1, stream); }
 static int visit_xfer_dl(lmz_env *h, DLManagedTensor *t, int set, void *stream) {
   if (int rc = check_handle(h)) return rc;
   void *pt = nullptr;
-  Want w{"visit", kDLFloat, 32, 3, {h->cfg.num_envs, 18, 18, 0}, false, 4};
-  if (int rc = check_dl(h, t, w, &pt, nullptr)) return rc;
+  const Want w{"visit", kDLFloat, 32, 3, {h->cfg.num_envs, 18, 18, 0}, 4};
+  if (int rc = check_dl(h, t, w, &pt)) return rc;
   return visit_xfer(h, static_cast<float *>(pt), set, stream);
 }
 int lmz_get_visit_dl(lmz_env *h, DLManagedTensor *out, void *stream) { return visit_xfer_dl(h, out, 0, stream); }
@@ -1258,7 +1187,7 @@ int lmz_set_visit_dl(lmz_env *h, DLManagedTensor *in, void *stream) { return vis
 int lmz_bind_local(lmz_env *h, float *loc_obs, float *local_reward, uint8_t *local_done, uint8_t *loc_err,
                    uint8_t *foveal_goal) {
   if (int rc = check_handle(h)) return rc;
-  if (h->cfg.variant != LMZ_V5) return fail(LMZ_ERR_UNSUPPORTED, "lmz_bind_local: only lmaze-v5/v6 have local outputs");
+  if (!h->var->hier) return fail(LMZ_ERR_UNSUPPORTED, "lmz_bind_local: only lmaze-v5/v6 have local outputs");
   if (!local_reward || !local_done) return fail(LMZ_ERR_INVALID, "local_reward/local_done must not be NULL");
   if ((reinterpret_cast<uintptr_t>(loc_obs) & 15u) != 0) return fail(LMZ_ERR_INVALID, "loc_obs must be 16-byte aligned");
   if ((reinterpret_cast<uintptr_t>(local_reward) & 3u) != 0)
@@ -1275,55 +1204,46 @@ int lmz_bind_local_dl(lmz_env *h, DLManagedTensor *loc_obs, DLManagedTensor *loc
   void *po = nullptr, *pr = nullptr, *pd = nullptr, *pe = nullptr, *pg = nullptr;
   if (loc_obs) {
     const int64_t side = h->cfg.obs_mode == LMZ_OBS_COMPACT ? 5 : lmz::V5::S;
-    Want w{"loc_obs", kDLFloat, 32, 4, {n, lmz::V5::CL, side, side}, false, 16};
-    if (int rc = check_dl(h, loc_obs, w, &po, nullptr)) return rc;
+    const Want w{"loc_obs", kDLFloat, 32, 4, {n, lmz::V5::CL, side, side}, 16};
+    if (int rc = check_dl(h, loc_obs, w, &po)) return rc;
   }
-  Want wr{"local_reward", kDLFloat, 32, 1, {n, 0, 0, 0}, false, 4};
-  if (int rc = check_dl(h, local_reward, wr, &pr, nullptr)) return rc;
-  Want wd{"local_done", kDLUInt, 8, 1, {n, 0, 0, 0}, false, 1};
-  if (int rc = check_dl(h, local_done, wd, &pd, nullptr)) return rc;
-  if (loc_err) {
-    Want w{"loc_err", kDLUInt, 8, 1, {n, 0, 0, 0}, false, 1};
-    if (int rc = check_dl(h, loc_err, w, &pe, nullptr)) return rc;
-  }
-  if (foveal_goal) {
-    Want w{"foveal_goal", kDLUInt, 8, 1, {n, 0, 0, 0}, false, 1};
-    if (int rc = check_dl(h, foveal_goal, w, &pg, nullptr)) return rc;
-  }
+  if (int rc = check_dl(h, local_reward, per_env(h, "local_reward", kDLFloat, 32), &pr)) return rc;
+  if (int rc = check_dl(h, local_done, per_env(h, "local_done", kDLUInt, 8), &pd)) return rc;
+  if (loc_err)
+    if (int rc = check_dl(h, loc_err, per_env(h, "loc_err", kDLUInt, 8), &pe)) return rc;
+  if (foveal_goal)
+    if (int rc = check_dl(h, foveal_goal, per_env(h, "foveal_goal", kDLUInt, 8), &pg)) return rc;
   return lmz_bind_local(h, static_cast<float *>(po), static_cast<float *>(pr), static_cast<uint8_t *>(pd),
                         static_cast<uint8_t *>(pe), static_cast<uint8_t *>(pg));
 }
 
-int lmz_planner_step(lmz_env *h, const void *goals, int32_t goal_dtype, const uint8_t *mask, void *stream) {
+// plannerStep on the envs of `mask` (null: all), or with auto_mask on the envs whose foveal goal is done
+static int planner_step(const char *fn, lmz_env *h, const void *goals, int32_t goal_dtype, const uint8_t *mask,
+                        bool auto_mask, void *stream) {
   if (int rc = check_handle(h)) return rc;
-  if (h->cfg.variant != LMZ_V5) return fail(LMZ_ERR_UNSUPPORTED, "lmz_planner_step: only lmaze-v5/v6 have a planner level");
+  if (!h->var->hier) return fail(LMZ_ERR_UNSUPPORTED, "%s: only lmaze-v5/v6 have a planner level", fn);
   if (int rc = check_bound(h)) return rc;
   if (!goals) return fail(LMZ_ERR_INVALID, "goals is NULL");
-  if (goal_dtype < LMZ_ACT_U8 || goal_dtype > LMZ_ACT_I64) return fail(LMZ_ERR_INVALID, "unknown goal dtype %d", goal_dtype);
+  if (int rc = check_action_dtype(goal_dtype, "goal dtype")) return rc;
   DeviceGuard guard(h->cfg.device);
   lmz::KParams p = base_params(h);
-  p.mode = lmz::MODE_PLANNER; p.actions = goals; p.action_dtype = goal_dtype; p.mask = mask;
+  p.mode = lmz::MODE_PLANNER; p.actions = goals; p.action_dtype = goal_dtype; p.mask = mask; p.auto_mask = auto_mask;
   return launch_env(h, p, static_cast<cudaStream_t>(stream));
 }
 
+int lmz_planner_step(lmz_env *h, const void *goals, int32_t goal_dtype, const uint8_t *mask, void *stream) {
+  return planner_step("lmz_planner_step", h, goals, goal_dtype, mask, false, stream);
+}
+
 int lmz_planner_step_auto(lmz_env *h, const void *goals, int32_t goal_dtype, void *stream) {
-  if (int rc = check_handle(h)) return rc;
-  if (h->cfg.variant != LMZ_V5) return fail(LMZ_ERR_UNSUPPORTED, "lmz_planner_step_auto: only lmaze-v5/v6 have a planner level");
-  if (int rc = check_bound(h)) return rc;
-  if (!goals) return fail(LMZ_ERR_INVALID, "goals is NULL");
-  if (goal_dtype < LMZ_ACT_U8 || goal_dtype > LMZ_ACT_I64) return fail(LMZ_ERR_INVALID, "unknown goal dtype %d", goal_dtype);
-  DeviceGuard guard(h->cfg.device);
-  lmz::KParams p = base_params(h);
-  p.mode = lmz::MODE_PLANNER; p.actions = goals; p.action_dtype = goal_dtype; p.auto_mask = 1;
-  return launch_env(h, p, static_cast<cudaStream_t>(stream));
+  return planner_step("lmz_planner_step_auto", h, goals, goal_dtype, nullptr, true, stream);
 }
 
 int lmz_planner_step_auto_dl(lmz_env *h, DLManagedTensor *goals, void *stream) {
   if (int rc = check_handle(h)) return rc;
   void *pg = nullptr;
   int ad = 0;
-  Want wg{"goals", 255, 0, 1, {h->cfg.num_envs, 0, 0, 0}, false, 1};
-  if (int rc = check_dl(h, goals, wg, &pg, &ad)) return rc;
+  if (int rc = check_dl(h, goals, per_env(h, "goals", ANY_INT), &pg, &ad)) return rc;
   return lmz_planner_step_auto(h, pg, ad, stream);
 }
 
@@ -1331,17 +1251,17 @@ int lmz_hier_step_host(lmz_env *h, const void *goals_host, const void *actions_h
                        float *global_reward_host, float *local_reward_host, uint8_t *global_done_host,
                        uint8_t *local_done_host, void *stream) {
   if (int rc = check_handle(h)) return rc;
-  if (h->cfg.variant != LMZ_V5) return fail(LMZ_ERR_UNSUPPORTED, "lmz_hier_step_host: only lmaze-v5/v6");
+  if (!h->var->hier) return fail(LMZ_ERR_UNSUPPORTED, "lmz_hier_step_host: only lmaze-v5/v6");
   if (int rc = check_bound(h)) return rc;
   if (!h->local_bound) return fail(LMZ_ERR_STATE, "local outputs not bound: call lmz_bind_local first");
   if (!goals_host || !actions_host || !global_reward_host || !local_reward_host || !global_done_host || !local_done_host)
     return fail(LMZ_ERR_INVALID, "host buffers must not be NULL");
-  if (dtype < LMZ_ACT_U8 || dtype > LMZ_ACT_I64) return fail(LMZ_ERR_INVALID, "unknown dtype %d", dtype);
+  if (int rc = check_action_dtype(dtype, "dtype")) return rc;
   DeviceGuard guard(h->cfg.device);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const size_t n = (size_t)h->cfg.num_envs;
   if (!h->act_stage) LMZ_CUDA(cudaMalloc(&h->act_stage, n * 16));       // goals | actions
-  const size_t esz = dtype == LMZ_ACT_U8 ? 1 : dtype == LMZ_ACT_I32 ? 4 : 8;
+  const size_t esz = action_bytes(dtype);
   unsigned char *stage = static_cast<unsigned char *>(h->act_stage);
   LMZ_CUDA(cudaMemcpyAsync(stage, goals_host, n * esz, cudaMemcpyHostToDevice, s));
   LMZ_CUDA(cudaMemcpyAsync(stage + n * 8, actions_host, n * esz, cudaMemcpyHostToDevice, s));
@@ -1358,13 +1278,14 @@ int lmz_hier_step_host(lmz_env *h, const void *goals_host, const void *actions_h
 int lmz_hier_rollout(lmz_env *h, int32_t T, const void *goals, const void *actions, int32_t dtype, float *global_rewards,
                      float *local_rewards, uint8_t *global_dones, uint8_t *local_dones, void *stream) {
   if (int rc = check_handle(h)) return rc;
-  if (h->cfg.variant != LMZ_V5) return fail(LMZ_ERR_UNSUPPORTED, "lmz_hier_rollout: only lmaze-v5/v6");
+  if (!h->var->hier) return fail(LMZ_ERR_UNSUPPORTED, "lmz_hier_rollout: only lmaze-v5/v6");
   if (T < 1) return fail(LMZ_ERR_INVALID, "T must be >= 1 (got %d)", T);
   if (!global_rewards || !local_rewards || !global_dones || !local_dones)
     return fail(LMZ_ERR_INVALID, "reward / done buffers must not be NULL");
   if ((goals == nullptr) != (actions == nullptr))
     return fail(LMZ_ERR_INVALID, "goals and actions must both be given, or both NULL (device-side random goals and actions)");
-  if (actions && (dtype < LMZ_ACT_U8 || dtype > LMZ_ACT_I64)) return fail(LMZ_ERR_INVALID, "unknown dtype %d", dtype);
+  if (actions)
+    if (int rc = check_action_dtype(dtype, "dtype")) return rc;
   DeviceGuard guard(h->cfg.device);
   lmz::KParams p = base_params(h);
   p.mode = lmz::MODE_STEP; p.actions = actions; p.goals = goals; p.action_dtype = dtype;
@@ -1379,58 +1300,42 @@ int lmz_hier_rollout_dl(lmz_env *h, int32_t T, DLManagedTensor *goals, DLManaged
                         DLManagedTensor *local_rewards, DLManagedTensor *global_dones, DLManagedTensor *local_dones,
                         void *stream) {
   if (int rc = check_handle(h)) return rc;
-  const int64_t n = h->cfg.num_envs;
   void *pg = nullptr, *pa = nullptr, *pr = nullptr, *pr2 = nullptr, *pd = nullptr, *pd2 = nullptr;
   int ad = 0, gd = 0;
-  if (actions) {
-    Want wa{"actions", 255, 0, 2, {T, n, 0, 0}, false, 1};
-    if (int rc = check_dl(h, actions, wa, &pa, &ad)) return rc;
-  }
+  if (actions)
+    if (int rc = check_dl(h, actions, per_step(h, "actions", T, ANY_INT), &pa, &ad)) return rc;
   if (goals) {
-    Want wg{"goals", 255, 0, 2, {T, n, 0, 0}, false, 1};
-    if (int rc = check_dl(h, goals, wg, &pg, &gd)) return rc;
+    if (int rc = check_dl(h, goals, per_step(h, "goals", T, ANY_INT), &pg, &gd)) return rc;
     if (actions && gd != ad) return fail(LMZ_ERR_INVALID, "goals and actions must have the same dtype");
   }
-  Want wr{"global_rewards", kDLFloat, 32, 2, {T, n, 0, 0}, false, 4};
-  if (int rc = check_dl(h, global_rewards, wr, &pr, nullptr)) return rc;
-  Want wr2{"local_rewards", kDLFloat, 32, 2, {T, n, 0, 0}, false, 4};
-  if (int rc = check_dl(h, local_rewards, wr2, &pr2, nullptr)) return rc;
-  Want wd{"global_dones", kDLUInt, 8, 2, {T, n, 0, 0}, false, 1};
-  if (int rc = check_dl(h, global_dones, wd, &pd, nullptr)) return rc;
-  Want wd2{"local_dones", kDLUInt, 8, 2, {T, n, 0, 0}, false, 1};
-  if (int rc = check_dl(h, local_dones, wd2, &pd2, nullptr)) return rc;
+  if (int rc = check_dl(h, global_rewards, per_step(h, "global_rewards", T, kDLFloat, 32), &pr)) return rc;
+  if (int rc = check_dl(h, local_rewards, per_step(h, "local_rewards", T, kDLFloat, 32), &pr2)) return rc;
+  if (int rc = check_dl(h, global_dones, per_step(h, "global_dones", T, kDLUInt, 8), &pd)) return rc;
+  if (int rc = check_dl(h, local_dones, per_step(h, "local_dones", T, kDLUInt, 8), &pd2)) return rc;
   return lmz_hier_rollout(h, T, pg, pa, ad, static_cast<float *>(pr), static_cast<float *>(pr2), static_cast<uint8_t *>(pd),
                           static_cast<uint8_t *>(pd2), stream);
 }
 
 int lmz_planner_step_dl(lmz_env *h, DLManagedTensor *goals, DLManagedTensor *mask, void *stream) {
   if (int rc = check_handle(h)) return rc;
-  const int64_t n = h->cfg.num_envs;
   void *pg = nullptr, *pm = nullptr;
   int ad = 0;
-  Want wg{"goals", 255, 0, 1, {n, 0, 0, 0}, false, 1};
-  if (int rc = check_dl(h, goals, wg, &pg, &ad)) return rc;
-  if (mask) {
-    Want w{"mask", kDLUInt, 8, 1, {n, 0, 0, 0}, false, 1};
-    if (int rc = check_dl(h, mask, w, &pm, nullptr)) return rc;
-  }
+  if (int rc = check_dl(h, goals, per_env(h, "goals", ANY_INT), &pg, &ad)) return rc;
+  if (mask)
+    if (int rc = check_dl(h, mask, per_env(h, "mask", kDLUInt, 8), &pm)) return rc;
   return lmz_planner_step(h, pg, ad, static_cast<const uint8_t *>(pm), stream);
 }
 
 int lmz_safe_goal(lmz_env *h, const int64_t *draws, int32_t n_draws, uint8_t *goals_out, int32_t *used_out, void *stream) {
   if (int rc = check_handle(h)) return rc;
-  if (h->cfg.variant != LMZ_V5) return fail(LMZ_ERR_UNSUPPORTED, "lmz_safe_goal: only lmaze-v6 (variant 5) has safeFovealGoal");
+  if (!h->var->hier) return fail(LMZ_ERR_UNSUPPORTED, "lmz_safe_goal: only lmaze-v6 (variant 5) has safeFovealGoal");
   if (!goals_out) return fail(LMZ_ERR_INVALID, "goals_out is NULL");
   if (draws && n_draws < 1) return fail(LMZ_ERR_INVALID, "n_draws must be >= 1 when draws are given");
   DeviceGuard guard(h->cfg.device);
   const int64_t n = h->cfg.num_envs;
-  const unsigned blocks = (unsigned)((n + 255) / 256);
-  lmz::lmz_safe_goal_kernel<lmz::V5><<<blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(
-      n, h->state, h->aux2, h->episode, h->blob, reinterpret_cast<const long long *>(draws), n_draws, goals_out, used_out,
-      h->cfg.seed, (uint64_t)h->cfg.env_id0);
-  LMZ_CUDA(cudaGetLastError());
-  h->launches += 1;
-  return LMZ_OK;
+  return launch(h, lmz::lmz_safe_goal_kernel<lmz::V5>, ceil_div(n, 256), 256, 0, static_cast<cudaStream_t>(stream), n,
+                h->state, h->aux2, h->episode, h->blob, reinterpret_cast<const long long *>(draws), n_draws, goals_out,
+                used_out, h->cfg.seed, (uint64_t)h->cfg.env_id0);
 }
 
 int lmz_safe_goal_dl(lmz_env *h, DLManagedTensor *draws, DLManagedTensor *goals_out, DLManagedTensor *used_out,
@@ -1442,15 +1347,12 @@ int lmz_safe_goal_dl(lmz_env *h, DLManagedTensor *draws, DLManagedTensor *goals_
   if (draws) {
     if (draws->dl_tensor.ndim != 2) return fail(LMZ_ERR_INVALID, "draws: ndim %d, want 2", draws->dl_tensor.ndim);
     nd = (int32_t)draws->dl_tensor.shape[1];
-    Want w{"draws", kDLInt, 64, 2, {n, nd, 0, 0}, false, 8};
-    if (int rc = check_dl(h, draws, w, &pd, nullptr)) return rc;
+    const Want w{"draws", kDLInt, 64, 2, {n, nd, 0, 0}, 8};
+    if (int rc = check_dl(h, draws, w, &pd)) return rc;
   }
-  Want wg{"goals_out", kDLUInt, 8, 1, {n, 0, 0, 0}, false, 1};
-  if (int rc = check_dl(h, goals_out, wg, &pg, nullptr)) return rc;
-  if (used_out) {
-    Want w{"used_out", kDLInt, 32, 1, {n, 0, 0, 0}, false, 4};
-    if (int rc = check_dl(h, used_out, w, &pu, nullptr)) return rc;
-  }
+  if (int rc = check_dl(h, goals_out, per_env(h, "goals_out", kDLUInt, 8), &pg)) return rc;
+  if (used_out)
+    if (int rc = check_dl(h, used_out, per_env(h, "used_out", kDLInt, 32), &pu)) return rc;
   return lmz_safe_goal(h, static_cast<const int64_t *>(pd), nd, static_cast<uint8_t *>(pg), static_cast<int32_t *>(pu), stream);
 }
 
