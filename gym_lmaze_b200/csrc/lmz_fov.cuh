@@ -300,11 +300,7 @@ __global__ void __launch_bounds__(THREADS) lmz_env_fov_kernel(const KParams p) {
     if (tl < tiles && e < p.n) pre_next = fov_preload<W>(p, e);
     tl_next = tl;
   };
-  auto grab = [&]() {
-    int64_t tl = 0;
-    if (lane == 0) tl = p.tile_begin + grab_tile(p.work);
-    return __shfl_sync(0xffffffffu, tl, 0);
-  };
+  auto grab = [&]() { return warp_grab(p, lane, 1); };
   auto produce = [&](int buf) {              // warp 0 only
     const int64_t tl = tl_next;
     const FovPre pre = pre_next;
@@ -312,8 +308,7 @@ __global__ void __launch_bounds__(THREADS) lmz_env_fov_kernel(const KParams p) {
     const int64_t e = tl * 32 + lane;
     const bool valid = tl < tiles && e < p.n;
     FovLane<W::NBIT> v;
-    v.o.st = 0; v.o.st_old = 0; v.o.render = false; v.o.done = false; v.o.cls = -1; v.o.eplen = 0; v.info = 0;
-    v.vinfo = 0; v.rfov = false; v.rloc = false;
+    v.o = LaneOut::blank(); v.info = 0; v.vinfo = 0; v.rfov = false; v.rloc = false;
     if (valid) v = fov_lane(static_cast<const W *>(nullptr), p, e, t, smem, pre);
     if (p.mode == MODE_STEP) ws.add(valid, v.o);
     float *mv = vals + (buf * 32 + lane) * W::VALS;
@@ -329,12 +324,7 @@ __global__ void __launch_bounds__(THREADS) lmz_env_fov_kernel(const KParams p) {
 #endif
     if (valid && (v.rfov || v.rloc)) {       // 25-bit planes -> float planes (lane stride VALS is odd: no bank conflicts)
 #pragma unroll
-      for (int b = 0; b < W::NBIT; ++b) {
-        const uint32_t m = v.mask[b];
-        float *pl = mv + W::bit_slot(b) * 25;
-#pragma unroll
-        for (int c = 0; c < 25; ++c) pl[c] = ((m >> c) & 1u) ? 1.0f : 0.0f;
-      }
+      for (int b = 0; b < W::NBIT; ++b) expand_plane(v.mask[b], mv + W::bit_slot(b) * 25);
     }
     const unsigned ff = __ballot_sync(0xffffffffu, valid && v.rfov);
     const unsigned fl = __ballot_sync(0xffffffffu, valid && v.rloc);
@@ -469,11 +459,7 @@ __global__ void __launch_bounds__(THREADS) lmz_fov_small_kernel(const KParams p)
   const int64_t tiles = p.tile_end;
   const bool need_visit = W::NVIS > 0 && p.mode != MODE_PLANNER;
   WarpStats ws;
-  auto grab = [&]() {
-    int64_t tl = 0;
-    if (lane == 0) tl = p.tile_begin + grab_tile(p.work);
-    return __shfl_sync(0xffffffffu, tl, 0);
-  };
+  auto grab = [&]() { return warp_grab(p, lane, 1); };
   // copy of the first `bytes` of the warp's smem tile to global (both 16-byte aligned): ONE shared -> global bulk
   // copy issued by lane 0 -- the TMA engine moves the tile's rows as one contiguous run, no LSU store is issued
   auto copy_out = [&](float *dst, uint32_t bytes) {
@@ -493,11 +479,7 @@ __global__ void __launch_bounds__(THREADS) lmz_fov_small_kernel(const KParams p)
       if (valid && v.rfov) {                                     // 25-bit planes -> float planes (stride PER is odd: no bank conflicts)
 #pragma unroll
         for (int b = 0; b < W::NBIT; ++b) {
-          if (W::bit_slot(b) >= W::C) continue;                  // (v5: the local obs's planes, below)
-          const uint32_t m = v.mask[b];
-          float *pl = mine + W::bit_slot(b) * 25;
-#pragma unroll
-          for (int c = 0; c < 25; ++c) pl[c] = ((m >> c) & 1u) ? 1.0f : 0.0f;
+          if (W::bit_slot(b) < W::C) expand_plane(v.mask[b], mine + W::bit_slot(b) * 25);   // (v5: local planes below)
         }
       }
       float *dst = reinterpret_cast<float *>(p.obs) + row0 * (int64_t)PER;
@@ -517,11 +499,8 @@ __global__ void __launch_bounds__(THREADS) lmz_fov_small_kernel(const KParams p)
       float *minel = rows + lane * PERL;
       if (valid && v.rloc) {
 #pragma unroll
-        for (int c4 = 0; c4 < 4; ++c4) {
-          const uint32_t m = v.mask[W::NBIT > 8 ? (c4 == 0 ? 7 : c4 == 1 ? 5 : c4 == 2 ? 6 : 8) : 0];
-#pragma unroll
-          for (int c = 0; c < 25; ++c) minel[c4 * 25 + c] = ((m >> c) & 1u) ? 1.0f : 0.0f;
-        }
+        for (int c4 = 0; c4 < 4; ++c4)
+          expand_plane(v.mask[W::NBIT > 8 ? (c4 == 0 ? 7 : c4 == 1 ? 5 : c4 == 2 ? 6 : 8) : 0], minel + c4 * 25);
       }
       float *dst = reinterpret_cast<float *>(p.obs2) + row0 * (int64_t)PERL;
       if (fl == 0xffffffffu) copy_out(dst, 32 * PERL * 4);

@@ -150,15 +150,14 @@ template <class W, int THREADS>
 __global__ void __launch_bounds__(THREADS) lmz_fov_rollout_kernel(const KParams p) {
   extern __shared__ __align__(128) unsigned char smem[];         // the per-maze tables (blob from ROWBITS_OFF on) + the history rows
   __shared__ unsigned long long blk_stats[NUM_STATS];
-  constexpr uint32_t STAGE_OFF = W::ROWBITS_OFF;
-  constexpr uint32_t TAB_BYTES = (W::BLOB_BYTES - STAGE_OFF + 15u) & ~15u;
-  for (uint32_t i = threadIdx.x; i < (W::BLOB_BYTES - STAGE_OFF) / 4; i += THREADS)
-    reinterpret_cast<uint32_t *>(smem)[i] = reinterpret_cast<const uint32_t *>(p.blob + STAGE_OFF)[i];
+  using FS = FovSmall<W>;
+  for (uint32_t i = threadIdx.x; i < (W::BLOB_BYTES - FS::STAGE_OFF) / 4; i += THREADS)
+    reinterpret_cast<uint32_t *>(smem)[i] = reinterpret_cast<const uint32_t *>(p.blob + FS::STAGE_OFF)[i];
   if (threadIdx.x < NUM_STATS) blk_stats[threadIdx.x] = 0;
   __syncthreads();
-  const unsigned char *sb = smem - STAGE_OFF;
+  const unsigned char *sb = smem - FS::STAGE_OFF;
   const FovTables<W> t(sb);
-  uint8_t *hrow = smem + TAB_BYTES + threadIdx.x * HIST_STRIDE;  // this thread's visit history (v4 / v5)
+  uint8_t *hrow = smem + FS::TAB_BYTES + threadIdx.x * HIST_STRIDE;  // this thread's visit history (v4 / v5)
   RolloutCounters c;
   for (int64_t e = (int64_t)blockIdx.x * THREADS + threadIdx.x; e < p.n; e += (int64_t)gridDim.x * THREADS) {
     if (W::NVIS > 0) {                                           // history in: 64 contiguous bytes per env

@@ -33,7 +33,7 @@
 
 namespace lmz {
 
-enum : int { MODE_STEP = 0, MODE_RESET = 1, MODE_RENDER = 2 };
+enum : int { MODE_STEP = 0, MODE_RESET = 1, MODE_RENDER = 2, MODE_PLANNER = 3 };
 enum : int { ACT_U8 = 0, ACT_I32 = 1, ACT_I64 = 2 };
 enum : int { RENDER_TMA = 0, RENDER_ST128 = 1, RENDER_INCREMENTAL = 2 };
 enum : int { OBS_FULL = 0, OBS_COMPACT = 1, OBS_BITS = 2 };
@@ -300,15 +300,20 @@ struct LaneOut {
   bool done;
   int cls;            // branch taken by the transition (-1: no step)
   uint32_t eplen;     // stepCount of an episode that finished in this call
+  // what a lane without an env (past the end of the batch) reports
+  __device__ static __forceinline__ LaneOut blank() {
+    LaneOut o;
+    o.st = 0; o.st_old = 0; o.render = false; o.done = false; o.cls = -1; o.eplen = 0;
+    return o;
+  }
 };
 
-// `st_old` and `a` are the env's packed state and action, loaded by the caller (so that a kernel can have
-// the loads of several tiles in flight before it needs any of them).
+// One env of a v0 / v3 tile kernel.  `st_old` and `a` are the env's packed state and action, loaded by the caller (so
+// that a kernel can have the loads of several tiles in flight before it needs any of them).
 template <class V>
-__device__ __forceinline__ LaneOut env_lane_pre(const KParams &p, int64_t e, uint32_t st_old, long long a,
-                                                const uint8_t *cls, const uint16_t *cand) {
-  LaneOut o;
-  o.render = false; o.done = false; o.cls = -1; o.eplen = 0;
+__device__ __forceinline__ LaneOut tile_lane(const KParams &p, int64_t e, uint32_t st_old, long long a,
+                                             const uint8_t *cls, const uint16_t *cand) {
+  LaneOut o = LaneOut::blank();
   o.st_old = st_old;
   EnvRegs r = V::unpack(o.st_old);
   bool reset_now = false;
@@ -335,14 +340,8 @@ __device__ __forceinline__ LaneOut env_lane_pre(const KParams &p, int64_t e, uin
   }
   o.st = V::pack(r);
   if (p.mode != MODE_RENDER) p.state[e] = o.st;
+  o.render = o.render && p.obs != nullptr && e >= p.win_lo && e < p.win_lo + p.win_n;   // render window
   return o;
-}
-
-template <class V>
-__device__ __forceinline__ LaneOut env_lane(const KParams &p, int64_t e, const uint8_t *cls, const uint16_t *cand) {
-  const uint32_t st_old = p.state[e];
-  const long long a = (p.mode == MODE_STEP) ? load_action(p.actions, p.action_dtype, e) : 0;
-  return env_lane_pre<V>(p, e, st_old, a, cls, cand);
 }
 
 // Latency-tolerant tile pipeline of the small-observation kernels (compact, incremental, transition-only).
@@ -356,9 +355,6 @@ struct TileGroup {
   uint32_t st[G];
   int act[G];           // action, clamped to 0..255 (anything outside 0..3 is the same no-op)
 };
-__device__ __forceinline__ int64_t grab_tiles(unsigned long long *work, int count) {
-  return (int64_t)atomicAdd(&work[0], (unsigned long long)count);
-}
 template <int G>
 __device__ __forceinline__ void preload_group(const KParams &p, int64_t tile0, int lane, int64_t tiles, TileGroup<G> &g) {
 #pragma unroll
@@ -374,20 +370,6 @@ __device__ __forceinline__ void preload_group(const KParams &p, int64_t tile0, i
     }
   }
 }
-template <class V>
-__device__ __forceinline__ LaneOut tile_lane_pre(const KParams &p, int64_t tile, int lane, int64_t tiles, uint32_t st,
-                                                 int act, const uint8_t *cls, const uint16_t *cand, bool &valid) {
-  LaneOut o;
-  o.st = 0; o.st_old = 0; o.render = false; o.done = false; o.cls = -1; o.eplen = 0;
-  const int64_t e = tile * 32 + lane;
-  valid = tile < tiles && e < p.n;
-  if (valid) {
-    o = env_lane_pre<V>(p, e, st, (long long)act, cls, cand);
-    o.render = o.render && p.obs != nullptr && e >= p.win_lo && e < p.win_lo + p.win_n;   // render window
-  }
-  return o;
-}
-
 // Episode statistics of one warp: a ballot + popc per counter (the counts are warp-uniform
 // registers), a shuffle reduction for the episode-length sum, one atomicAdd per counter at the end.
 struct WarpStats {
@@ -439,8 +421,14 @@ __device__ __forceinline__ void stage_blob(unsigned char *smem, uint64_t *bar, c
 // 0.02 ms and the same copies reach 7.5 TB/s).  So tiles of 32 consecutive envs are grabbed from
 // work[0]; work[1] counts finished grabbers and the last one re-arms both for the next launch
 // (self-contained, so the launch is also safe to replay from a CUDA graph).
-__device__ __forceinline__ int64_t grab_tile(unsigned long long *work) {
-  return (int64_t)atomicAdd(&work[0], 1ull);
+__device__ __forceinline__ int64_t grab_tiles(unsigned long long *work, int count) {
+  return (int64_t)atomicAdd(&work[0], (unsigned long long)count);
+}
+// Lane 0 grabs `count` consecutive tiles for the whole warp; every lane gets the first one's index.
+__device__ __forceinline__ int64_t warp_grab(const KParams &p, int lane, int count) {
+  int64_t t = 0;
+  if (lane == 0) t = p.tile_begin + grab_tiles(p.work, count);
+  return __shfl_sync(0xffffffffu, t, 0);
 }
 // The same grab as inline PTX: the compiler aggregates a result-returning atomicAdd across the warp and broadcasts the
 // result with a shuffle RIGHT BEHIND the atomic, which makes every grab synchronous; this form lets the result be
@@ -453,20 +441,6 @@ __device__ __forceinline__ int64_t grab_tile_async(unsigned long long *work) {
 __device__ __forceinline__ void finish_grabber(unsigned long long *work, unsigned long long grabbers) {
   __threadfence();
   if (atomicAdd(&work[1], 1ull) == grabbers - 1) { work[0] = 0; work[1] = 0; }
-}
-
-template <class V>
-__device__ __forceinline__ LaneOut tile_lane(const KParams &p, int64_t tile, int lane, int64_t tiles,
-                                             const uint8_t *cls, const uint16_t *cand, bool &valid) {
-  LaneOut o;
-  o.st = 0; o.st_old = 0; o.render = false; o.done = false; o.cls = -1; o.eplen = 0;
-  const int64_t e = tile * 32 + lane;
-  valid = tile < tiles && e < p.n;
-  if (valid) {
-    o = env_lane<V>(p, e, cls, cand);
-    o.render = o.render && p.obs != nullptr && e >= p.win_lo && e < p.win_lo + p.win_n;   // render window
-  }
-  return o;
 }
 
 // ---- render path 1: the TMA engine writes the observation ------------------------------------
@@ -488,20 +462,25 @@ __global__ void __launch_bounds__(THREADS, 1) lmz_env_tma_kernel(const KParams p
   const int64_t tiles = p.tile_end;
   WarpStats ws;
 
-  auto next_tile = [&]() {
-    int64_t t = 0;
-    if (lane == 0) t = p.tile_begin + grab_tile(p.work);
-    return __shfl_sync(0xffffffffu, t, 0);
+  auto step_tile = [&](int64_t tl, bool &valid) {        // this lane's env of tile `tl`: load, step, count
+    const int64_t e = tl * 32 + lane;
+    valid = tl < tiles && e < p.n;
+    LaneOut o = LaneOut::blank();
+    if (valid) {
+      const uint32_t st = p.state[e];
+      const long long a = (p.mode == MODE_STEP) ? load_action(p.actions, p.action_dtype, e) : 0;
+      o = tile_lane<V>(p, e, st, a, cls, cand);
+    }
+    if (p.mode == MODE_STEP) ws.add(valid, o);
+    return o;
   };
-  int64_t tile = next_tile();
+  int64_t tile = warp_grab(p, lane, 1);
   bool valid;
-  LaneOut o = tile_lane<V>(p, tile, lane, tiles, cls, cand, valid);
-  if (p.mode == MODE_STEP) ws.add(valid, o);
+  LaneOut o = step_tile(tile, valid);
   while (tile < tiles) {
-    const int64_t ntile = next_tile();
+    const int64_t ntile = warp_grab(p, lane, 1);
     bool nvalid;
-    const LaneOut no = tile_lane<V>(p, ntile, lane, tiles, cls, cand, nvalid);
-    if (p.mode == MODE_STEP) ws.add(nvalid, no);
+    const LaneOut no = step_tile(ntile, nvalid);
     // ---- observation render (lmaze_env.py:208-234): the env's image is NSEG blob segments
     unsigned rmask = __ballot_sync(0xffffffffu, valid && o.render);
     while (rmask) {
@@ -555,11 +534,14 @@ __global__ void __launch_bounds__(THREADS, 1) lmz_env_st_kernel(const KParams p)
   WarpStats ws;
 
   auto produce = [&](int buf) {                          // warp 0 only
-    int64_t t = 0;
-    if (lane == 0) t = p.tile_begin + grab_tile(p.work);
-    t = __shfl_sync(0xffffffffu, t, 0);
-    bool valid;
-    const LaneOut o = tile_lane<V>(p, t, lane, tiles, cls, cand, valid);
+    const int64_t t = warp_grab(p, lane, 1), e = t * 32 + lane;
+    const bool valid = t < tiles && e < p.n;
+    LaneOut o = LaneOut::blank();
+    if (valid) {
+      const uint32_t st = p.state[e];
+      const long long a = (p.mode == MODE_STEP) ? load_action(p.actions, p.action_dtype, e) : 0;
+      o = tile_lane<V>(p, e, st, a, cls, cand);
+    }
     if (p.mode == MODE_STEP) ws.add(valid, o);
     s_st[buf][lane] = (valid && o.render) ? o.st : NO_RENDER;
     if (lane == 0) s_tile[buf] = t;
@@ -634,22 +616,19 @@ __global__ void __launch_bounds__(THREADS) lmz_env_compact_kernel(const KParams 
   WarpStats ws;
   // persistent warps; groups of G tiles handed out dynamically, two groups ahead (see TileGroup)
   constexpr int G = (V::ID == 0) ? LMZ_G_COMPACT_V0 : LMZ_G_COMPACT_V3;
-  auto next_group = [&]() {
-    int64_t t = 0;
-    if (lane == 0) t = p.tile_begin + grab_tiles(p.work, G);
-    return __shfl_sync(0xffffffffu, t, 0);
-  };
-  int64_t t0 = next_group(), t1 = next_group();
+  int64_t t0 = warp_grab(p, lane, G), t1 = warp_grab(p, lane, G);
   TileGroup<G> pre;
   preload_group<G>(p, t0, lane, tiles, pre);
   while (t0 < tiles) {
-    const int64_t t2 = next_group();                 // needed two iterations from now
+    const int64_t t2 = warp_grab(p, lane, G);                 // needed two iterations from now
     uint32_t st[G];
     unsigned rmask[G];
 #pragma unroll
     for (int k = 0; k < G; ++k) {                    // transitions of the group loaded one iteration ago
-      bool valid;
-      const LaneOut o = tile_lane_pre<V>(p, t0 + k, lane, tiles, pre.st[k], pre.act[k], cls, cand, valid);
+      const int64_t e = (t0 + k) * 32 + lane;
+      const bool valid = t0 + k < tiles && e < p.n;
+      LaneOut o = LaneOut::blank();
+      if (valid) o = tile_lane<V>(p, e, pre.st[k], pre.act[k], cls, cand);
       if (p.mode == MODE_STEP) ws.add(valid, o);
       st[k] = o.st;
       rmask[k] = __ballot_sync(0xffffffffu, valid && o.render);
@@ -732,11 +711,6 @@ __global__ void __launch_bounds__(THREADS) lmz_env_incr_kernel(const KParams p) 
   const uint16_t *cand = reinterpret_cast<const uint16_t *>(tab + (V::CAND_OFF - V::TABLES_OFF));
   const int64_t tiles = p.tile_end;
   WarpStats ws;
-  auto next_tile = [&]() {
-    int64_t t = 0;
-    if (lane == 0) t = p.tile_begin + grab_tile(p.work);
-    return __shfl_sync(0xffffffffu, t, 0);
-  };
   // block b of a packed state: channel and top-left element
   auto block_of = [](uint32_t st, int b, int &ch, int &row, int &col) {
     const EnvRegs r = V::unpack(st);
@@ -745,22 +719,19 @@ __global__ void __launch_bounds__(THREADS) lmz_env_incr_kernel(const KParams p) 
     else { ch = 2; row = r.gx * V::E; col = r.gy * V::E; }
   };
   constexpr int G = LMZ_G_INCR;
-  auto next_group = [&]() {
-    int64_t t = 0;
-    if (lane == 0) t = p.tile_begin + grab_tiles(p.work, G);
-    return __shfl_sync(0xffffffffu, t, 0);
-  };
-  int64_t t0 = next_group(), t1 = next_group();
+  int64_t t0 = warp_grab(p, lane, G), t1 = warp_grab(p, lane, G);
   TileGroup<G> pre;
   preload_group<G>(p, t0, lane, tiles, pre);
   while (t0 < tiles) {
-    const int64_t t2 = next_group();
+    const int64_t t2 = warp_grab(p, lane, G);
     uint32_t st_new[G], st_old[G];
     unsigned mmask[G];
 #pragma unroll
     for (int k = 0; k < G; ++k) {
-      bool valid;
-      const LaneOut o = tile_lane_pre<V>(p, t0 + k, lane, tiles, pre.st[k], pre.act[k], cls, cand, valid);
+      const int64_t e = (t0 + k) * 32 + lane;
+      const bool valid = t0 + k < tiles && e < p.n;
+      LaneOut o = LaneOut::blank();
+      if (valid) o = tile_lane<V>(p, e, pre.st[k], pre.act[k], cls, cand);
       ws.add(valid, o);
       // which envs of the tile have a block that moved?
       bool moved = false;

@@ -141,6 +141,12 @@ __device__ __forceinline__ uint4 f4_pick(uint32_t en, const float *gv) {
   return make_uint4(va, k > 1 ? va : vb, k > 2 ? va : vb, k > 3 ? va : vb);
 }
 
+// a 25-bit plane (bit c = cell c of a 5x5 window) as 25 floats 1.0 / 0.0
+__device__ __forceinline__ void expand_plane(uint32_t m, float *dst) {
+#pragma unroll
+  for (int c = 0; c < 25; ++c) dst[c] = ((m >> c) & 1u) ? 1.0f : 0.0f;
+}
+
 // 5x5 crop of the free-cell layer around (x,y) as 25 bits, bit i*5+j = cell (x-2+i, y-2+j)
 template <class W>
 __device__ __forceinline__ uint32_t v2_free_crop(const FovTables<W> &t, int L, int x, int y) {
@@ -231,8 +237,8 @@ template <class W>
 __device__ __forceinline__ FovPre fov_preload(const KParams &p, int64_t e) {
   FovPre q;
   q.w0 = p.state[e]; q.w1 = p.goal_count[e]; q.w2 = W::HAS_LOC ? p.aux2[e] : 0u;
-  q.act = (p.mode == MODE_STEP || p.mode == 3 /* MODE_PLANNER */) ? load_action(p.actions, p.action_dtype, e) : 0;
-  if (W::NVIS > 0 && p.mode != 3) {
+  q.act = (p.mode == MODE_STEP || p.mode == MODE_PLANNER) ? load_action(p.actions, p.action_dtype, e) : 0;
+  if (W::NVIS > 0 && p.mode != MODE_PLANNER) {
     const uint4 *hp = reinterpret_cast<const uint4 *>(p.hist + e * HIST_MAX);
 #pragma unroll
     for (int k = 0; k < 4; ++k) q.h[k] = __ldcg(hp + k);

@@ -22,8 +22,6 @@
 
 namespace lmz {
 
-enum : int { MODE_PLANNER = 3 };
-
 struct V5 {
   static constexpr int ID = 5;
   static constexpr int G = 18, E = 7, F = 5, C = 7, CL = 4, S = F * E;       // lmaze_env_v5.py:25-37,357-358
@@ -250,9 +248,7 @@ __global__ void __launch_bounds__(THREADS) lmz_planner_kernel(const KParams p) {
   constexpr uint32_t PER = W::LOC_FLOATS / 4;
   float *mv = s_vals[warp];
   for (;;) {
-    int64_t tl = 0;
-    if (lane == 0) tl = p.tile_begin + grab_tile(p.work);
-    tl = __shfl_sync(0xffffffffu, tl, 0);
+    const int64_t tl = warp_grab(p, lane, 1);
     if (tl >= p.tile_end) break;
     const int64_t e = tl * 32 + lane;
     const bool valid = e < p.n;
