@@ -7,6 +7,7 @@ gym; when gym or gymnasium is importable the ids are registered there as well.
 from .envs import LmazeVecCuda, shard_range, allreduce_stats, INVALID_ACTION  # noqa: F401
 from .envs import LmazeEnv, LmazeEnv_v2, LmazeEnv_v3, LmazeEnv_v4, LmazeEnv_v5, LmazeEnv_v6  # noqa: F401
 from .envs import LmazeHierCuda  # noqa: F401
+from .envs.lmaze_vec_cuda import _VARIANTS
 
 __version__ = "0.1.0"
 
@@ -32,9 +33,7 @@ def make(id, **kwargs):
     if "-vec-" not in id and "num_envs" not in kwargs:
         kw.pop("num_envs", None)
         return _SINGLE[variant](**kw)
-    if variant in ("v5", "v6"):
-        return LmazeHierCuda(variant=variant, **kw)
-    return LmazeVecCuda(variant=variant, **kw)
+    return globals()[_VARIANTS[variant][2]](variant=variant, **kw)      # the class gym_entry_point(id) names
 
 
 def registered_ids():
@@ -62,8 +61,7 @@ def gym_entry_point(env_id):
     'lmaze-vec-vK' ids construct the batched classes."""
     variant, defaults = _REGISTRY[env_id]
     if "-vec-" in env_id:
-        cls = "LmazeHierCuda" if variant in ("v5", "v6") else "LmazeVecCuda"
-        return "gym_lmaze_b200:" + cls, dict(defaults, variant=variant)
+        return "gym_lmaze_b200:" + _VARIANTS[variant][2], dict(defaults, variant=variant)
     return "gym_lmaze_b200:" + _SINGLE[variant].__name__, {}
 
 

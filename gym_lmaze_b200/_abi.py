@@ -12,30 +12,12 @@ LIB_PATH = os.environ.get("LMAZE_B200_LIB") or os.path.join(_PKG, "liblmaze_b200
 LMZ_V0, LMZ_V2, LMZ_V3, LMZ_V4, LMZ_V5 = 0, 2, 3, 4, 5
 RENDER_TMA, RENDER_ST128, RENDER_INCREMENTAL = 0, 1, 2
 OBS_FULL, OBS_COMPACT, OBS_BITS = 0, 1, 2
-ACT_U8, ACT_I32, ACT_I64 = 0, 1, 2
 NUM_STATS = 8
 SPAWN_FORCE = 64          # LMZ_SPAWN_FORCE
-ST_COLS = 8
-ST_COLS_HIER = 17
 STAT_NAMES = ("steps", "episodes", "goals", "timeouts", "wall_bumps", "moves", "stale", "eplen_sum")
 STATE_COLS = ("x", "y", "goal_x", "goal_y", "step_count", "reward_code", "goal_count", "episode")
 STATE_COLS_HIER = ("x", "y", "prev_x", "prev_y", "fovea_x1", "fovea_y1", "goal_x", "goal_y", "fgoal_x", "fgoal_y",
                    "last_x", "last_y", "fgoal_action", "step_count", "foveal_step_count", "flags", "episode")
-
-# every symbol include/lmaze_b200.h declares (tests/test_abi_symbols.py checks the header against this)
-EXPORTS = (
-    "lmz_abi_version", "lmz_last_error", "lmz_default_config", "lmz_obs_shape", "lmz_grid_size", "lmz_obs_desc",
-    "lmz_layout", "lmz_num_layouts", "lmz_layout_ex", "lmz_num_actions", "lmz_set_window", "lmz_set_window_dl",
-    "lmz_create", "lmz_destroy", "lmz_bind", "lmz_bind_dl", "lmz_reset", "lmz_reset_dl", "lmz_step",
-    "lmz_step_dl", "lmz_step_host", "lmz_step_host_async", "lmz_step_host_wait", "lmz_render", "lmz_rollout",
-    "lmz_rollout_dl", "lmz_rollout_codes", "lmz_rollout_codes_dl", "lmz_get_state",
-    "lmz_set_state", "lmz_get_state_dl", "lmz_set_state_dl", "lmz_get_visit", "lmz_set_visit", "lmz_get_visit_dl",
-    "lmz_set_visit_dl", "lmz_stats", "lmz_stats_reset", "lmz_launch_count",
-    "lmz_state_cols", "lmz_local_obs_shape", "lmz_bind_local", "lmz_bind_local_dl", "lmz_planner_step",
-    "lmz_planner_step_dl", "lmz_safe_goal", "lmz_safe_goal_dl", "lmz_planner_step_auto", "lmz_planner_step_auto_dl",
-    "lmz_hier_step_host", "lmz_hier_rollout", "lmz_hier_rollout_dl",
-)
-
 
 class LmzConfig(ctypes.Structure):
     _fields_ = [
@@ -61,6 +43,68 @@ class LmzError(RuntimeError):
         self.code = code
 
 
+_vp, _i32, _i64 = ctypes.c_void_p, ctypes.c_int32, ctypes.c_int64
+_SHAPE = ctypes.POINTER(_i64 * 3)
+
+# export -> argtypes, or (argtypes, restype) where it does not return int: every symbol include/lmaze_b200.h declares
+# (tests/test_abi_cpu.py checks the header against EXPORTS)
+_PROTOTYPES = {
+    "lmz_abi_version": [],
+    "lmz_last_error": ([], ctypes.c_char_p),
+    "lmz_default_config": ([ctypes.POINTER(LmzConfig)], None),
+    "lmz_obs_shape": [_i32, _SHAPE],
+    "lmz_grid_size": [_i32],
+    "lmz_obs_desc": [_i32, _i32, _SHAPE, ctypes.POINTER(_i32)],
+    "lmz_layout": [_i32, ctypes.c_char_p],
+    "lmz_num_layouts": [_i32],
+    "lmz_layout_ex": [_i32, _i32, ctypes.c_char_p],
+    "lmz_num_actions": [_i32],
+    "lmz_set_window": [_vp, _vp, _i64, _i64],
+    "lmz_set_window_dl": [_vp, _vp, _i64],
+    "lmz_create": [ctypes.POINTER(LmzConfig), ctypes.POINTER(_vp)],
+    "lmz_destroy": [_vp],
+    "lmz_bind": [_vp, _vp, _vp, _vp],
+    "lmz_bind_dl": [_vp, _vp, _vp, _vp],
+    "lmz_reset": [_vp, _vp, _vp, _vp],
+    "lmz_reset_dl": [_vp, _vp, _vp, _vp],
+    "lmz_step": [_vp, _vp, _i32, _vp, _vp],
+    "lmz_step_dl": [_vp, _vp, _vp, _vp],
+    "lmz_step_host": [_vp, _vp, _i32, _vp, _vp, _vp, _vp],
+    "lmz_step_host_async": [_vp, _vp, _i32, _vp, _vp, _vp, _vp, ctypes.POINTER(_i32)],
+    "lmz_step_host_wait": [_vp, _i32],
+    "lmz_render": [_vp, _vp],
+    "lmz_rollout": [_vp, _i32, _vp, _i32, _vp, _vp, _vp],
+    "lmz_rollout_dl": [_vp, _i32, _vp, _vp, _vp, _vp],
+    "lmz_rollout_codes": [_vp, _i32, _vp, _i32, _vp, _vp, _vp],
+    "lmz_rollout_codes_dl": [_vp, _i32, _vp, _vp, _vp, _vp],
+    "lmz_get_state": [_vp, _vp, _vp],
+    "lmz_set_state": [_vp, _vp, _vp],
+    "lmz_get_state_dl": [_vp, _vp, _vp],
+    "lmz_set_state_dl": [_vp, _vp, _vp],
+    "lmz_get_visit": [_vp, _vp, _vp],
+    "lmz_set_visit": [_vp, _vp, _vp],
+    "lmz_get_visit_dl": [_vp, _vp, _vp],
+    "lmz_set_visit_dl": [_vp, _vp, _vp],
+    "lmz_stats": [_vp, ctypes.POINTER(_i64 * NUM_STATS), ctypes.POINTER(_i64), _vp],
+    "lmz_stats_reset": [_vp, _vp],
+    "lmz_launch_count": ([_vp], _i64),
+    "lmz_state_cols": [_i32],
+    "lmz_local_obs_shape": [_i32, _SHAPE],
+    "lmz_bind_local": [_vp] * 6,
+    "lmz_bind_local_dl": [_vp] * 6,
+    "lmz_planner_step": [_vp, _vp, _i32, _vp, _vp],
+    "lmz_planner_step_dl": [_vp, _vp, _vp, _vp],
+    "lmz_safe_goal": [_vp, _vp, _i32, _vp, _vp, _vp],
+    "lmz_safe_goal_dl": [_vp, _vp, _vp, _vp, _vp],
+    "lmz_planner_step_auto": [_vp, _vp, _i32, _vp],
+    "lmz_planner_step_auto_dl": [_vp, _vp, _vp],
+    "lmz_hier_step_host": [_vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp],
+    "lmz_hier_rollout": [_vp, _i32, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp],
+    "lmz_hier_rollout_dl": [_vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
+}
+EXPORTS = tuple(_PROTOTYPES)
+
+
 _lib = None
 
 
@@ -74,65 +118,9 @@ def load():
             "%s is missing: build it with `python -m gym_lmaze_b200.build` (needs nvcc, sm_100a). "
             "gym_lmaze_b200 has no CPU fallback." % LIB_PATH)
     L = ctypes.CDLL(LIB_PATH)
-    vp, i32, i64 = ctypes.c_void_p, ctypes.c_int32, ctypes.c_int64
-    L.lmz_abi_version.restype = ctypes.c_int
-    L.lmz_last_error.restype = ctypes.c_char_p
-    L.lmz_default_config.argtypes = [ctypes.POINTER(LmzConfig)]
-    L.lmz_default_config.restype = None
-    L.lmz_obs_shape.argtypes = [i32, ctypes.POINTER(i64 * 3)]
-    L.lmz_grid_size.argtypes = [i32]
-    L.lmz_obs_desc.argtypes = [i32, i32, ctypes.POINTER(i64 * 3), ctypes.POINTER(i32)]
-    L.lmz_set_window.argtypes = [vp, vp, i64, i64]
-    L.lmz_set_window_dl.argtypes = [vp, vp, i64]
-    L.lmz_layout.argtypes = [i32, ctypes.c_char_p]
-    L.lmz_num_layouts.argtypes = [i32]
-    L.lmz_layout_ex.argtypes = [i32, i32, ctypes.c_char_p]
-    L.lmz_num_actions.argtypes = [i32]
-    L.lmz_create.argtypes = [ctypes.POINTER(LmzConfig), ctypes.POINTER(vp)]
-    L.lmz_destroy.argtypes = [vp]
-    L.lmz_bind.argtypes = [vp, vp, vp, vp]
-    L.lmz_bind_dl.argtypes = [vp, vp, vp, vp]
-    L.lmz_reset.argtypes = [vp, vp, vp, vp]
-    L.lmz_reset_dl.argtypes = [vp, vp, vp, vp]
-    L.lmz_step.argtypes = [vp, vp, i32, vp, vp]
-    L.lmz_step_dl.argtypes = [vp, vp, vp, vp]
-    L.lmz_step_host.argtypes = [vp, vp, i32, vp, vp, vp, vp]
-    L.lmz_step_host_async.argtypes = [vp, vp, i32, vp, vp, vp, vp, ctypes.POINTER(i32)]
-    L.lmz_step_host_wait.argtypes = [vp, i32]
-    L.lmz_rollout_codes.argtypes = [vp, i32, vp, i32, vp, vp, vp]
-    L.lmz_rollout_codes_dl.argtypes = [vp, i32, vp, vp, vp, vp]
-    L.lmz_render.argtypes = [vp, vp]
-    L.lmz_rollout.argtypes = [vp, i32, vp, i32, vp, vp, vp]
-    L.lmz_rollout_dl.argtypes = [vp, i32, vp, vp, vp, vp]
-    L.lmz_get_state.argtypes = [vp, vp, vp]
-    L.lmz_set_state.argtypes = [vp, vp, vp]
-    L.lmz_get_state_dl.argtypes = [vp, vp, vp]
-    L.lmz_set_state_dl.argtypes = [vp, vp, vp]
-    L.lmz_get_visit.argtypes = [vp, vp, vp]
-    L.lmz_set_visit.argtypes = [vp, vp, vp]
-    L.lmz_get_visit_dl.argtypes = [vp, vp, vp]
-    L.lmz_set_visit_dl.argtypes = [vp, vp, vp]
-    L.lmz_state_cols.argtypes = [i32]
-    L.lmz_local_obs_shape.argtypes = [i32, ctypes.POINTER(i64 * 3)]
-    L.lmz_bind_local.argtypes = [vp] * 6
-    L.lmz_bind_local_dl.argtypes = [vp] * 6
-    L.lmz_planner_step.argtypes = [vp, vp, i32, vp, vp]
-    L.lmz_planner_step_dl.argtypes = [vp, vp, vp, vp]
-    L.lmz_planner_step_auto.argtypes = [vp, vp, i32, vp]
-    L.lmz_planner_step_auto_dl.argtypes = [vp, vp, vp]
-    L.lmz_hier_step_host.argtypes = [vp, vp, vp, i32, vp, vp, vp, vp, vp]
-    L.lmz_hier_rollout.argtypes = [vp, i32, vp, vp, i32, vp, vp, vp, vp, vp]
-    L.lmz_hier_rollout_dl.argtypes = [vp, i32, vp, vp, vp, vp, vp, vp, vp]
-    L.lmz_safe_goal.argtypes = [vp, vp, i32, vp, vp, vp]
-    L.lmz_safe_goal_dl.argtypes = [vp, vp, vp, vp, vp]
-    L.lmz_stats.argtypes = [vp, ctypes.POINTER(i64 * NUM_STATS), ctypes.POINTER(i64), vp]
-    L.lmz_stats_reset.argtypes = [vp, vp]
-    L.lmz_launch_count.argtypes = [vp]
-    L.lmz_launch_count.restype = i64
-    for name in EXPORTS:
+    for name, proto in _PROTOTYPES.items():
         fn = getattr(L, name)
-        if name not in ("lmz_abi_version", "lmz_last_error", "lmz_default_config", "lmz_launch_count"):
-            fn.restype = ctypes.c_int
+        fn.argtypes, fn.restype = proto if isinstance(proto, tuple) else (proto, ctypes.c_int)
     if L.lmz_abi_version() != 1:
         raise ImportError("liblmaze_b200.so ABI version %d, binding expects 1" % L.lmz_abi_version())
     _lib = L
@@ -150,25 +138,21 @@ _PyCapsule_GetPointer.restype = ctypes.c_void_p
 _PyCapsule_GetPointer.argtypes = [ctypes.py_object, ctypes.c_char_p]
 
 
-class Borrowed(object):
-    """Keeps a tensor's DLPack capsule alive while the C side borrows its pointer.
+def dl(tensor):
+    """(pointer-or-None, capsule) for an optional tensor argument: the pointer is valid while the capsule lives.
 
     The capsule is never renamed to "used_dltensor", so when it is collected
     PyTorch's capsule destructor calls the DLManagedTensor deleter itself -- the
     shim never takes ownership (include/lmaze_b200.h conventions).
     """
-
-    __slots__ = ("capsule", "ptr", "tensor")
-
-    def __init__(self, tensor):
-        self.tensor = tensor
-        self.capsule = tensor.__dlpack__()
-        self.ptr = _PyCapsule_GetPointer(self.capsule, b"dltensor")
-
-
-def dl(tensor):
-    """(pointer-or-None, keepalive) for an optional tensor argument."""
     if tensor is None:
         return None, None
-    b = Borrowed(tensor)
-    return b.ptr, b
+    capsule = tensor.__dlpack__()
+    return _PyCapsule_GetPointer(capsule, b"dltensor"), capsule
+
+
+def call(fn, *args):
+    """fn(*args) for an lmz_*_dl export, raising LmzError if it fails.  Each tensor argument goes in as a borrowed
+    DLPack capsule that stays alive until fn returns; None and the other arguments are passed as they are."""
+    borrowed = [dl(a) if hasattr(a, "__dlpack__") else (a, None) for a in args]
+    check(fn(*[p for p, _ in borrowed]))

@@ -16,26 +16,47 @@ kernels (one env); only the result is copied to the host.  For throughput use Lm
 import numpy as np
 import torch
 
-from .lmaze_vec_cuda import LmazeVecCuda, INVALID_ACTION, _V3_WORDS
+from .lmaze_vec_cuda import LmazeVecCuda, INVALID_ACTION, _ReferenceSurface, _V3_WORDS
 from .lmaze_hier_cuda import LmazeHierCuda
 
-# f32 bit pattern -> the reference's Python float (lmaze_env.py:21-23,109)
-_REWARD = {0x80000000: -0.0, 0xBF800000: -1.0, 0xBC23D70A: -0.01, 0x42C80000: 100.0}
+# f32 bit pattern -> the reference's Python float (lmaze_env.py:21-23,109): the shortest decimal that reads back as
+# that f32, which is the literal the reference wrote (-0.01, not the f32's -0.009999999776...)
+_REWARD = {b: float(str(np.uint32(b).view(np.float32))) for b in LmazeVecCuda.REWARD_BITS}
 
 
-class _SingleMaze(object):
-    metadata = {"render.modes": ["human"]}
-    _variant = "v0"
+class _OneMaze(_ReferenceSurface):
+    """One env of a batched class (no auto-reset), read back with the reference's Python types."""
+    _vec_class = LmazeVecCuda
 
     def __init__(self, device=None, seed=0, **kwargs):
-        self._vec = LmazeVecCuda(1, self._variant, device=device, seed=seed, autoreset=False, **kwargs)
-        self.action_space = self._vec.single_action_space
-        self.observation_space = self._vec.single_observation_space
+        self._vec = self._vec_class(1, self._variant, device=device, seed=seed, autoreset=False, **kwargs)
         self.VISUALIZE = False
         self.reset()                                   # the reference constructors end with reset()
 
     def _obs(self):
         return self._vec.obs[0].cpu().numpy()          # a fresh array per call, like the reference's np.zeros
+
+    @staticmethod
+    def _reward(t):
+        """A one-env f32 reward tensor -> the reference's Python float."""
+        return _REWARD[int(t.view(torch.int32).item()) & 0xFFFFFFFF]
+
+    def close(self):
+        self._vec.close()
+
+    @property
+    def state_vector(self):
+        """x, y, goal_x, goal_y, stepCount, ... of the single env (see LmazeVecCuda.get_state)."""
+        return self._vec.get_state()[0].tolist()
+
+
+class _SingleMaze(_OneMaze):
+    _variant = "v0"
+
+    def __init__(self, device=None, seed=0, **kwargs):
+        super().__init__(device=device, seed=seed, **kwargs)
+        self.action_space = self._vec.single_action_space
+        self.observation_space = self._vec.single_observation_space
 
     def reset(self, spawn=None, **kwargs):
         """spawn: optional (ball_x, ball_y[, goal_x, goal_y[, layout]]) to pin the cells the reference's
@@ -52,25 +73,7 @@ class _SingleMaze(object):
         code = self._code(action)
         wire = code if 0 <= code < 255 else INVALID_ACTION     # any unmatched value takes the (0,0) branch
         self._vec.step(torch.tensor([wire], dtype=torch.uint8))
-        bits = int(self._vec.reward.view(torch.int32).item()) & 0xFFFFFFFF
-        return self._obs(), _REWARD[bits], bool(self._vec.done.item()), code      # msg = int(msg) is what comes back
-
-    def render(self, mode="human", close=False):       # lmaze_env.py:55-59: only flips the display flag
-        self.VISUALIZE = (mode == "human")
-
-    def rendering(self, msg):
-        self.VISUALIZE = msg
-
-    def writing(self, msg):
-        self.SAVEFRAME = msg
-
-    def close(self):
-        self._vec.close()
-
-    @property
-    def state_vector(self):
-        """x, y, goal_x, goal_y, stepCount, ... of the single env (see LmazeVecCuda.get_state)."""
-        return self._vec.get_state()[0].tolist()
+        return self._obs(), self._reward(self._vec.reward), bool(self._vec.done.item()), code      # msg = int(msg)
 
 
 class LmazeEnv(_SingleMaze):
@@ -110,23 +113,21 @@ class LmazeEnv_v3(_SingleMaze):
         return super().reset(spawn=spawn)
 
 
-class LmazeEnv_v5(object):
+class LmazeEnv_v5(_OneMaze):
     """Reference LmazeEnv_v5: reset() -> foveal obs; plannerStep(goal) -> local obs; step(a) -> the 8-tuple
     (fovobs, locobs, globalReward, originalReward, globalDone, localDone, fovealGoal, local_action),
     lmaze_env_v5.py:285-292.  The constructor ends with reset(), like the reference's (lmaze_env_v5.py:92)."""
-    metadata = {"render.modes": ["human"]}
+    _vec_class = LmazeHierCuda
     _variant = "v5"
 
     def __init__(self, device=None, seed=0, **kwargs):
-        self._vec = LmazeHierCuda(1, self._variant, device=device, seed=seed, autoreset=False, **kwargs)
-        self.VISUALIZE = False
         self.step_limit, self.foveal_step_limit = 10, 50
-        self.reset()
+        super().__init__(device=device, seed=seed, **kwargs)
 
     def reset(self, spawn=None):
         """spawn: optional (ball_x, ball_y, goal_x, goal_y, layout) pinning the reference's random draws."""
         self._vec.reset(spawn=None if spawn is None else [list(spawn)])
-        return self._vec.obs[0].cpu().numpy()
+        return self._obs()
 
     def _loc(self):
         if bool(self._vec.loc_err.item()):
@@ -146,27 +147,8 @@ class LmazeEnv_v5(object):
         wire = code if 0 <= code < 255 else INVALID_ACTION
         v = self._vec
         v.step(torch.tensor([wire], dtype=torch.uint8), goal_plane=False)
-        fov = v.obs[0].cpu().numpy()
-        gbits = int(v.reward.view(torch.int32).item()) & 0xFFFFFFFF
-        lbits = int(v.local_reward.view(torch.int32).item()) & 0xFFFFFFFF
-        return (fov, self._loc(), _REWARD[gbits], _REWARD[lbits], bool(v.done.item()), bool(v.local_done.item()),
-                v.goal_plane()[0].cpu().numpy(), code)
-
-    def render(self, mode="human", close=False):
-        self.VISUALIZE = (mode == "human")
-
-    def rendering(self, msg):
-        self.VISUALIZE = msg
-
-    def writing(self, msg):
-        self.SAVEFRAME = msg
-
-    def close(self):
-        self._vec.close()
-
-    @property
-    def state_vector(self):
-        return self._vec.get_state()[0].tolist()
+        return (self._obs(), self._loc(), self._reward(v.reward), self._reward(v.local_reward), bool(v.done.item()),
+                bool(v.local_done.item()), v.goal_plane()[0].cpu().numpy(), code)
 
 
 class LmazeEnv_v6(LmazeEnv_v5):

@@ -16,16 +16,18 @@ import ctypes
 import torch
 
 from .. import _abi
-from .lmaze_vec_cuda import LmazeVecCuda
+from .lmaze_vec_cuda import LmazeVecCuda, _ACTION_DTYPES, _VARIANTS
 
 
 class LmazeHierCuda(LmazeVecCuda):
+    _batched = "LmazeHierCuda"
+
     def __init__(self, num_envs=1, variant="v5", device=None, seed=0, autoreset=True, env_id0=0, random_ball=True,
                  random_goal=True, tune=None, obs_mode="full"):
-        if variant not in ("v5", "v6", 5, 6, "lmaze-v5", "lmaze-v6"):
+        if variant not in _VARIANTS or _VARIANTS[variant][2] != self._batched:
             raise ValueError("LmazeHierCuda is the planner/actor env: variant must be 'v5' or 'v6'")
-        self.variant_name = "v6" if variant in ("v6", 6, "lmaze-v6") else "v5"
-        super().__init__(num_envs, "v5", device=device, seed=seed, autoreset=autoreset, env_id0=env_id0,
+        self.variant_name = _VARIANTS[variant][0]
+        super().__init__(num_envs, variant, device=device, seed=seed, autoreset=autoreset, env_id0=env_id0,
                          random_ball=random_ball, random_goal=random_goal, tune=tune, obs_mode=obs_mode)
         shape = (ctypes.c_int64 * 3)()
         _abi.check(self._lib.lmz_local_obs_shape(self.variant, ctypes.byref(shape)))
@@ -40,9 +42,8 @@ class LmazeHierCuda(LmazeVecCuda):
         self._loc_err_u8 = torch.zeros(n, dtype=torch.uint8, device=dev)
         self.loc_err = self._loc_err_u8.view(torch.bool)
         self.foveal_goal = torch.full((n,), 12, dtype=torch.uint8, device=dev)      # hot cell of fovealGoal
-        ptrs = [_abi.dl(t) for t in (self.loc_obs, self.local_reward, self._ldone_u8, self._loc_err_u8, self.foveal_goal)]
-        _abi.check(self._lib.lmz_bind_local_dl(self._h, *[p for p, _ in ptrs]))
-        self._local_keepalive = [k for _, k in ptrs]
+        _abi.call(self._lib.lmz_bind_local_dl, self._h, self.loc_obs, self.local_reward, self._ldone_u8,
+                  self._loc_err_u8, self.foveal_goal)
         self.global_reward, self.global_done, self.fov_obs = self.reward, self.done, self.obs
         self.step_limit, self.foveal_step_limit = 10, 50                           # lmaze_env_v5.py:47-48
 
@@ -55,14 +56,11 @@ class LmazeHierCuda(LmazeVecCuda):
         if isinstance(mask, str):
             if mask != "auto":
                 raise ValueError("mask must be a tensor, None or 'auto'")
-            pg, kg = _abi.dl(goals)
-            _abi.check(self._lib.lmz_planner_step_auto_dl(self._h, pg, self._stream()))
+            _abi.call(self._lib.lmz_planner_step_auto_dl, self._h, goals, self._stream())
             return self.loc_obs
         if mask is not None:
             mask = torch.as_tensor(mask).to(device=self.device).to(torch.uint8).contiguous()
-        pg, kg = _abi.dl(goals)
-        pm, km = _abi.dl(mask)
-        _abi.check(self._lib.lmz_planner_step_dl(self._h, pg, pm, self._stream()))
+        _abi.call(self._lib.lmz_planner_step_dl, self._h, goals, mask, self._stream())
         return self.loc_obs
 
     planner_step = plannerStep
@@ -81,11 +79,7 @@ class LmazeHierCuda(LmazeVecCuda):
     def step(self, actions, spawn=None, goal_plane=True):
         """Reference step (lmaze_env_v5.py:187-292), batched 8-tuple.  `loc_err` marks the envs where the
         reference's buildLocalObservation would raise IndexError (their local rows are zeros)."""
-        actions = self._as_actions(actions)
-        spawn = self._as_spawn(spawn)
-        pa, ka = _abi.dl(actions)
-        ps, ks = _abi.dl(spawn)
-        _abi.check(self._lib.lmz_step_dl(self._h, pa, ps, self._stream()))
+        actions = self._step(actions, spawn)
         return (self.obs, self.loc_obs, self.reward, self.local_reward, self.done, self.local_done,
                 self.goal_plane() if goal_plane else self.foveal_goal, actions)
 
@@ -94,50 +88,26 @@ class LmazeHierCuda(LmazeVecCuda):
         wall.  draws: optional int64 [N, K] = the values np.random.randint(0, 25) would return, consumed until
         a non-wall cell comes up; then returns (goals, used).  Default: device RNG, returns goals u8 [N]."""
         goals = torch.empty(self.num_envs, dtype=torch.uint8, device=self.device)
-        pg, kg = _abi.dl(goals)
         if draws is None:
-            _abi.check(self._lib.lmz_safe_goal_dl(self._h, None, pg, None, self._stream()))
+            _abi.call(self._lib.lmz_safe_goal_dl, self._h, None, goals, None, self._stream())
             return goals
         draws = torch.as_tensor(draws).to(device=self.device, dtype=torch.int64).contiguous()
         used = torch.empty(self.num_envs, dtype=torch.int32, device=self.device)
-        pd, kd = _abi.dl(draws)
-        pu, ku = _abi.dl(used)
-        _abi.check(self._lib.lmz_safe_goal_dl(self._h, pd, pg, pu, self._stream()))
+        _abi.call(self._lib.lmz_safe_goal_dl, self._h, draws, goals, used, self._stream())
         return goals, used
 
     safe_foveal_goal = safeFovealGoal
 
-    # ------------------------------------------------------------------ state
-    def get_state(self):
-        """int32 [N, 17]: _abi.STATE_COLS_HIER."""
-        out = torch.empty((self.num_envs, _abi.ST_COLS_HIER), dtype=torch.int32, device=self.device)
-        p, k = _abi.dl(out)
-        _abi.check(self._lib.lmz_get_state_dl(self._h, p, self._stream()))
-        return out
-
-    def capture_step(self, actions_buf, spawn_buf=None):
-        actions_buf = self._as_actions(actions_buf)
-        spawn_buf = self._as_spawn(spawn_buf)
-        self.render_obs()
-        torch.cuda.synchronize(self.device)
-        graph = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(graph):
-            self.step(actions_buf, spawn=spawn_buf, goal_plane=False)
-        self._graphs = getattr(self, "_graphs", []) + [(graph, actions_buf, spawn_buf)]
-        return graph.replay
-
     def step_host(self, goals_host, actions_host, greward_host, lreward_host, gdone_host, ldone_host):
         """End-to-end planner + actor step with HOST buffers (pinned CPU tensors): H2D goals and actions,
         plannerStep(mask="auto") + step, D2H both rewards and both done flags, stream synchronised on return."""
-        n = self.num_envs
-        for t in (goals_host, actions_host, greward_host, lreward_host, gdone_host, ldone_host):
-            if t.device.type != "cpu" or not t.is_contiguous() or t.numel() != n:
-                raise ValueError("step_host takes contiguous CPU tensors of num_envs elements")
-        if goals_host.dtype != actions_host.dtype or actions_host.dtype not in (torch.uint8, torch.int32, torch.int64):
-            raise ValueError("goals_host / actions_host must share a dtype of uint8/int32/int64")
-        if greward_host.dtype != torch.float32 or lreward_host.dtype != torch.float32:
-            raise ValueError("reward buffers must be float32")
-        ad = (torch.uint8, torch.int32, torch.int64).index(actions_host.dtype)
+        ad = self._host_buffer("actions_host", actions_host, _ACTION_DTYPES)
+        if self._host_buffer("goals_host", goals_host, _ACTION_DTYPES) != ad:
+            raise ValueError("goals_host must have actions_host's dtype")
+        self._host_buffer("greward_host", greward_host, (torch.float32,))
+        self._host_buffer("lreward_host", lreward_host, (torch.float32,))
+        self._host_buffer("gdone_host", gdone_host)
+        self._host_buffer("ldone_host", ldone_host)
         _abi.check(self._lib.lmz_hier_step_host(
             self._h, goals_host.data_ptr(), actions_host.data_ptr(), ad, greward_host.data_ptr(),
             lreward_host.data_ptr(), gdone_host.data_ptr(), ldone_host.data_ptr(), self._stream()))
@@ -160,8 +130,7 @@ class LmazeHierCuda(LmazeVecCuda):
         lr = torch.empty((T, n), dtype=torch.float32, device=dev)
         gd = torch.empty((T, n), dtype=torch.uint8, device=dev)
         ld = torch.empty((T, n), dtype=torch.uint8, device=dev)
-        ptrs = [_abi.dl(t) for t in (goals, actions, gr, lr, gd, ld)]
-        _abi.check(self._lib.lmz_hier_rollout_dl(self._h, T, *[p for p, _ in ptrs], self._stream()))
+        _abi.call(self._lib.lmz_hier_rollout_dl, self._h, T, goals, actions, gr, lr, gd, ld, self._stream())
         return gr, lr, gd.view(torch.bool), ld.view(torch.bool)
 
     def _unsupported(self, *a, **k):

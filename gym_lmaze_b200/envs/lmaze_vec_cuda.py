@@ -22,11 +22,12 @@ import torch
 from .. import _abi
 from ..spaces import make_spaces
 
-_VARIANTS = {"v0": _abi.LMZ_V0, 0: _abi.LMZ_V0, "lmaze-v0": _abi.LMZ_V0,
-             "v2": _abi.LMZ_V2, 2: _abi.LMZ_V2, "lmaze-v2": _abi.LMZ_V2,
-             "v4": _abi.LMZ_V4, 4: _abi.LMZ_V4, "lmaze-v4": _abi.LMZ_V4,
-             "v3": _abi.LMZ_V3, 3: _abi.LMZ_V3, "lmaze-v3": _abi.LMZ_V3,
-             "v5": _abi.LMZ_V5, 5: _abi.LMZ_V5, "lmaze-v5": _abi.LMZ_V5}    # v5/v6: use LmazeHierCuda
+# every accepted variant spelling -> (name, ABI id, batched class).  v6 is v5 plus safeFovealGoal: one ABI variant.
+_VARIANTS = {spelling: (name, abi_id, batched)
+             for name, abi_id, batched in (("v0", _abi.LMZ_V0, "LmazeVecCuda"), ("v2", _abi.LMZ_V2, "LmazeVecCuda"),
+                                           ("v3", _abi.LMZ_V3, "LmazeVecCuda"), ("v4", _abi.LMZ_V4, "LmazeVecCuda"),
+                                           ("v5", _abi.LMZ_V5, "LmazeHierCuda"), ("v6", _abi.LMZ_V5, "LmazeHierCuda"))
+             for spelling in (name, int(name[1:]), "lmaze-" + name)}
 _RENDER = {"tma": _abi.RENDER_TMA, "st128": _abi.RENDER_ST128, "incremental": _abi.RENDER_INCREMENTAL}
 _OBS_MODE = {"full": _abi.OBS_FULL, "compact": _abi.OBS_COMPACT, "bits": _abi.OBS_BITS}
 # lmaze_env_v3.py:236-247 -- the strings v3's step() accepts; anything else is its unmatched branch
@@ -45,15 +46,30 @@ def shard_range(total_envs, rank, world_size):
     return lo, hi
 
 
-class LmazeVecCuda(object):
-    metadata = {"render.modes": ["human"]}          # lmaze_env.py:12
+class _ReferenceSurface(object):
+    """The reference's display hooks (lmaze_env.py:12,55-59,251-256).  cv2 display is out of scope: they only set
+    the flags."""
+    metadata = {"render.modes": ["human"]}
+
+    def render(self, mode="human", close=False):
+        self.VISUALIZE = (mode == "human")
+
+    def rendering(self, msg):
+        self.VISUALIZE = msg
+
+    def writing(self, msg):
+        self.SAVEFRAME = msg
+
+
+class LmazeVecCuda(_ReferenceSurface):
+    _batched = "LmazeVecCuda"            # the batched class _VARIANTS names for the variants this class runs
 
     def __init__(self, num_envs=1, variant="v0", device=None, seed=0, autoreset=True, render_mode="tma",
                  env_id0=0, random_ball=True, random_goal=True, with_obs=True, tune=None, obs_mode="full",
                  obs_window=None):
         if variant not in _VARIANTS:
             raise ValueError("unknown variant %r (built: v0, v2, v3, v4; v5/v6 through LmazeHierCuda)" % (variant,))
-        if _VARIANTS[variant] == _abi.LMZ_V5 and not hasattr(self, "plannerStep"):
+        if _VARIANTS[variant][2] != self._batched:
             raise ValueError("lmaze-v5/v6 is the planner/actor env: construct LmazeHierCuda")
         if render_mode not in _RENDER:
             raise ValueError("render_mode must be 'tma', 'st128' or 'incremental'")
@@ -67,7 +83,7 @@ class LmazeVecCuda(object):
             raise ValueError("device must be a CUDA device")
         if self.device.index is None:
             self.device = torch.device("cuda", torch.cuda.current_device())
-        self.variant = _VARIANTS[variant]
+        self.variant = _VARIANTS[variant][1]
         self.num_envs = int(num_envs)
         self.autoreset = bool(autoreset)
         self.env_id0 = int(env_id0)
@@ -92,6 +108,7 @@ class LmazeVecCuda(object):
         self.expansion = self.full_obs_shape[1] // (5 if foveal else self.grid_size)      # the reference's expansionRatio
         self.num_actions = self._lib.lmz_num_actions(self.variant)      # Discrete(4) / Discrete(25)
         self.num_layouts = self._lib.lmz_num_layouts(self.variant)
+        self._state_cols = self._lib.lmz_state_cols(self.variant)      # get_state() columns
         self.single_action_space, self.single_observation_space = make_spaces(self.num_actions, self.full_obs_shape)
         self.action_space, self.observation_space = self.single_action_space, self.single_observation_space
         self.VISUALIZE = False           # lmaze_env.py:26; cv2 display is out of scope
@@ -128,11 +145,7 @@ class LmazeVecCuda(object):
 
     def _bind(self):
         windowed = self.obs is not None and self.obs_window < self.num_envs
-        po, ko = _abi.dl(None if windowed else self.obs)
-        pr, kr = _abi.dl(self.reward)
-        pd, kd = _abi.dl(self._done_u8)
-        _abi.check(self._lib.lmz_bind_dl(self._h, po, pr, pd))
-        self._bound_keepalive = (ko, kr, kd)
+        _abi.call(self._lib.lmz_bind_dl, self._h, None if windowed else self.obs, self.reward, self._done_u8)
         if windowed:
             self.set_window(0)
 
@@ -141,11 +154,9 @@ class LmazeVecCuda(object):
         write only those rows (every env still steps).  For batches whose full observation
         tensor does not fit in HBM."""
         env_lo = int(env_lo)
-        po, ko = _abi.dl(self.obs)
-        _abi.check(self._lib.lmz_set_window_dl(self._h, po, env_lo))
+        _abi.call(self._lib.lmz_set_window_dl, self._h, self.obs, env_lo)
         self._obs_desync = True
         self.window_lo = env_lo
-        self._window_keepalive = ko
 
     def render_window(self, env_lo):
         """set_window(env_lo) + render the current state of that window into `obs`."""
@@ -224,9 +235,7 @@ class LmazeVecCuda(object):
         spawn = self._as_spawn(spawn)
         if mask is not None:
             mask = torch.as_tensor(mask).to(device=self.device).to(torch.uint8).contiguous()
-        pm, km = _abi.dl(mask)
-        ps, ks = _abi.dl(spawn)
-        _abi.check(self._lib.lmz_reset_dl(self._h, pm, ps, self._stream()))
+        _abi.call(self._lib.lmz_reset_dl, self._h, mask, spawn, self._stream())
         if mask is None:
             self._obs_desync = False
         return self.obs
@@ -239,13 +248,15 @@ class LmazeVecCuda(object):
         (lmaze_env.py:237).  With autoreset the obs rows of finished envs already
         show the next episode's first observation.
         """
-        actions = self._as_actions(actions)
-        spawn = self._as_spawn(spawn)
-        pa, ka = _abi.dl(actions)
-        ps, ks = _abi.dl(spawn)
-        _abi.check(self._lib.lmz_step_dl(self._h, pa, ps, self._stream()))
-        self._obs_desync = False         # a step always leaves the window fully rendered (full render when out of sync)
+        actions = self._step(actions, spawn)
         return self.obs, self.reward, self.done, {"action": actions}
+
+    def _step(self, actions, spawn):
+        """Launch the fused step; returns the actions as the kernel read them."""
+        actions = self._as_actions(actions)
+        _abi.call(self._lib.lmz_step_dl, self._h, actions, self._as_spawn(spawn), self._stream())
+        self._obs_desync = False         # a step always leaves the window fully rendered (full render when out of sync)
+        return actions
 
     def capture_step(self, actions_buf, spawn_buf=None):
         """Capture one fused step into a CUDA graph and return `replay()`.
@@ -267,7 +278,7 @@ class LmazeVecCuda(object):
         torch.cuda.synchronize(self.device)
         graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(graph):
-            self.step(actions_buf, spawn=spawn_buf)
+            self._step(actions_buf, spawn_buf)
         self._graphs = getattr(self, "_graphs", []) + [(graph, actions_buf, spawn_buf)]
         if self.render_mode != "incremental":
             return graph.replay
@@ -282,25 +293,28 @@ class LmazeVecCuda(object):
     def step_host(self, actions_host, reward_host, done_host, obs_host=None):
         """End-to-end step with HOST buffers (pinned CPU tensors): H2D actions, fused
         step, D2H reward/done (and obs if given), stream synchronised on return."""
-        for t in (actions_host, reward_host, done_host):
-            if t.device.type != "cpu" or not t.is_contiguous():
-                raise ValueError("step_host takes contiguous CPU tensors")
-        if actions_host.dtype not in _ACTION_DTYPES:
-            raise ValueError("actions_host dtype must be uint8/int32/int64")
-        if actions_host.numel() != self.num_envs or reward_host.numel() != self.num_envs \
-                or done_host.numel() != self.num_envs:
-            raise ValueError("host buffers must have num_envs elements")
-        if reward_host.dtype != torch.float32 or done_host.dtype not in (torch.uint8, torch.bool):
-            raise ValueError("reward_host must be float32 and done_host uint8/bool")
+        ad = self._host_buffer("actions_host", actions_host, _ACTION_DTYPES)
+        self._host_buffer("reward_host", reward_host, (torch.float32,))
+        self._host_buffer("done_host", done_host, (torch.uint8, torch.bool))
         if obs_host is not None and (obs_host.dtype != self.obs_dtype or not obs_host.is_contiguous()
                                      or obs_host.numel() != self.obs.numel()):
             raise ValueError("obs_host must be a contiguous tensor with obs's dtype and size")
-        ad = _ACTION_DTYPES.index(actions_host.dtype)
         _abi.check(self._lib.lmz_step_host(
             self._h, actions_host.data_ptr(), ad, reward_host.data_ptr(), done_host.data_ptr(),
             None if obs_host is None else obs_host.data_ptr(), self._stream()))
         self._obs_desync = False
         return reward_host, done_host
+
+    def _host_buffer(self, name, t, dtypes=None):
+        """Check one buffer of the host-step calls: a contiguous CPU tensor of num_envs elements and, unless dtypes
+        is None, of one of `dtypes`.  Returns the index of its dtype there: for _ACTION_DTYPES, the ABI dtype code."""
+        if t.device.type != "cpu" or not t.is_contiguous() or t.numel() != self.num_envs:
+            raise ValueError("%s must be a contiguous CPU tensor of num_envs elements" % name)
+        if dtypes is None:
+            return None
+        if t.dtype not in dtypes:
+            raise ValueError("%s dtype must be %s" % (name, "/".join(str(d)[len("torch."):] for d in dtypes)))
+        return dtypes.index(t.dtype)
 
     # f32 value of each reward code (lmaze_env.py:21-23,109): REWARD_TABLE[codes] is the reward tensor, bit for bit
     REWARD_BITS = (0x80000000, 0xBF800000, 0xBC23D70A, 0x42C80000)
@@ -320,19 +334,15 @@ class LmazeVecCuda(object):
         if dones is None:
             dones = torch.empty((T, self.num_envs), dtype=torch.uint8, device=self.device)
         dones_u8 = dones.view(torch.uint8) if dones.dtype == torch.bool else dones
-        pa, ka = _abi.dl(actions)
-        pd, kd = _abi.dl(dones_u8)
         if reward_codes is not None and reward_codes is not False:
             if reward_codes is True:
                 reward_codes = torch.empty((T, self.num_envs), dtype=torch.uint8, device=self.device)
-            pr, kr = _abi.dl(reward_codes)
-            _abi.check(self._lib.lmz_rollout_codes_dl(self._h, T, pa, pr, pd, self._stream()))
+            _abi.call(self._lib.lmz_rollout_codes_dl, self._h, T, actions, reward_codes, dones_u8, self._stream())
             rewards = reward_codes
         else:
             if rewards is None:
                 rewards = torch.empty((T, self.num_envs), dtype=torch.float32, device=self.device)
-            pr, kr = _abi.dl(rewards)
-            _abi.check(self._lib.lmz_rollout_dl(self._h, T, pa, pr, pd, self._stream()))
+            _abi.call(self._lib.lmz_rollout_dl, self._h, T, actions, rewards, dones_u8, self._stream())
         self._obs_desync = True          # every env moved, nothing was rendered
         return rewards, dones_u8.view(torch.bool)
 
@@ -346,41 +356,28 @@ class LmazeVecCuda(object):
         self._obs_desync = False
         return self.obs
 
-    def render(self, mode="human", close=False):
-        # the reference's render() only flips the cv2 display flag (lmaze_env.py:55-59)
-        self.VISUALIZE = (mode == "human")
-
-    def rendering(self, msg):                          # lmaze_env.py:251-252
-        self.VISUALIZE = msg
-
-    def writing(self, msg):                            # lmaze_env.py:255-256
-        self.SAVEFRAME = msg
-
     # ------------------------------------------------------------------ state / stats
     def get_state(self):
-        """int32 [N, 8]: x, y, goal_x, goal_y, step_count, reward_code, goal_count, episode."""
-        out = torch.empty((self.num_envs, _abi.ST_COLS), dtype=torch.int32, device=self.device)
-        p, k = _abi.dl(out)
-        _abi.check(self._lib.lmz_get_state_dl(self._h, p, self._stream()))
+        """int32 [N, 8]: _abi.STATE_COLS (x, y, goal_x, goal_y, step_count, reward_code, goal_count, episode);
+        for v5/v6 int32 [N, 17]: _abi.STATE_COLS_HIER."""
+        out = torch.empty((self.num_envs, self._state_cols), dtype=torch.int32, device=self.device)
+        _abi.call(self._lib.lmz_get_state_dl, self._h, out, self._stream())
         return out
 
     def set_state(self, state):
         state = torch.as_tensor(state).to(device=self.device, dtype=torch.int32).contiguous()
-        p, k = _abi.dl(state)
-        _abi.check(self._lib.lmz_set_state_dl(self._h, p, self._stream()))
+        _abi.call(self._lib.lmz_set_state_dl, self._h, state, self._stream())
         self._obs_desync = True
 
     def get_visit(self):
         """v4: the float visit layer state[2] of every env, f32 [N, 18, 18]."""
         out = torch.empty((self.num_envs, 18, 18), dtype=torch.float32, device=self.device)
-        p, k = _abi.dl(out)
-        _abi.check(self._lib.lmz_get_visit_dl(self._h, p, self._stream()))
+        _abi.call(self._lib.lmz_get_visit_dl, self._h, out, self._stream())
         return out
 
     def set_visit(self, visit):
         visit = torch.as_tensor(visit).to(device=self.device, dtype=torch.float32).contiguous()
-        p, k = _abi.dl(visit)
-        _abi.check(self._lib.lmz_set_visit_dl(self._h, p, self._stream()))
+        _abi.call(self._lib.lmz_set_visit_dl, self._h, visit, self._stream())
 
     def stats(self, check_errors=True):
         out = (ctypes.c_int64 * _abi.NUM_STATS)()
@@ -452,14 +449,12 @@ class HostPipeline(object):
 
     def submit(self, actions_host):
         env = self.env
-        if actions_host.device.type != "cpu" or not actions_host.is_contiguous() or actions_host.numel() != env.num_envs \
-                or actions_host.dtype not in _ACTION_DTYPES:
-            raise ValueError("submit takes a contiguous CPU uint8/int32/int64 tensor of num_envs actions")
+        ad = env._host_buffer("actions_host", actions_host, _ACTION_DTYPES)
         ticket = ctypes.c_int32(-1)
         slot = self.slots[self._k & 1]                       # the handle alternates its two device slots the same way
         self._k += 1
         _abi.check(env._lib.lmz_step_host_async(
-            env._h, actions_host.data_ptr(), _ACTION_DTYPES.index(actions_host.dtype), slot.reward.data_ptr(),
+            env._h, actions_host.data_ptr(), ad, slot.reward.data_ptr(),
             slot.done.data_ptr(), None if slot.obs is None else slot.obs.data_ptr(), env._stream(), ctypes.byref(ticket)))
         assert self.slots[ticket.value] is slot
         prev, self._pending = self._pending, ticket.value

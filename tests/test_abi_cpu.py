@@ -134,19 +134,6 @@ def test_gym_registration_entry_points(monkeypatch):
     assert len(w) == len(g.registered_ids()) and "id clash" in str(w[0].message)
 
 
-def test_shard_range_partitions_exactly():
-    from gym_lmaze_b200 import shard_range
-    for total in (1, 7, 4096, 1_000_000, 16_000_000):
-        for world in (1, 2, 3, 4, 8):
-            spans = [shard_range(total, r, world) for r in range(world)]
-            assert spans[0][0] == 0 and spans[-1][1] == total
-            assert all(spans[i][1] == spans[i + 1][0] for i in range(world - 1))
-            sizes = [hi - lo for lo, hi in spans]
-            assert max(sizes) - min(sizes) <= 1
-    with pytest.raises(ValueError):
-        shard_range(10, 3, 3)
-
-
 def test_missing_extension_fails_loudly(abi, monkeypatch):
     """No .so -> ImportError naming the build command; never a silent fallback."""
     monkeypatch.setattr(abi, "_lib", None)
@@ -157,7 +144,7 @@ def test_missing_extension_fails_loudly(abi, monkeypatch):
 
 def test_shard_range_partitions_the_batch():
     """Contiguous global-id shards (SURVEY 8e): disjoint, ordered, covering, sizes differ by at most one."""
-    from hypothesis import given, settings, strategies as st
+    from hypothesis import example, given, settings, strategies as st
     from gym_lmaze_b200 import shard_range
 
     @settings(max_examples=200, deadline=None)
@@ -169,6 +156,9 @@ def test_shard_range_partitions_the_batch():
             assert lo <= hi == lo2 <= hi2
         sizes = [hi - lo for lo, hi in edges]
         assert max(sizes) - min(sizes) <= 1
+    for total in (1, 7, 4096, 1_000_000, 16_000_000):      # batch sizes in use, over the world sizes of one node
+        for world in (1, 2, 3, 4, 8):
+            check = example(total, world)(check)
     check()
     with pytest.raises(ValueError):
         shard_range(10, 3, 3)
