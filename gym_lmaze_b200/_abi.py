@@ -14,6 +14,7 @@ RENDER_TMA, RENDER_ST128, RENDER_INCREMENTAL = 0, 1, 2
 OBS_FULL, OBS_COMPACT, OBS_BITS = 0, 1, 2
 NUM_STATS = 8
 SPAWN_FORCE = 64          # LMZ_SPAWN_FORCE
+OBS_MEM_COMPRESSIBLE = 1  # LMZ_OBS_MEM_COMPRESSIBLE
 STAT_NAMES = ("steps", "episodes", "goals", "timeouts", "wall_bumps", "moves", "stale", "eplen_sum")
 STATE_COLS = ("x", "y", "goal_x", "goal_y", "step_count", "reward_code", "goal_count", "episode")
 STATE_COLS_HIER = ("x", "y", "prev_x", "prev_y", "fovea_x1", "fovea_y1", "goal_x", "goal_y", "fgoal_x", "fgoal_y",
@@ -63,6 +64,8 @@ _PROTOTYPES = {
     "lmz_set_window_dl": [_vp, _vp, _i64],
     "lmz_create": [ctypes.POINTER(LmzConfig), ctypes.POINTER(_vp)],
     "lmz_destroy": [_vp],
+    "lmz_alloc_obs": [_i32, _i64, _i32, ctypes.POINTER(_vp), ctypes.POINTER(_i64)],
+    "lmz_free_obs": [_vp],
     "lmz_bind": [_vp, _vp, _vp, _vp],
     "lmz_bind_dl": [_vp, _vp, _vp, _vp],
     "lmz_reset": [_vp, _vp, _vp, _vp],
@@ -149,6 +152,40 @@ def dl(tensor):
         return None, None
     capsule = tensor.__dlpack__()
     return _PyCapsule_GetPointer(capsule, b"dltensor"), capsule
+
+
+_TYPESTR = {"torch.float32": "<f4", "torch.uint8": "|u1"}     # the observation dtypes
+
+
+class _ObsMemory(object):
+    """One lmz_alloc_obs allocation, shown to torch through __cuda_array_interface__.  torch holds this object for as
+    long as any tensor or view of the memory lives; dropping the last one returns the memory at once (lmz_free_obs),
+    whatever became of the env handle it was bound to."""
+
+    def __init__(self, lib, device, shape, dtype, compressible):
+        nbytes = dtype.itemsize
+        for d in shape:
+            nbytes *= int(d)
+        ptr, granted = ctypes.c_void_p(), ctypes.c_int64()
+        check(lib.lmz_alloc_obs(device, nbytes, OBS_MEM_COMPRESSIBLE if compressible else 0, ctypes.byref(ptr),
+                                ctypes.byref(granted)))
+        self._free, self.ptr, self.compressed_bytes = lib.lmz_free_obs, ptr.value, granted.value
+        self.__cuda_array_interface__ = {"shape": tuple(int(d) for d in shape), "typestr": _TYPESTR[str(dtype)],
+                                         "data": (ptr.value, False), "version": 2}
+
+    def __del__(self):
+        self._free(self.ptr)
+
+
+def obs_empty(shape, dtype, device, compressible):
+    """(tensor, compressed bytes): an uninitialised tensor like torch.empty(shape, dtype=dtype, device=device) in
+    memory from lmz_alloc_obs, compressible where the device and driver grant it."""
+    import torch
+    device = torch.device(device)
+    if device.index is None:
+        device = torch.device("cuda", torch.cuda.current_device())
+    mem = _ObsMemory(load(), device.index, shape, dtype, compressible)
+    return torch.as_tensor(mem, device=device), mem.compressed_bytes
 
 
 def call(fn, *args):

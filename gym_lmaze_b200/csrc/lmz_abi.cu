@@ -5,13 +5,16 @@
 // stream.  No torch types, no exceptions across the boundary, no hidden syncs on
 // the step path, and NO CPU implementation of the env -- if there is no CUDA
 // device lmz_create fails.
+#include <cuda.h>           // driver API types only: lmz_alloc_obs fetches its entry points at run time (no -lcuda)
 #include <cuda_runtime.h>
 
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <mutex>
 #include <new>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/lmaze_b200.h"
@@ -650,6 +653,120 @@ cudaError_t fill_u32(uint32_t *dst, size_t n, uint32_t value) {
   return e;
 }
 
+// ------------------------------------------------------------------ observation memory (lmz_alloc_obs)
+// The driver's virtual-memory calls, fetched through the runtime so that the library keeps linking cudart only.
+struct DriverVmm {
+  decltype(&cuDeviceGetAttribute) attribute = nullptr;
+  decltype(&cuMemGetAllocationGranularity) granularity = nullptr;
+  decltype(&cuMemCreate) create = nullptr;
+  decltype(&cuMemGetAllocationPropertiesFromHandle) properties = nullptr;
+  decltype(&cuMemAddressReserve) reserve = nullptr;
+  decltype(&cuMemMap) map = nullptr;
+  decltype(&cuMemSetAccess) set_access = nullptr;
+  decltype(&cuMemUnmap) unmap = nullptr;
+  decltype(&cuMemRelease) release = nullptr;
+  decltype(&cuMemAddressFree) address_free = nullptr;
+  bool ok = false;
+};
+
+const DriverVmm &vmm() {
+  static const DriverVmm d = [] {
+    DriverVmm v;
+    auto get = [](const char *name, auto &fn) {
+      void *p = nullptr;
+      cudaDriverEntryPointQueryResult q;
+      if (cudaGetDriverEntryPointByVersion(name, &p, 12000, cudaEnableDefault, &q) != cudaSuccess ||
+          q != cudaDriverEntryPointSuccess)
+        p = nullptr;
+      fn = reinterpret_cast<std::remove_reference_t<decltype(fn)>>(p);
+      return p != nullptr;
+    };
+    v.ok = get("cuDeviceGetAttribute", v.attribute) && get("cuMemGetAllocationGranularity", v.granularity) &&
+           get("cuMemCreate", v.create) && get("cuMemGetAllocationPropertiesFromHandle", v.properties) &&
+           get("cuMemAddressReserve", v.reserve) && get("cuMemMap", v.map) && get("cuMemSetAccess", v.set_access) &&
+           get("cuMemUnmap", v.unmap) && get("cuMemRelease", v.release) && get("cuMemAddressFree", v.address_free);
+    return v;
+  }();
+  return d;
+}
+
+// One lmz_alloc_obs allocation: `chunks` empty = cudaMalloc memory, else the physical chunks mapped back to back
+// from `ptr`.
+struct ObsAlloc {
+  void *ptr = nullptr;
+  int device = 0;
+  size_t size = 0;
+  std::vector<std::pair<CUmemGenericAllocationHandle, size_t>> chunks;
+};
+std::mutex g_obs_mu;
+std::vector<ObsAlloc> g_obs;
+
+void release_vmm(ObsAlloc &a) {
+  const DriverVmm &d = vmm();
+  const CUdeviceptr base = reinterpret_cast<CUdeviceptr>(a.ptr);
+  size_t off = 0;
+  for (const auto &c : a.chunks) {
+    d.unmap(base + off, c.second);
+    d.release(c.first);
+    off += c.second;
+  }
+  d.address_free(base, a.size);
+  a.chunks.clear();
+}
+
+// Compressible memory (cuMemCreate with generic compression) for `bytes`, rounded up to the granularity: physical
+// chunks of at most OBS_CHUNK_BYTES mapped into one reserved range.  Returns the bytes the driver made compressible;
+// on 0 nothing is kept and `a` is untouched.
+constexpr size_t OBS_CHUNK_BYTES = size_t(1) << 30;
+int64_t alloc_compressible(int device, size_t bytes, ObsAlloc &a) {
+  const DriverVmm &d = vmm();
+  int supported = 0;
+  if (!d.ok || d.attribute(&supported, CU_DEVICE_ATTRIBUTE_GENERIC_COMPRESSION_SUPPORTED, device) != CUDA_SUCCESS ||
+      !supported)
+    return 0;
+  CUmemAllocationProp prop;
+  memset(&prop, 0, sizeof(prop));
+  prop.type = CU_MEM_ALLOCATION_TYPE_PINNED;
+  prop.location.type = CU_MEM_LOCATION_TYPE_DEVICE;
+  prop.location.id = device;
+  prop.allocFlags.compressionType = CU_MEM_ALLOCATION_COMP_GENERIC;
+  size_t gran = 0;
+  if (d.granularity(&gran, &prop, CU_MEM_ALLOC_GRANULARITY_RECOMMENDED) != CUDA_SUCCESS || gran == 0) return 0;
+  ObsAlloc v;
+  v.device = device;
+  v.size = (bytes + gran - 1) / gran * gran;
+  CUdeviceptr base = 0;
+  if (d.reserve(&base, v.size, gran, 0, 0) != CUDA_SUCCESS) return 0;
+  v.ptr = reinterpret_cast<void *>(base);
+  int64_t granted = 0;
+  for (size_t off = 0; off < v.size;) {
+    const size_t sz = v.size - off < OBS_CHUNK_BYTES ? v.size - off : OBS_CHUNK_BYTES;
+    CUmemGenericAllocationHandle hd;
+    if (d.create(&hd, sz, &prop, 0) != CUDA_SUCCESS) break;
+    if (d.map(base + off, sz, 0, hd, 0) != CUDA_SUCCESS) {
+      d.release(hd);
+      break;
+    }
+    v.chunks.push_back({hd, sz});
+    CUmemAllocationProp got;
+    if (d.properties(&got, hd) == CUDA_SUCCESS && got.allocFlags.compressionType == CU_MEM_ALLOCATION_COMP_GENERIC)
+      granted += (int64_t)sz;
+    off += sz;
+  }
+  size_t mapped = 0;
+  for (const auto &c : v.chunks) mapped += c.second;
+  CUmemAccessDesc acc;
+  memset(&acc, 0, sizeof(acc));
+  acc.location = prop.location;
+  acc.flags = CU_MEM_ACCESS_FLAGS_PROT_READWRITE;
+  if (mapped != v.size || d.set_access(base, v.size, &acc, 1) != CUDA_SUCCESS || granted == 0) {
+    release_vmm(v);
+    return 0;
+  }
+  a = std::move(v);
+  return granted;
+}
+
 }  // namespace
 
 // ================================================================== exports
@@ -860,6 +977,51 @@ int lmz_destroy(lmz_env *h) {
   cudaFree(h->act_stage); cudaFree(h->visit); cudaFree(h->hist); cudaFree(h->aux2);
   release_pipe(h);
   delete h;
+  return LMZ_OK;
+}
+
+int lmz_alloc_obs(int32_t device, int64_t bytes, int32_t flags, void **ptr, int64_t *compressed_bytes) {
+  if (!ptr || bytes <= 0) return fail(LMZ_ERR_INVALID, "lmz_alloc_obs: ptr must not be NULL and bytes must be > 0");
+  if (flags & ~LMZ_OBS_MEM_COMPRESSIBLE) return fail(LMZ_ERR_INVALID, "lmz_alloc_obs: unknown flags 0x%x", flags);
+  *ptr = nullptr;
+  if (compressed_bytes) *compressed_bytes = 0;
+  int count = 0;
+  LMZ_CUDA(cudaGetDeviceCount(&count));
+  if (device < 0 || device >= count) return fail(LMZ_ERR_INVALID, "lmz_alloc_obs: no CUDA device %d", device);
+  DeviceGuard guard(device);
+  LMZ_CUDA(cudaFree(nullptr));      // the device's primary context, current for the driver calls
+  ObsAlloc a;
+  const int64_t granted = (flags & LMZ_OBS_MEM_COMPRESSIBLE) ? alloc_compressible(device, (size_t)bytes, a) : 0;
+  if (granted == 0) {               // not asked for, not supported, or refused: plain memory
+    a.device = device;
+    a.size = (size_t)bytes;
+    LMZ_CUDA(cudaMalloc(&a.ptr, a.size));
+  }
+  *ptr = a.ptr;
+  if (compressed_bytes) *compressed_bytes = granted;
+  std::lock_guard<std::mutex> lock(g_obs_mu);
+  g_obs.push_back(std::move(a));
+  return LMZ_OK;
+}
+
+int lmz_free_obs(void *ptr) {
+  if (!ptr) return LMZ_OK;
+  ObsAlloc a;
+  {
+    std::lock_guard<std::mutex> lock(g_obs_mu);
+    auto it = g_obs.begin();
+    while (it != g_obs.end() && it->ptr != ptr) ++it;
+    if (it == g_obs.end()) return fail(LMZ_ERR_INVALID, "lmz_free_obs: %p was not returned by lmz_alloc_obs", ptr);
+    a = std::move(*it);
+    g_obs.erase(it);
+  }
+  DeviceGuard guard(a.device);
+  if (a.chunks.empty()) {
+    LMZ_CUDA(cudaFree(a.ptr));
+    return LMZ_OK;
+  }
+  LMZ_CUDA(cudaDeviceSynchronize());      // as cudaFree does: work still writing the memory finishes first
+  release_vmm(a);
   return LMZ_OK;
 }
 

@@ -35,7 +35,7 @@ class LmazeHierCuda(LmazeVecCuda):
         # obs_mode="compact": both observations are the 5x5 crops before the x7 upsample (f32 [N,7,5,5] / [N,4,5,5])
         self.local_obs_shape = tuple(shape) if obs_mode == "full" else (shape[0], 5, 5)
         n, dev = self.num_envs, self.device
-        self.loc_obs = torch.zeros((n,) + self.local_obs_shape, dtype=torch.float32, device=dev)
+        self.loc_obs = self._obs_tensor((n,) + self.local_obs_shape, torch.float32).zero_()
         self.local_reward = torch.zeros(n, dtype=torch.float32, device=dev)
         self._ldone_u8 = torch.zeros(n, dtype=torch.uint8, device=dev)
         self.local_done = self._ldone_u8.view(torch.bool)

@@ -132,14 +132,35 @@ class LmazeVecCuda(_ReferenceSurface):
         if not (1 <= self.obs_window <= n):
             raise ValueError("obs_window must be in [1, num_envs]")
         self.window_lo = 0
-        self.obs = (torch.empty((self.obs_window,) + self.obs_shape, dtype=self.obs_dtype, device=self.device)
-                    if with_obs else None)
+        self._obs_compressed = False
+        self.obs = self._obs_tensor((self.obs_window,) + self.obs_shape, self.obs_dtype) if with_obs else None
         self.reward = torch.zeros(n, dtype=torch.float32, device=self.device)
         self._done_u8 = torch.zeros(n, dtype=torch.uint8, device=self.device)
         self.done = self._done_u8.view(torch.bool)
         self._bind()
 
     # ------------------------------------------------------------------ plumbing
+    def _obs_tensor(self, shape, dtype):
+        """An uninitialised observation tensor: compressible device memory for the modes whose kernels write it
+        faster there (DESIGN.md §2, observation memory), torch.empty for the others."""
+        if not self._compressible_obs():
+            return torch.empty(shape, dtype=dtype, device=self.device)
+        t, compressed_bytes = _abi.obs_empty(shape, dtype, self.device, True)
+        self._obs_compressed = compressed_bytes > 0
+        return t
+
+    def _compressible_obs(self):
+        # full renders write whole rows, about half of whose 128 B lines are all zeros: +12.5 % on the v0 step, +2 to
+        # +17 % on the other full renders.  The incremental kernel patches parts of lines, which compressed memory
+        # turns into read-modify-writes (-73 %); compact modes stay plain until each of their kernels is measured
+        return self.obs_mode == "full" and self.render_mode != "incremental"
+
+    @property
+    def obs_compressed(self):
+        """True when the observation tensors this env allocated are in compressible memory (the device and driver
+        granted it for this mode); a tensor bound by the caller is whatever the caller made it."""
+        return self._obs_compressed
+
     def _stream(self):
         return ctypes.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
 

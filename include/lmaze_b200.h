@@ -152,6 +152,17 @@ int         lmz_num_actions(int32_t variant);
 int lmz_create(const lmz_config *cfg, lmz_env **out);
 int lmz_destroy(lmz_env *env);
 
+/* ---- observation memory ---- */
+/* Device memory for an observation tensor, bound like any other buffer.  With LMZ_OBS_MEM_COMPRESSIBLE it is memory
+ * the L2 may keep compressed in DRAM (cuMemCreate with generic compression, on devices that support it): lossless and
+ * invisible to kernels, copies and DLPack consumers, and an observation is largely whole lines of zeros, so fewer
+ * bytes reach DRAM.  *compressed_bytes (may be NULL) returns how many bytes the driver made compressible; 0 means
+ * plain cudaMalloc memory (not asked for, not supported, or refused).  The memory belongs to the caller, not to any
+ * handle: lmz_destroy never frees it.  lmz_free_obs waits for the device, then releases it. */
+enum { LMZ_OBS_MEM_COMPRESSIBLE = 1 };
+int lmz_alloc_obs(int32_t device, int64_t bytes, int32_t flags, void **ptr, int64_t *compressed_bytes);
+int lmz_free_obs(void *ptr);
+
 /* Bind the output buffers every later call writes: obs (f32 [N,C,H,W], or u8 [N,C,G,G] in
  * compact mode; may be NULL: transition only, nothing rendered), reward f32 [N], done u8 [N].
  * obs must be 16-byte aligned. */
