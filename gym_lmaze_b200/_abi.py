@@ -62,6 +62,8 @@ _PROTOTYPES = {
     "lmz_num_actions": [_i32],
     "lmz_set_window": [_vp, _vp, _i64, _i64],
     "lmz_set_window_dl": [_vp, _vp, _i64],
+    "lmz_bind_final": [_vp, _vp, _i32],
+    "lmz_bind_final_dl": [_vp, _vp, _i32],
     "lmz_create": [ctypes.POINTER(LmzConfig), ctypes.POINTER(_vp)],
     "lmz_destroy": [_vp],
     "lmz_alloc_obs": [_i32, _i64, _i32, ctypes.POINTER(_vp), ctypes.POINTER(_i64)],

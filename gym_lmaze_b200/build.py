@@ -13,7 +13,7 @@ LIB_PATH = os.path.join(_PKG, "liblmaze_b200.so")
 SOURCES = [os.path.join(_PKG, "csrc", "lmz_abi.cu")]
 HEADERS = [os.path.join(_PKG, "csrc", "lmz_kernels.cuh"), os.path.join(_PKG, "csrc", "lmz_variants.h"),
            os.path.join(_PKG, "csrc", "lmz_v2.cuh"), os.path.join(_PKG, "csrc", "lmz_v5.cuh"), os.path.join(_PKG, "csrc", "lmz_fov.cuh"),
-           os.path.join(_PKG, "csrc", "lmz_fov_rollout.cuh"),
+           os.path.join(_PKG, "csrc", "lmz_fov_rollout.cuh"), os.path.join(_PKG, "csrc", "lmz_final.cuh"),
            os.path.join(_ROOT, "include", "lmaze_b200.h"), os.path.join(_ROOT, "include", "lmz_dlpack.h")]
 
 

@@ -21,6 +21,7 @@
 #include "lmz_kernels.cuh"
 #include "lmz_fov.cuh"
 #include "lmz_fov_rollout.cuh"
+#include "lmz_final.cuh"
 
 namespace {
 
@@ -251,7 +252,7 @@ struct lmz_env {
   uint8_t *done2, *loc_err, *fgoal_out;
   bool local_bound;
   unsigned char *blob;
-  unsigned long long *stats;     // NUM_STATS counters + 1 error counter + 2 work-distribution words
+  unsigned long long *stats;     // NUM_STATS counters + 1 error counter + 2 work-distribution words + 1 scratch word
   void *act_stage;               // lmz_step_host staging, lazily allocated (N * 8 bytes)
   // bound outputs (caller-owned)
   void *obs;                     // f32 [win_n][C][S][S] or u8 [win_n][C][G][G]
@@ -260,6 +261,8 @@ struct lmz_env {
   bool bound;
   int64_t win_lo, win_n;         // obs rows hold envs [win_lo, win_lo + win_n)
   bool obs_synced;               // incremental render: obs currently holds a full render of the window
+  void *final_obs;               // lmz_bind_final: terminal rows of the envs that finish in a step (caller-owned), or null
+  int32_t final_mode;            // LMZ_OBS_COMPACT or LMZ_OBS_BITS
   int n_cand, s_cell, x_cell;
   uint64_t rollout_t;            // rollout steps taken so far (keys the action RNG)
   int64_t launches;
@@ -527,6 +530,42 @@ int launch_fov_rollout(lmz_env *h, const lmz::KParams &p, cudaStream_t s) {
   const int fit = resident_ctas<kern>(h, THREADS, SMEM, false, "foveal rollout kernel");
   if (fit < 0) return fit;
   return launch(h, kern, persistent_grid(h, fit, ceil_div(p.n, THREADS)), THREADS, SMEM, s, p);
+}
+
+// The final-observation pre-pass of lmz_step (lmz_final.cuh): a plain grid of 4-warp CTAs, FINAL_TILES tiles per warp
+int launch_final(lmz_env *h, const void *actions, int32_t action_dtype, cudaStream_t s) {
+  constexpr int THREADS = 128;
+  lmz::FinalParams f;
+  memset(&f, 0, sizeof(f));
+  f.n = h->cfg.num_envs;
+  f.state = h->state; f.aux = h->goal_count; f.hist = h->hist; f.visit = h->visit;
+  f.actions = actions; f.action_dtype = action_dtype;
+  f.out = h->final_obs; f.bits = h->final_mode == LMZ_OBS_BITS;
+  f.blob = h->blob;
+  f.scratch = reinterpret_cast<unsigned int *>(h->stats + lmz::NUM_STATS + 3);
+  const int64_t grid = ceil_div(ceil_div(f.n, 32), (THREADS / 32) * lmz::FINAL_TILES);
+  switch (h->cfg.variant) {
+    case LMZ_V0: return launch(h, lmz::lmz_final_kernel<lmz::V0, THREADS>, grid, THREADS, 0, s, f);
+    case LMZ_V3: return launch(h, lmz::lmz_final_kernel<lmz::V3, THREADS>, grid, THREADS, 0, s, f);
+    case LMZ_V2:
+      return launch(h, lmz::lmz_final_fov_kernel<lmz::V2, THREADS>, grid, THREADS, (int)lmz::final_fov_smem<lmz::V2>(), s, f);
+    default:
+      return launch(h, lmz::lmz_final_fov_kernel<lmz::V4, THREADS>, grid, THREADS, (int)lmz::final_fov_smem<lmz::V4>(), s, f);
+  }
+}
+
+// what lmz_bind_final refuses whatever the buffer
+int check_final(const lmz_env *h, int32_t mode) {
+  if (h->var->hier) return fail(LMZ_ERR_UNSUPPORTED, "lmz_bind_final is not built for lmaze-v5/v6");
+  if (!h->cfg.autoreset)
+    return fail(LMZ_ERR_STATE, "lmz_bind_final needs autoreset: without it the step itself returns the terminal observation");
+  if (mode == LMZ_OBS_FULL)
+    return fail(LMZ_ERR_UNSUPPORTED, "final observations are compact or bit-packed rows (the full image is their exact "
+                "xE replication)");
+  if (mode != LMZ_OBS_COMPACT && mode != LMZ_OBS_BITS) return fail(LMZ_ERR_INVALID, "unknown final_mode %d", mode);
+  if (mode == LMZ_OBS_BITS && !h->var->bits_bytes)
+    return fail(LMZ_ERR_UNSUPPORTED, "bit-packed observations exist for the full-view variants (v0, v3) only");
+  return LMZ_OK;
 }
 
 int check_handle(lmz_env *h) {
@@ -929,7 +968,7 @@ int lmz_create(const lmz_config *cfg, lmz_env **out) {
   alloc_zero(&h->state, n32 * sizeof(uint32_t));
   alloc_zero(&h->goal_count, n32 * sizeof(uint32_t));
   alloc_zero(&h->episode, n * sizeof(uint32_t));
-  alloc_zero(&h->stats, (lmz::NUM_STATS + 3) * sizeof(unsigned long long));
+  alloc_zero(&h->stats, (lmz::NUM_STATS + 4) * sizeof(unsigned long long));
   if (v->hier) alloc_zero(&h->aux2, n32 * sizeof(uint32_t));
   if (v->has_visit) {
     alloc_zero(&h->visit, n * 324 * sizeof(float));     // state[2], the float visit layer (lmaze_env_v4.py:106-113)
@@ -1036,13 +1075,13 @@ int lmz_bind(lmz_env *h, void *obs, float *reward, uint8_t *done) {
   return LMZ_OK;
 }
 
-static int check_obs_dl(lmz_env *h, DLManagedTensor *obs, int64_t rows, void **po) {
+static int check_obs_dl(lmz_env *h, DLManagedTensor *obs, int64_t rows, int32_t obs_mode, const char *name, void **po) {
   int64_t shape[3];
   int32_t elem = 0;
-  if (int rc = lmz_obs_desc(h->cfg.variant, h->cfg.obs_mode, shape, &elem)) return rc;
+  if (int rc = lmz_obs_desc(h->cfg.variant, obs_mode, shape, &elem)) return rc;
   // f32 [rows][C][side][side] or u8 [rows][C][G][G]; bit-packed rows are u8 [rows][bytes]
-  const bool bits = h->cfg.obs_mode == LMZ_OBS_BITS;
-  const Want w{"obs", elem == 4 ? (uint8_t)kDLFloat : (uint8_t)kDLUInt, (uint8_t)(8 * elem), bits ? 2 : 4,
+  const bool bits = obs_mode == LMZ_OBS_BITS;
+  const Want w{name, elem == 4 ? (uint8_t)kDLFloat : (uint8_t)kDLUInt, (uint8_t)(8 * elem), bits ? 2 : 4,
                {rows, shape[0], shape[1], shape[2]}, 16};
   return check_dl(h, obs, w, po);
 }
@@ -1052,7 +1091,7 @@ int lmz_bind_dl(lmz_env *h, DLManagedTensor *obs, DLManagedTensor *reward, DLMan
   const int64_t n = h->cfg.num_envs;
   void *po = nullptr, *pr = nullptr, *pd = nullptr;
   if (obs)
-    if (int rc = check_obs_dl(h, obs, n, &po)) return rc;
+    if (int rc = check_obs_dl(h, obs, n, h->cfg.obs_mode, "obs", &po)) return rc;
   if (int rc = check_dl(h, reward, per_env(h, "reward", kDLFloat, 32), &pr)) return rc;
   if (int rc = check_dl(h, done, per_env(h, "done", kDLUInt, 8), &pd)) return rc;
   return lmz_bind(h, po, static_cast<float *>(pr), static_cast<uint8_t *>(pd));
@@ -1078,8 +1117,29 @@ int lmz_set_window_dl(lmz_env *h, DLManagedTensor *obs, int64_t env_lo) {
   if (obs->dl_tensor.ndim < 1) return fail(LMZ_ERR_INVALID, "obs: ndim %d, want 4", obs->dl_tensor.ndim);
   const int64_t rows = obs->dl_tensor.shape[0];
   void *po = nullptr;
-  if (int rc = check_obs_dl(h, obs, rows, &po)) return rc;
+  if (int rc = check_obs_dl(h, obs, rows, h->cfg.obs_mode, "obs", &po)) return rc;
   return lmz_set_window(h, po, env_lo, rows);
+}
+
+int lmz_bind_final(lmz_env *h, void *final_obs, int32_t final_mode) {
+  if (int rc = check_handle(h)) return rc;
+  if (!final_obs) {
+    h->final_obs = nullptr;
+    return LMZ_OK;
+  }
+  if (int rc = check_final(h, final_mode)) return rc;
+  if ((reinterpret_cast<uintptr_t>(final_obs) & 15u) != 0) return fail(LMZ_ERR_INVALID, "final_obs must be 16-byte aligned");
+  h->final_obs = final_obs; h->final_mode = final_mode;
+  return LMZ_OK;
+}
+
+int lmz_bind_final_dl(lmz_env *h, DLManagedTensor *final_obs, int32_t final_mode) {
+  if (int rc = check_handle(h)) return rc;
+  if (!final_obs) return lmz_bind_final(h, nullptr, final_mode);
+  if (int rc = check_final(h, final_mode)) return rc;
+  void *pf = nullptr;
+  if (int rc = check_obs_dl(h, final_obs, h->cfg.num_envs, final_mode, "final_obs", &pf)) return rc;
+  return lmz_bind_final(h, pf, final_mode);
 }
 
 int lmz_reset(lmz_env *h, const uint8_t *mask, const int32_t *spawn, void *stream) {
@@ -1115,6 +1175,8 @@ int lmz_step(lmz_env *h, const void *actions, int32_t action_dtype, const int32_
   lmz::KParams p = base_params(h);
   p.mode = lmz::MODE_STEP; p.actions = actions; p.action_dtype = action_dtype;
   p.spawn = reinterpret_cast<const int4 *>(spawn);
+  if (h->final_obs)     // the terminal rows, from the state words this step starts from
+    if (int rc = launch_final(h, actions, action_dtype, static_cast<cudaStream_t>(stream))) return rc;
   return launch_env(h, p, static_cast<cudaStream_t>(stream));
 }
 
@@ -1164,6 +1226,9 @@ int lmz_step_host_async(lmz_env *h, const void *actions_host, int32_t action_dty
   if (!actions_host || !reward_host || !done_host || !ticket) return fail(LMZ_ERR_INVALID, "host buffers / ticket must not be NULL");
   if (int rc = check_action_dtype(action_dtype, "action dtype")) return rc;
   if (h->var->hier) return fail(LMZ_ERR_UNSUPPORTED, "lmz_step_host_async is not built for lmaze-v5/v6");
+  if (h->final_obs)
+    return fail(LMZ_ERR_UNSUPPORTED, "lmz_step_host_async does not write final observations: unbind them first "
+                "(lmz_bind_final with NULL)");
   if (obs_host && h->cfg.obs_mode == LMZ_OBS_FULL)
     return fail(LMZ_ERR_UNSUPPORTED, "the full f32 observation is not double-buffered (2 x N x %zu bytes of HBM): a host "
                 "consumer takes obs_mode compact or bits; pass obs_host = NULL to keep the observation on the device",

@@ -66,7 +66,7 @@ class LmazeVecCuda(_ReferenceSurface):
 
     def __init__(self, num_envs=1, variant="v0", device=None, seed=0, autoreset=True, render_mode="tma",
                  env_id0=0, random_ball=True, random_goal=True, with_obs=True, tune=None, obs_mode="full",
-                 obs_window=None):
+                 obs_window=None, final_obs=False):
         if variant not in _VARIANTS:
             raise ValueError("unknown variant %r (built: v0, v2, v3, v4; v5/v6 through LmazeHierCuda)" % (variant,))
         if _VARIANTS[variant][2] != self._batched:
@@ -75,6 +75,8 @@ class LmazeVecCuda(_ReferenceSurface):
             raise ValueError("render_mode must be 'tma', 'st128' or 'incremental'")
         if obs_mode not in _OBS_MODE:
             raise ValueError("obs_mode must be 'full', 'compact' or 'bits'")
+        if final_obs and not autoreset:
+            raise ValueError("final_obs needs autoreset: without it step() itself returns the terminal observation")
         self._lib = _abi.load()          # raises if the CUDA extension is missing: no fallback
         if not torch.cuda.is_available():
             raise RuntimeError("LmazeVecCuda needs a CUDA device; gym_lmaze_b200 has no CPU path")
@@ -138,6 +140,15 @@ class LmazeVecCuda(_ReferenceSurface):
         self._done_u8 = torch.zeros(n, dtype=torch.uint8, device=self.device)
         self.done = self._done_u8.view(torch.bool)
         self._bind()
+        # terminal observations of the envs that finish in a step (lmz_bind_final): compact rows, or bit-packed rows
+        # in obs_mode "bits", one per env of the batch; expand(final_obs[idx]) gives the reference image
+        self.final_obs = None
+        if final_obs:
+            mode = _abi.OBS_BITS if obs_mode == "bits" else _abi.OBS_COMPACT
+            _abi.check(self._lib.lmz_obs_desc(self.variant, mode, ctypes.byref(shape), None))
+            row = (int(shape[0]),) if obs_mode == "bits" else tuple(shape)
+            self.final_obs = torch.empty((n,) + row, dtype=torch.float32 if foveal else torch.uint8, device=self.device)
+            _abi.call(self._lib.lmz_bind_final_dl, self._h, self.final_obs, mode)
 
     # ------------------------------------------------------------------ plumbing
     def _obs_tensor(self, shape, dtype):
@@ -268,9 +279,17 @@ class LmazeVecCuda(_ReferenceSurface):
         batched form of the reference returning `msg` as its 4th element
         (lmaze_env.py:237).  With autoreset the obs rows of finished envs already
         show the next episode's first observation.
+
+        With final_obs=True `info` also holds "final_obs" (the observation each finished env ended in, valid in the rows
+        where done is set), "_final_obs" (= done), "terminated" (done at the goal, reward 100) and "truncated" (done
+        at the step limit).
         """
         actions = self._step(actions, spawn)
-        return self.obs, self.reward, self.done, {"action": actions}
+        if self.final_obs is None:
+            return self.obs, self.reward, self.done, {"action": actions}
+        terminated = self.done & (self.reward == 100.0)
+        return self.obs, self.reward, self.done, {"action": actions, "final_obs": self.final_obs, "_final_obs": self.done,
+                                                  "terminated": terminated, "truncated": self.done & ~terminated}
 
     def _step(self, actions, spawn):
         """Launch the fused step; returns the actions as the kernel read them."""
@@ -369,6 +388,8 @@ class LmazeVecCuda(_ReferenceSurface):
 
     def host_pipeline(self, with_obs=True):
         """Double-buffered end-to-end stepping for a HOST consumer (lmz_step_host_async / lmz_step_host_wait)."""
+        if self.final_obs is not None:
+            raise ValueError("the host pipeline does not write final observations: construct the env with final_obs=False")
         return HostPipeline(self, with_obs)
 
     def render_obs(self):

@@ -176,6 +176,26 @@ int lmz_bind_dl(lmz_env *env, DLManagedTensor *obs, DLManagedTensor *reward, DLM
 int lmz_set_window(lmz_env *env, void *obs, int64_t env_lo, int64_t env_count);
 int lmz_set_window_dl(lmz_env *env, DLManagedTensor *obs, int64_t env_lo);
 
+/* Final observations under auto-reset.  With autoreset an env that finishes is re-spawned inside the step, and its
+ * obs row already shows the next episode; the observation the episode ENDED in -- what a learner bootstraps a
+ * truncated episode from -- goes to the final-observation buffer bound here, one row per env of the handle (all envs,
+ * not only the render window).
+ *   - lmz_step (and lmz_step_host, and graph replays of lmz_step) writes the row of every env whose done flag is raised
+ *     in that step, and only those rows: the observation the step would have returned with autoreset off (the
+ *     terminal state, before the re-spawn).  Other rows are left untouched; the caller's mask is `done`.
+ *   - Row format: the un-expanded form of lmz_obs_desc(variant, final_mode) -- LMZ_OBS_COMPACT: u8 [N,C,G,G] (v0, v3)
+ *     or f32 [N,C,5,5] (v2, v4); LMZ_OBS_BITS: u8 [N,R] (v0, v3).  LMZ_OBS_FULL is refused: the reference image is
+ *     the exact xE replication of a compact row.
+ *   - lmz_reset, lmz_render and the rollouts do not write it; lmz_step_host_async fails with LMZ_ERR_UNSUPPORTED
+ *     while a buffer is bound.
+ *   - Refused: LMZ_ERR_STATE without autoreset (the step returns the terminal observation itself); LMZ_ERR_UNSUPPORTED
+ *     for lmaze-v5/v6 and for a mode the variant lacks (bits on v2/v4, full anywhere); LMZ_ERR_INVALID for a bad
+ *     pointer, dtype, shape or alignment (16 bytes).  final_obs NULL unbinds.
+ * The rows come from a pre-pass kernel enqueued before the step kernel (it re-runs the deterministic transition on
+ * the same state and actions), so the step costs more only while a buffer is bound. */
+int lmz_bind_final(lmz_env *env, void *final_obs, int32_t final_mode);
+int lmz_bind_final_dl(lmz_env *env, DLManagedTensor *final_obs, int32_t final_mode);
+
 /* reset(): replaces LmazeEnv.reset (lmaze_env.py:64-141) / LmazeEnv_v3.reset
  * (lmaze_env_v3.py:134-206) for every env whose mask byte is non-zero (mask NULL =
  * all).  spawn NULL => device RNG; else int32 [N][4] = ball_x, ball_y, goal_x,
