@@ -413,6 +413,7 @@ int launch_env_v(lmz_env *h, const lmz::KParams &p, cudaStream_t s) {
     if (rc == LMZ_OK && (p.mode != lmz::MODE_RESET || p.mask == nullptr)) h->obs_synced = true;
     return rc;
   }
+  // tune[0] is one of cta_sizes() (lmz_create): the default branches take 0 and the default size
   if (h->cfg.render_mode == LMZ_RENDER_ST128) {
     if (h->cfg.tune[0] == 512) return launch_env_t<V, lmz::RENDER_ST128, 512>(h, p, s);
     if (h->cfg.tune[0] == 256) return launch_env_t<V, lmz::RENDER_ST128, 256>(h, p, s);
@@ -424,6 +425,34 @@ int launch_env_v(lmz_env *h, const lmz::KParams &p, cudaStream_t s) {
     case 256: return launch_env_t<V, lmz::RENDER_TMA, 256>(h, p, s);
     default: return launch_env_t<V, lmz::RENDER_TMA, TMA_THREADS>(h, p, s);
   }
+}
+
+// The CTA sizes (tune[0]) built for the kernel that renders the observation a config asks for; 0 = the default.
+// Launches with nothing to render (no obs bound) run their kernel's default CTA size whatever tune[0] says.
+struct CtaSizes {
+  const char *kernel;
+  int count;
+  int threads[8];
+};
+
+CtaSizes cta_sizes(const lmz_config *cfg, const VariantInfo *v) {
+  if (v->foveal && cfg->obs_mode == LMZ_OBS_COMPACT) return {"foveal compact kernel", 4, {0, 64, 128, 256}};
+  if (v->foveal) return {"foveal render kernel", 8, {0, 128, 160, 192, 224, 256, 512, 1024}};
+  if (cfg->obs_mode != LMZ_OBS_FULL) return {"compact / bit-packed kernel", 1, {0}};
+  if (cfg->render_mode == LMZ_RENDER_INCREMENTAL) return {"incremental render", 1, {0}};
+  if (cfg->render_mode == LMZ_RENDER_ST128) return {"ST128 render kernel", 4, {0, 256, 512, 1024}};
+  return {"TMA render kernel", 5, {0, 32, 64, 128, 256}};
+}
+
+int check_cta_size(const lmz_config *cfg, const VariantInfo *v) {
+  const CtaSizes c = cta_sizes(cfg, v);
+  for (int i = 0; i < c.count; ++i)
+    if (cfg->tune[0] == c.threads[i]) return LMZ_OK;
+  char list[64] = "";
+  for (int i = 0, len = 0; i < c.count; ++i)
+    len += snprintf(list + len, sizeof(list) - len, "%s%d", i ? ", " : "", c.threads[i]);
+  return fail(LMZ_ERR_INVALID, "tune[0] = %d: the %s of this variant / obs_mode / render_mode is built for tune[0] in "
+              "{%s} (0: default)", cfg->tune[0], c.kernel, list);
 }
 
 // default CTA size of the foveal render kernel per variant (1 producer warp + the rendering warps)
@@ -448,6 +477,7 @@ int launch_fov(lmz_env *h, const lmz::KParams &p, cudaStream_t s) {
   // v2 with ONE 128-thread CTA per SM (1 producer warp + 3 rendering warps) streams 7.47 TB/s, the pure-write
   // ceiling, against 7.0 TB/s with 1024 threads and 6.3 TB/s with two 128-thread CTAs per SM.  v4 / v5 run the
   // same organisation since round 2 (the scaled visit layer needs no producer warps of its own).
+  // tune[0] is 0 or one of the sizes below (lmz_create refuses any other)
   const int t = h->cfg.tune[0] ? h->cfg.tune[0] : LMZ_FOV_THREADS(W::ID);
   switch (t) {
     case 128: return launch_fov_t<W, 128>(h, p, s);
@@ -459,7 +489,7 @@ int launch_fov(lmz_env *h, const lmz::KParams &p, cudaStream_t s) {
     case 1024: return launch_fov_t<W, 1024>(h, p, s);
     default: break;
   }
-  return fail(LMZ_ERR_INVALID, "foveal kernels are built for tune[0] = 128, 160, 192, 224, 256, 512 or 1024 threads (got %d)", t);
+  return fail(LMZ_ERR_INVALID, "LMZ_FOV_THREADS(%d) = %d: no foveal render kernel is built for it", W::ID, t);
 }
 
 // compact observations / nothing to render (foveal variants): warp-granular kernel, several small CTAs per SM
@@ -480,8 +510,10 @@ int launch_fov_small_t(lmz_env *h, const lmz::KParams &p, cudaStream_t s) {
 
 template <class W>
 int launch_fov_small(lmz_env *h, const lmz::KParams &p, cudaStream_t s) {
-  if (h->cfg.tune[0] == 64) return launch_fov_small_t<W, 64>(h, p, s);       // (tuning: 2 warps per CTA)
-  if (h->cfg.tune[0] == 256) return launch_fov_small_t<W, 256>(h, p, s);     // (tuning: 8 warps per CTA)
+  // tune[0] sizes this kernel only where it renders the configured (compact) observation
+  const int t = h->cfg.obs_mode == LMZ_OBS_COMPACT ? h->cfg.tune[0] : 0;
+  if (t == 64) return launch_fov_small_t<W, 64>(h, p, s);       // (tuning: 2 warps per CTA)
+  if (t == 256) return launch_fov_small_t<W, 256>(h, p, s);     // (tuning: 8 warps per CTA)
   return launch_fov_small_t<W, 128>(h, p, s);
 }
 
@@ -927,9 +959,7 @@ int lmz_create(const lmz_config *cfg, lmz_env **out) {
   if (cfg->obs_mode == LMZ_OBS_BITS && !v->bits_bytes)
     return fail(LMZ_ERR_UNSUPPORTED, "bit-packed observations exist for the full-view variants (v0, v3) only");
   {
-    const int t = cfg->tune[0];
-    if (t < 0 || t > 1024 || (t & 31))
-      return fail(LMZ_ERR_INVALID, "tune[0] (threads per CTA) must be 0 or a multiple of 32 up to 1024");
+    if (int rc = check_cta_size(cfg, v)) return rc;
     if (cfg->tune[1] < 0 || cfg->tune[1] > 4) return fail(LMZ_ERR_INVALID, "tune[1] (L2 policy) must be 0..4");
     if (cfg->tune[2] < 0 || cfg->tune[2] > 32) return fail(LMZ_ERR_INVALID, "tune[2] (CTAs per SM cap) must be 0..32");
     if (cfg->tune[3] < 0 || (cfg->tune[3] & 15)) return fail(LMZ_ERR_INVALID, "tune[3] (bulk split) must be a multiple of 16");

@@ -98,9 +98,15 @@ typedef struct lmz_config {
   int32_t  random_goal;   /* RANDOM_GOAL  (lmaze_env_v3.py:104); ignored by v0 */
   int32_t  render_mode;   /* lmz_render_mode */
   int32_t  tune[4];       /* launch tuning for the TMA render path, 0 = library default:
-                             [0] threads per CTA (TMA path: 32/64/128/256 issuing warps x32; ST128 path: 256/512/1024;
-                                 foveal render kernels: 128 (default), 160, 192, 224, 256, 512, 1024;
-                                 compact foveal kernel: 64, 128 (default), 256)
+                             [0] threads per CTA of the kernel that renders the configured observation; lmz_create
+                                 refuses (LMZ_ERR_INVALID) a size that kernel is not built for:
+                                   v0/v3 full, TMA: 32 (default), 64, 128, 256 (1, 2, 4 or 8 issuing warps);
+                                   v0/v3 full, ST128: 256, 512, 1024 (default);
+                                   v0/v3 incremental, compact or bits: 0 only;
+                                   v2/v4/v5 full: 128 (default), 160, 192, 224, 256, 512, 1024;
+                                   v2/v4/v5 compact: 64, 128 (default), 256.
+                                 Launches with nothing to render (no obs bound) keep their kernel's fixed default
+                                 shape whatever this says.
                              [1] L2 policy of the obs stores: 1 evict_first, 2 evict_normal, 3 evict_last, 4 none
                              [2] resident CTAs per SM (0 = library default)
                              [3] split bulk copies into pieces of at most this many bytes (multiple of 16) */
