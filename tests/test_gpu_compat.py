@@ -1,35 +1,30 @@
 """GPU tier: the single-maze compat classes replay the reference's golden traces in the reference's own
 types (numpy obs, Python-float reward, bool done, info = the action passed)."""
-import os
-
 import numpy as np
 import pytest
+
+from golden_io import Traces, unpack
 
 pytestmark = pytest.mark.gpu
 
 
-def unpack(bits, shape):
-    n = int(np.prod(shape))
-    return np.unpackbits(bits)[:n].reshape(shape).astype(np.float32)
-
-
 def test_lmaze_v0_drop_in(golden_dir):
     import gym_lmaze_b200 as g
-    z = np.load(os.path.join(golden_dir, "v0_traces.npz"))
+    tr = Traces(golden_dir, "v0")
     env = g.make("lmaze-v0")
     assert isinstance(env, g.LmazeEnv) and env.action_space.n == 4 and tuple(env.observation_space.shape) == (4, 84, 84)
-    for e in range(int(z["n_envs"])):
-        obs = env.reset(spawn=tuple(z["e%d_spawn0" % e]))
+    for e in range(tr.n_envs):
+        z = tr.env(e)
+        obs = env.reset(spawn=tuple(z["spawn0"]))
         assert isinstance(obs, np.ndarray) and obs.dtype == np.float32 and obs.shape == (4, 84, 84)
-        for t in range(len(z["e%d_actions" % e])):
-            a = int(z["e%d_actions" % e][t])
+        for t in range(tr.T):
+            a = int(z["actions"][t])
             obs, r, d, info = env.step(a)
-            ref_r = np.int64(z["e%d_reward_bits" % e][t]).view(np.float64)
-            assert type(r) is float and np.float64(r).view(np.int64) == np.float64(ref_r).view(np.int64), (e, t)
-            assert type(d) is bool and d == bool(z["e%d_done" % e][t]) and info == a
+            assert type(r) is float and np.float64(r).view(np.int64) == z["reward_bits"][t], (e, t)
+            assert type(d) is bool and d == bool(z["done"][t]) and info == a
             if d:
-                obs = env.reset(spawn=tuple(z["e%d_spawn" % e][t]))
-            assert np.array_equal(obs, unpack(z["e%d_obs" % e][t], (4, 84, 84))), (e, t)
+                obs = env.reset(spawn=tuple(z["spawn"][t]))
+            assert np.array_equal(obs, unpack(z["obs"][t], (4, 84, 84))), (e, t)
     # float / numeric-string actions go through int() like the reference (lmaze_env.py:148)
     env.reset(spawn=(3, 3))
     assert env.step(1.9)[3] == 1 and env.step("3")[3] == 3
@@ -38,22 +33,21 @@ def test_lmaze_v0_drop_in(golden_dir):
 
 def test_lmaze_v3_drop_in_takes_strings(golden_dir):
     import gym_lmaze_b200 as g
-    z = np.load(os.path.join(golden_dir, "v3_traces.npz"))
+    tr = Traces(golden_dir, "v3")
     env = g.make("lmaze-v3")
     spell = {0: ("left", "0"), 1: ("right", "1"), 2: ("up", "2"), 3: ("down", "3")}
     for e in range(2):
-        s0 = z["e%d_spawn0" % e]
-        env.reset(spawn=tuple(s0))
-        for t in range(len(z["e%d_actions" % e])):
-            code = int(z["e%d_actions" % e][t])
+        z = tr.env(e)
+        env.reset(spawn=tuple(z["spawn0"]))
+        for t in range(tr.T):
+            code = int(z["actions"][t])
             a = spell[code][t % 2] if code in spell else ("noop", 0, 3, "4")[t % 4]
             obs, r, d, info = env.step(a)
-            ref_r = np.int64(z["e%d_reward_bits" % e][t]).view(np.float64)
-            assert np.float64(r).view(np.int64) == np.float64(ref_r).view(np.int64) and d == bool(z["e%d_done" % e][t])
+            assert np.float64(r).view(np.int64) == z["reward_bits"][t] and d == bool(z["done"][t])
             assert info == a
             if d:
-                obs = env.reset(spawn=tuple(z["e%d_spawn" % e][t]))
-            assert np.array_equal(obs, unpack(z["e%d_obs" % e][t], (3, 72, 72))), (e, t)
+                obs = env.reset(spawn=tuple(z["spawn"][t]))
+            assert np.array_equal(obs, unpack(z["obs"][t], (3, 72, 72))), (e, t)
     o = env.reset(mode="test")
     assert env.state_vector[:4] == [7, 8, 8, 8] and o.shape == (3, 72, 72)
     env.close()
@@ -61,21 +55,21 @@ def test_lmaze_v3_drop_in_takes_strings(golden_dir):
 
 def test_lmaze_v2_v4_drop_in(golden_dir):
     import gym_lmaze_b200 as g
-    z = np.load(os.path.join(golden_dir, "v2_traces.npz"))
+    tr = Traces(golden_dir, "v2")
+    z = tr.env(0)
     env = g.make("lmaze-v2")
     assert env.action_space.n == 25 and tuple(env.observation_space.shape) == (5, 35, 35)
-    init = z["e0_init"]                                  # bx, by, gx, gy, layout, layout-before
+    init = z["init"]                                     # bx, by, gx, gy, layout, layout-before
     env._vec.set_state([[4, 4, 8, 8, 0, int(init[5]), 4 | (4 << 5), 0]])
     obs = env.reset(spawn=tuple(init[:5]))
-    assert np.array_equal(obs, unpack(z["e0_first_obs"], (5, 35, 35)))
-    for t in range(len(z["e0_actions"])):
-        a = int(z["e0_actions"][t])
+    assert np.array_equal(obs, unpack(z["first_obs"], (5, 35, 35)))
+    for t in range(tr.T):
+        a = int(z["actions"][t])
         obs, r, d, info = env.step(a)
-        ref_r = np.int64(z["e0_reward_bits"][t]).view(np.float64)
-        assert np.float64(r).view(np.int64) == np.float64(ref_r).view(np.int64) and d == bool(z["e0_done"][t]) and info == a
+        assert np.float64(r).view(np.int64) == z["reward_bits"][t] and d == bool(z["done"][t]) and info == a
         if d:
-            obs = env.reset(spawn=tuple(z["e0_spawn"][t]))
-        assert np.array_equal(obs, unpack(z["e0_obs"][t], (5, 35, 35))), t
+            obs = env.reset(spawn=tuple(z["spawn"][t]))
+        assert np.array_equal(obs, unpack(z["obs"][t], (5, 35, 35))), t
     with pytest.raises(IndexError):
         env.step(25)
     env.close()

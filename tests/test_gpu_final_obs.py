@@ -10,6 +10,8 @@ import numpy as np
 import pytest
 import torch
 
+from gpu_helpers import lmz, same_bytes
+
 pytestmark = pytest.mark.gpu
 
 THREADS = os.cpu_count() or 1
@@ -18,15 +20,6 @@ STEP_LIMIT_STEPS = {"v0": 100, "v3": 101, "v2": 51, "v4": 51}       # the step w
 NO_MOVE = {"v0": 7, "v3": 7, "v2": 12, "v4": 12}                     # an action that never reaches the goal
 CASES = [(v, m) for v in FULL_VIEW for m in ("tma", "st128", "incremental", "compact", "bits")] + \
         [(v, m) for v in ("v2", "v4") for m in ("full", "compact")]
-
-
-@pytest.fixture(scope="module")
-def lmz():
-    import gym_lmaze_b200 as g
-    from gym_lmaze_b200 import _abi
-    _abi.load()
-    assert torch.cuda.is_available()
-    return g
 
 
 def make(lmz, variant, mode, n, seed=0, **kw):
@@ -71,10 +64,6 @@ def stats_with_errors(env):
     return list(out), err.value
 
 
-def same_bits(a, b):
-    return torch.equal(a.view(torch.uint8), b.view(torch.uint8))
-
-
 # ---------------------------------------------------------------- 1 + 2: oracle parity, nothing else changes
 @pytest.mark.parametrize("variant,mode", CASES)
 def test_final_rows_match_oracle_terminal_obs(lmz, oracle_mod, variant, mode):
@@ -108,10 +97,10 @@ def test_final_rows_match_oracle_terminal_obs(lmz, oracle_mod, variant, mode):
             direct_done = direct_done or (variant == "v4" and t >= 30 and bool(d[0]))
         ora.reset_masked(d_ref)
         # the twin without a final buffer: every output and all state bit-identical
-        assert same_bits(obs, obs2) and same_bits(rew, rew2) and torch.equal(done, done2), t
+        assert same_bytes(obs, obs2) and same_bytes(rew, rew2) and torch.equal(done, done2), t
         assert torch.equal(env.get_state(), twin.get_state()), t
         if variant == "v4":
-            assert same_bits(env.get_visit(), twin.get_visit()), t
+            assert same_bytes(env.get_visit(), twin.get_visit()), t
         assert info["_final_obs"] is env.done and info["final_obs"] is env.final_obs
     assert finished >= N                                  # every env finished at least one episode
     assert stats_with_errors(env) == stats_with_errors(twin)
@@ -155,8 +144,8 @@ def test_synchronised_timeout_step_writes_every_row(lmz, variant, n):
     env.final_obs.view(torch.uint8).fill_(0xA5)
     _, _, done, info = env.step(a)
     assert bool(done.all()) and not bool(info["terminated"].any()) and bool(info["truncated"].all())
-    assert same_bits(env.final_obs, before)
-    assert not same_bits(env.obs, before)                 # the obs rows show the new episodes
+    assert same_bytes(env.final_obs, before)
+    assert not same_bytes(env.obs, before)                 # the obs rows show the new episodes
     env.close()
 
 
@@ -186,7 +175,7 @@ def test_graph_replay_and_step_host_write_final_rows(lmz, variant, mode):
         assert torch.equal(gr.done, done) and torch.equal(d_host.to(done.device).bool(), done), t
         m = done
         finished += int(m.sum())
-        assert same_bits(gr.final_obs[m], ref.final_obs[m]) and same_bits(host.final_obs[m], ref.final_obs[m]), t
+        assert same_bytes(gr.final_obs[m], ref.final_obs[m]) and same_bytes(host.final_obs[m], ref.final_obs[m]), t
     assert finished > 0
     for e in (ref, gr, host):
         e.close()

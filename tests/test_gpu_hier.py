@@ -3,77 +3,49 @@
 seeded inputs -- every returned value per call, bit for bit (both observation tensors, both rewards'
 bit patterns, both done flags, the IndexError flag, the packed state and the float visit layer).
 """
-import os
-
 import numpy as np
 import pytest
 import torch
 
+from golden_io import Traces, fov_image, loc_image, reward_f32_bits
+from gpu_helpers import lmz, need_free, u32
+
 pytestmark = pytest.mark.gpu
-
-
-@pytest.fixture(scope="module")
-def lmz():
-    import gym_lmaze_b200 as g
-    from gym_lmaze_b200 import _abi
-    _abi.load()
-    assert torch.cuda.is_available()
-    return g
-
-
-def f64(bits):
-    return np.int64(bits).view(np.float64)
-
-
-def u32(t):
-    if torch.is_tensor(t):
-        t = t.detach().cpu().numpy()
-    return np.ascontiguousarray(t).view(np.uint32)
-
-
-def fov_obs(bits, visit):
-    b = np.unpackbits(bits)[:125].reshape(5, 5, 5).astype(np.float32)
-    small = np.stack([b[0], b[1], visit[0], b[2], b[3], b[4], visit[1]])
-    return np.repeat(np.repeat(small, 7, 1), 7, 2)
-
-
-def loc_obs(bits):
-    small = np.unpackbits(bits)[:100].reshape(4, 5, 5).astype(np.float32)
-    return np.repeat(np.repeat(small, 7, 1), 7, 2)
 
 
 # ---------------------------------------------------------------- golden traces (reference outputs)
 @pytest.mark.parametrize("variant", ["v5", "v6", "v5_edge"])
 def test_hier_golden_traces(lmz, golden_dir, variant):
     """Every value the reference returned from reset / plannerStep / step over 4 x ~730 recorded events."""
-    z = np.load(os.path.join(golden_dir, variant + "_traces.npz"))
+    tr = Traces(golden_dir, variant)
     n_events = 0
-    for e in range(int(z["n_envs"])):
+    for e in range(tr.n_envs):
         env = lmz.LmazeHierCuda(1, variant[:2], autoreset=False)
-        ev = z["e%d_events" % e]
+        z = tr.env(e)
+        ev = z["events"]
         for k, row in enumerate(ev):
             kind, arg, grb, orb, gd, ld, bx, by = (int(v) for v in row[:8])
             sp = [int(v) for v in row[8:13]]
             if kind == 0:
                 fov = env.reset(spawn=[sp])
-                assert np.array_equal(u32(fov[0]), u32(fov_obs(z["e%d_fov_bits" % e][k], z["e%d_fov_visit" % e][k]))), (e, k)
+                assert np.array_equal(u32(fov[0]), u32(fov_image(z["fov_bits"][k], z["fov_visit"][k]))), (e, k)
             elif kind == 1:
                 loc = env.plannerStep([arg])
                 assert not bool(env.loc_err.item())
-                assert np.array_equal(u32(loc[0]), u32(loc_obs(z["e%d_loc_bits" % e][k]))), (e, k)
+                assert np.array_equal(u32(loc[0]), u32(loc_image(z["loc_bits"][k]))), (e, k)
             else:
                 fov, loc, gr, lr, gdo, ldo, fg, act = env.step([arg])
                 assert not bool(env.loc_err.item())
-                assert u32(gr)[0] == np.float32(f64(grb)).view(np.uint32), (e, k)
-                assert u32(lr)[0] == np.float32(f64(orb)).view(np.uint32), (e, k)
+                assert u32(gr)[0] == reward_f32_bits(grb), (e, k)
+                assert u32(lr)[0] == reward_f32_bits(orb), (e, k)
                 assert (int(gdo.item()), int(ldo.item())) == (gd, ld), (e, k)
-                assert np.array_equal(u32(fov[0]), u32(fov_obs(z["e%d_fov_bits" % e][k], z["e%d_fov_visit" % e][k]))), (e, k)
-                assert np.array_equal(u32(loc[0]), u32(loc_obs(z["e%d_loc_bits" % e][k]))), (e, k)
+                assert np.array_equal(u32(fov[0]), u32(fov_image(z["fov_bits"][k], z["fov_visit"][k]))), (e, k)
+                assert np.array_equal(u32(loc[0]), u32(loc_image(z["loc_bits"][k]))), (e, k)
                 assert fg.shape == (1, 1, 5, 5) and float(fg.sum()) == 1.0 and int(act.item()) == arg
             st = env.get_state()[0].tolist()
             assert (st[0], st[1]) == (bx, by), (e, k)
             if k % 16 == 0 or kind == 0:
-                assert float(env.get_visit()[0].cpu().numpy().astype(np.float64).sum()) == z["e%d_visit_sum" % e][k], (e, k)
+                assert float(env.get_visit()[0].cpu().numpy().astype(np.float64).sum()) == z["visit_sum"][k], (e, k)
             n_events += 1
         assert env.stats()["steps"] == int((ev[:, 0] == 2).sum())
         env.close()
@@ -82,10 +54,10 @@ def test_hier_golden_traces(lmz, golden_dir, variant):
 
 def test_v6_safe_goal_golden(lmz, golden_dir, oracle_mod):
     """safeFovealGoal (lmaze_env_v6.py:505-523) with the reference's own np.random draws injected."""
-    z = np.load(os.path.join(golden_dir, "v6_traces.npz"))
-    rows = [str(r) for r in z["safe_layout"]]
+    tr = Traces(golden_dir, "v6")
+    rows = [str(r) for r in tr["safe_layout"]]
     k = [i for i in range(1, 6) if oracle_mod.layout_v2(i) == rows][0]
-    res = z["safe_results"]
+    res = tr["safe_results"]
     n = len(res)
     env = lmz.LmazeHierCuda(n, "v6", autoreset=False)
     env.reset()
@@ -96,7 +68,7 @@ def test_v6_safe_goal_golden(lmz, golden_dir, oracle_mod):
     draws = np.zeros((n, 40), np.int64)
     pos = 0
     for i, (bx, by, want, used) in enumerate(res):
-        chunk = z["safe_draws"][pos:pos + 40]
+        chunk = tr["safe_draws"][pos:pos + 40]
         draws[i, :len(chunk)] = chunk
         pos += int(used)
     goals, used = env.safeFovealGoal(draws)
@@ -211,10 +183,10 @@ def test_hier_state_roundtrip_and_render(lmz, oracle_mod):
 
 def test_hier_compat_classes(lmz, golden_dir):
     """LmazeEnv_v5 / LmazeEnv_v6 with the reference's exact call surface and return types."""
-    z = np.load(os.path.join(golden_dir, "v6_traces.npz"))
+    z = Traces(golden_dir, "v6").env(0)
     env = lmz.make("lmaze-v6")
     assert type(env).__name__ == "LmazeEnv_v6"
-    ev = z["e0_events"]
+    ev = z["events"]
     for k, row in enumerate(ev[:120]):
         kind, arg, grb, orb, gd, ld = (int(v) for v in row[:6])
         if kind == 0:
@@ -222,14 +194,14 @@ def test_hier_compat_classes(lmz, golden_dir):
             assert isinstance(fov, np.ndarray) and fov.shape == (7, 35, 35) and fov.dtype == np.float32
         elif kind == 1:
             loc = env.plannerStep(arg)
-            assert loc.shape == (4, 35, 35) and np.array_equal(loc, loc_obs(z["e0_loc_bits"][k]))
+            assert loc.shape == (4, 35, 35) and np.array_equal(loc, loc_image(z["loc_bits"][k]))
         else:
             out = env.step(arg)
             assert len(out) == 8
             assert isinstance(out[2], float) and np.float64(out[2]).view(np.int64) == grb
             assert isinstance(out[3], float) and np.float64(out[3]).view(np.int64) == orb
             assert out[4] is bool(gd) and out[5] is bool(ld) and out[6].shape == (1, 5, 5) and out[7] == arg
-            assert np.array_equal(u32(out[0]), u32(fov_obs(z["e0_fov_bits"][k], z["e0_fov_visit"][k])))
+            assert np.array_equal(u32(out[0]), u32(fov_image(z["fov_bits"][k], z["fov_visit"][k])))
     assert 0 <= env.safeFovealGoal() <= 24
     with pytest.raises(IndexError):
         env.plannerStep(25)
@@ -329,8 +301,7 @@ def test_hier_one_million_envs(lmz, oracle_mod):
     by the oracle from the same seeds (the device RNG is keyed by global env id), and size-independent
     properties hold over the whole batch."""
     N = 1 << 20
-    if torch.cuda.mem_get_info()[0] < N * 53900 + (6 << 30):
-        pytest.fail("B200 expected: need %d GiB free" % ((N * 53900 + (6 << 30)) >> 30))
+    need_free(N * 53900 + (6 << 30))
     seed, B = 4242, 384
     env = lmz.LmazeHierCuda(N, "v5", seed=seed, autoreset=True)
     blocks = [(0, oracle_mod.OracleHier(B, seed=seed, env_id0=0)), (N - B - 37, oracle_mod.OracleHier(B, seed=seed, env_id0=N - B - 37))]

@@ -18,9 +18,10 @@ import numpy as np
 import pytest
 import torch
 
+from gpu_helpers import lmz, need_free, same_bytes, sms
+
 PATTERN = 0x3C5AA5C3                           # sentinel word of the guard rows and of unwritten rows
 SEED, ID0, T = 5, 3, 120
-CH = 1 << 28                                   # int32 words per chunk of the whole-buffer comparisons
 ROWS = 1 << 14                                 # rows per chunk of the oracle comparisons
 GROUP = 7                                      # tuned handles beside one default handle
 BAND = {"v0": 2352, "v3": 1152}                # bytes of one ball band (V::BAND_BYTES)
@@ -44,35 +45,8 @@ N_GROUPS = (len(_points("v0")) + GROUP - 1) // GROUP
 assert N_GROUPS == (len(_points("v3")) + GROUP - 1) // GROUP
 
 
-@pytest.fixture(scope="module")
-def lmz():
-    import gym_lmaze_b200 as g
-    from gym_lmaze_b200 import _abi
-    _abi.load()
-    assert torch.cuda.is_available()
-    return g
-
-
-def _sms():
-    return torch.cuda.get_device_properties(0).multi_processor_count
-
-
-def _need(nbytes):
-    import gc
-    gc.collect()
-    torch.cuda.empty_cache()
-    free_b = torch.cuda.mem_get_info()[0]
-    if free_b < nbytes:
-        pytest.fail("B200 expected: %d GiB free, need %d GiB" % (free_b >> 30, nbytes >> 30))
-
-
 def _words(t):
     return t.view(torch.int32).reshape(-1)
-
-
-def _same(a, b):
-    a, b = _words(a), _words(b)
-    return all(torch.equal(a[lo:lo + CH], b[lo:lo + CH]) for lo in range(0, a.numel(), CH))
 
 
 class Guarded(object):
@@ -116,7 +90,7 @@ class Handle(object):
 def _compare(ref, h, what):
     """h's observation buffer (guard rows included), reward and done against the default handle's."""
     assert h.cur.guards_intact(), ("guard row overwritten",) + what
-    assert _same(h.cur.buf, ref.cur.buf), ("obs",) + what
+    assert same_bytes(h.cur.buf, ref.cur.buf), ("obs",) + what
     assert torch.equal(_words(h.env.reward), _words(ref.env.reward)), ("reward",) + what
     assert torch.equal(h.env._done_u8, ref.env._done_u8), ("done",) + what
 
@@ -220,7 +194,7 @@ def _sequence(ref, tuned, states, renders, n, graph=None, steps=T):
     a = actions()
     _lockstep(ref, tuned, lambda h: h.env.step(a), ("window step",), refill=True)
     for h in everyone:
-        assert h.full.guards_intact() and _same(h.full.buf, ref.full.buf), (h.point, "whole batch while windowed")
+        assert h.full.guards_intact() and same_bytes(h.full.buf, ref.full.buf), (h.point, "whole batch while windowed")
         h.window(None)
     a = actions()
     _lockstep(ref, tuned, lambda h: h.env.step(a), ("step after window",))
@@ -248,7 +222,7 @@ def _sequence(ref, tuned, states, renders, n, graph=None, steps=T):
 def _run(lmz, oracle_mod, variant, points, n, graph_point=None, steps=T):
     row_shape = (4, 84, 84) if variant == "v0" else (3, 72, 72)
     n_incr = sum(mode == "incremental" for mode, _ in points)
-    _need((len(points) + n_incr + 3) * (n + 2) * ROW_BYTES[variant] + (8 << 30))
+    need_free((len(points) + n_incr + 3) * (n + 2) * ROW_BYTES[variant] + (8 << 30))
     states, renders = _states(oracle_mod, variant)
     ref = Handle(lmz, variant, n, "tma", None, Guarded(n - 100, row_shape))
     win = Guarded(n - 100, row_shape)
@@ -268,7 +242,7 @@ def _run(lmz, oracle_mod, variant, points, n, graph_point=None, steps=T):
 def test_full_render_knobs_lockstep(lmz, oracle_mod, variant, group):
     """Every TMA, ST128 and incremental knob point of _points(variant), GROUP at a time beside one default handle."""
     pts = _points(variant)[group * GROUP:(group + 1) * GROUP]
-    _run(lmz, oracle_mod, variant, pts, 3 * _sms() * 8 * 32 + 21, GRAPH_POINT if GRAPH_POINT in pts else None)
+    _run(lmz, oracle_mod, variant, pts, 3 * sms() * 8 * 32 + 21, GRAPH_POINT if GRAPH_POINT in pts else None)
 
 
 @pytest.mark.gpu
@@ -276,7 +250,7 @@ def test_full_render_knobs_lockstep(lmz, oracle_mod, variant, group):
 def test_bulk_split_16_bytes(lmz, oracle_mod, variant):
     """tune[3] = 16, the smallest piece the ABI accepts (every segment cut into 16-byte copies), on a batch of about
     two tiles per issuing warp, and the same with 8 issuing warps per CTA."""
-    n = 2 * _sms() * 32 + 5
+    n = 2 * sms() * 32 + 5
     _run(lmz, oracle_mod, variant, [("tma", (0, 0, 0, 16)), ("tma", (256, 4, 0, 16))], n, steps=30)
 
 

@@ -15,48 +15,22 @@ import numpy as np
 import pytest
 import torch
 
+from gpu_helpers import REWARD_BITS, lmz, need_free, resident_threads, u32
 from oracle.oracle import STAT_NAMES
 from philox_np import ActionStream, rng_hier
 
 pytestmark = pytest.mark.gpu
 
-RC_BITS = np.array([0x80000000, 0xBF800000, 0xBC23D70A, 0x42C80000], dtype=np.uint32).view(np.int32)
 THREADS = os.cpu_count() or 1
 CH = 1 << 14                                   # rows per chunk of the whole-tensor checks on the device
-
-
-@pytest.fixture(scope="module")
-def lmz():
-    import gym_lmaze_b200 as g
-    from gym_lmaze_b200 import _abi
-    _abi.load()
-    assert torch.cuda.is_available()
-    return g
-
-
-def u32(t):
-    return (t.detach().cpu().numpy() if torch.is_tensor(t) else t).view(np.uint32)
 
 
 def i32(t):
     return t.view(torch.int32) if t.dtype == torch.float32 else t
 
 
-def _need(nbytes):
-    import gc
-    gc.collect()
-    torch.cuda.empty_cache()
-    free_b = torch.cuda.mem_get_info()[0]
-    if free_b < nbytes:
-        pytest.fail("B200 expected: %d GiB free, need %d GiB" % (free_b >> 30, nbytes >> 30))
-
-
-def _resident():
-    return torch.cuda.get_device_properties(0).multi_processor_count * 2048
-
-
 def _multi(k=2, tail=21):
-    R = _resident()
+    R = resident_threads()
     N = k * R + tail
     assert N >= k * R
     return N
@@ -135,7 +109,7 @@ def test_compact_bits_transition_incremental_multitile(lmz, oracle_mod, variant)
     O = oracle_mod
     N, T, seed, id0 = _multi(), 130, 41, 7
     ov = O.V0 if variant == "v0" else O.V3
-    _need(N * 4 * int(np.prod(O.OBS_SHAPE[ov])) + (8 << 30))
+    need_free(N * 4 * int(np.prod(O.OBS_SHAPE[ov])) + (8 << 30))
     ora = _oracle(O, ov, N, seed=seed, env_id0=id0)
 
     def mk(**kw):
@@ -193,7 +167,7 @@ def test_foveal_step_kernels_multitile(lmz, oracle_mod, variant):
     O = oracle_mod
     N, T, seed, id0 = _multi(), 130, 23, 1000
     ov = O.V2 if variant == "v2" else O.V4
-    _need(2 * N * 4 * int(np.prod(O.OBS_SHAPE[ov])) + (8 << 30))
+    need_free(2 * N * 4 * int(np.prod(O.OBS_SHAPE[ov])) + (8 << 30))
     ora = _oracle(O, ov, N, seed=seed, env_id0=id0)
     full = lmz.LmazeVecCuda(N, variant, seed=seed, env_id0=id0)
     comp = lmz.LmazeVecCuda(N, variant, seed=seed, env_id0=id0, obs_mode="compact")
@@ -230,7 +204,7 @@ def test_v4_masked_reset_mixes_history_lengths(lmz, oracle_mod):
     history entries (the warp-cooperative materialisation) inside tiles whose other lanes are still in history mode."""
     O = oracle_mod
     N, T, seed, id0 = _multi(), 80, 31, 0
-    _need(2 * N * 34300 + (8 << 30))
+    need_free(2 * N * 34300 + (8 << 30))
     ora = _oracle(O, O.V4, N, seed=seed, env_id0=id0, autoreset=False)
     full = lmz.LmazeVecCuda(N, "v4", seed=seed, env_id0=id0, autoreset=False)
     comp = lmz.LmazeVecCuda(N, "v4", seed=seed, env_id0=id0, autoreset=False, obs_mode="compact")
@@ -287,7 +261,7 @@ def test_v5_compact_and_full_multitile(lmz, oracle_mod):
     step, and three 1,024-env oracle blocks (the first, a middle one, the one ending at the last env) every step."""
     O = oracle_mod
     N, T, seed = _multi(), 130, 19
-    _need(N * (34300 + 19600) + (8 << 30))
+    need_free(N * (34300 + 19600) + (8 << 30))
     full = lmz.LmazeHierCuda(N, "v5", seed=seed, autoreset=True)
     comp = lmz.LmazeHierCuda(N, "v5", seed=seed, autoreset=True, obs_mode="compact")
     f0 = full.reset(); comp.reset()
@@ -380,7 +354,7 @@ def test_full_foveal_kernel_every_cta_size(lmz, variant):
     """lmz_env_fov_kernel at every tune[0] the library builds besides the default 128 threads, R + 21 envs, 60 steps,
     against the default handle (which the tests above check against the oracle)."""
     N = _multi(k=1)
-    _need(2 * N * (34300 + 19600) + (8 << 30))
+    need_free(2 * N * (34300 + 19600) + (8 << 30))
     for thr in (160, 192, 224, 256, 512, 1024):
         _lockstep(_mk(lmz, variant, N, (thr, 0, 0, 0)), variant, 60, thr)
 
@@ -390,7 +364,7 @@ def test_compact_foveal_kernel_every_cta_shape(lmz, variant):
     """lmz_fov_small_kernel with 2 and 8 warps per CTA, one and two CTAs per SM (tune[2] = 1 also makes every warp
     work through many more tiles)."""
     N = _multi(k=1)
-    _need(8 << 30)
+    need_free(8 << 30)
     for thr in (64, 256):
         for cap in (1, 2):
             _lockstep(_mk(lmz, variant, N, (thr, 0, cap, 0), obs_mode="compact"), variant, 60, thr + cap)
@@ -400,7 +374,7 @@ def test_compact_foveal_kernel_every_cta_shape(lmz, variant):
 def test_compact_and_incremental_cta_caps(lmz, variant):
     """tune[2] (CTAs per SM) on the compact / transition-only launch and on the incremental render."""
     N = _multi(k=1)
-    _need(2 * N * 112896 + (8 << 30))
+    need_free(2 * N * 112896 + (8 << 30))
     for kw in (dict(obs_mode="compact"), dict(with_obs=False), dict(render_mode="incremental")):
         for cap in (1, 2):
             _lockstep(_mk(lmz, variant, N, (0, 0, cap, 0), **kw), variant, 60, cap)
@@ -447,7 +421,7 @@ def test_rollout_kernel_several_envs_per_thread(lmz, oracle_mod, variant):
     N = _multi(k=3, tail=5)
     seed, id0 = (5 << 32) + 77, (1 << 32) - 100_003
     ov = O.V0 if variant == "v0" else O.V3
-    _need(4 << 30)
+    need_free(4 << 30)
     ora = _oracle(O, ov, N, seed=seed, env_id0=id0)
     env = lmz.LmazeVecCuda(N, variant, seed=seed, env_id0=id0, obs_mode="compact")
     env.reset()
@@ -468,7 +442,7 @@ def test_foveal_rollout_kernel_several_envs_per_thread(lmz, oracle_mod, variant)
     N = _multi()
     seed, id0 = (3 << 32) + 9, (1 << 32) - 300_001
     ov = O.V2 if variant == "v2" else O.V4
-    _need(4 << 30)
+    need_free(4 << 30)
     ora = _oracle(O, ov, N, seed=seed, env_id0=id0)
     env = lmz.LmazeVecCuda(N, variant, seed=seed, env_id0=id0, obs_mode="compact")
     env.reset()
@@ -488,7 +462,7 @@ def test_hier_rollout_several_envs_per_thread(lmz, oracle_mod):
     the same goals and actions; then a rollout with caller-supplied goals= / actions= buffers against the same."""
     O = oracle_mod
     N, seed = _multi(), 21
-    _need(8 << 30)
+    need_free(8 << 30)
     roll = lmz.LmazeHierCuda(N, "v5", seed=seed, obs_mode="compact")
     step = lmz.LmazeHierCuda(N, "v5", seed=seed, obs_mode="compact")
     roll.reset(); step.reset()
@@ -548,7 +522,7 @@ def test_bench_sizes(lmz, oracle_mod, variant, obs_mode, N, LO):
     T, B, seed = 120, 1024, 2026
     hier = variant == "v5"
     per_env = {"v2": 24500, "v4": 34300}.get(variant, 0) if obs_mode == "full" else 2048
-    _need(N * (per_env + 2048) + (8 << 30))
+    need_free(N * (per_env + 2048) + (8 << 30))
     if hier:
         env = lmz.LmazeHierCuda(N, "v5", seed=seed, obs_mode=obs_mode)
         ora = O.OracleHier(B, seed=seed, env_id0=LO)
@@ -583,7 +557,7 @@ def test_bench_sizes(lmz, oracle_mod, variant, obs_mode, N, LO):
         assert np.array_equal(u32(env.get_visit()[sl]), u32(ora.export_visit()))
     assert int(ora.episode.min()) >= (1 if hier else 2) and int(ora.episode.max()) >= 2
     # every row
-    allowed = torch.as_tensor(RC_BITS).cuda()
+    allowed = torch.as_tensor(REWARD_BITS.view(np.int32)).cuda()
     assert torch.isin(env.reward.view(torch.int32), allowed).all()
     if hier:
         assert torch.isin(env.local_reward.view(torch.int32), allowed).all()

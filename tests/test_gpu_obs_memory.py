@@ -10,20 +10,13 @@ import gc
 import pytest
 import torch
 
+from gpu_helpers import lmz
+
 pytestmark = pytest.mark.gpu
 
 STEPS = 130
 CHECKPOINTS = (1, 64, STEPS)
 CH = 1 << 14                            # rows per chunk of a digest
-
-
-@pytest.fixture(scope="module")
-def lmz():
-    import gym_lmaze_b200 as g
-    from gym_lmaze_b200 import _abi
-    _abi.load()
-    assert torch.cuda.is_available()
-    return g
 
 
 @pytest.fixture(scope="module")

@@ -9,36 +9,18 @@ import numpy as np
 import pytest
 import torch
 
+from golden_io import Traces, fov_image, pack_v2_spawn, reward_f32_bits, unpack
+from gpu_helpers import REWARD_BITS, REWARD_F32, lmz, need_free, u32
 from philox_np import _rng_actions
 
 pytestmark = pytest.mark.gpu
 
 INVALID = 7
 RC = {0x8000000000000000: 0, 0xBFF0000000000000: 1, 0xBF847AE147AE147B: 2, 0x4059000000000000: 3}
-RC_F32_BITS = np.array([0x80000000, 0xBF800000, 0xBC23D70A, 0x42C80000], dtype=np.uint32)
-RC_VALUE = [-0.0, -1.0, -0.01, 100.0]
 
 
 def rcode_of_f64_bits(bits):
     return RC[int(np.int64(bits).view(np.uint64))]
-
-
-def unpack(bits, shape):
-    n = int(np.prod(shape))
-    return np.unpackbits(bits)[:n].reshape(shape).astype(np.float32)
-
-
-@pytest.fixture(scope="module")
-def lmz():
-    import gym_lmaze_b200 as g
-    from gym_lmaze_b200 import _abi
-    _abi.load()                      # must be the in-tree CUDA library; raises if missing
-    assert torch.cuda.is_available()
-    return g
-
-
-def rbits(t):
-    return t.detach().cpu().numpy().view(np.uint32)
 
 
 # ---------------------------------------------------------------- golden fixtures (reference outputs)
@@ -57,15 +39,14 @@ def test_v0_golden_table(lmz, golden_dir, render_mode):
     obs, rew, done, info = env.step(torch.as_tensor(tab[:, 2]))
     out = env.get_state().cpu().numpy()
     assert np.array_equal(out[:, 0], tab[:, 5]) and np.array_equal(out[:, 1], tab[:, 6])
-    want_bits = np.array([np.float32(np.int64(b).view(np.float64)).view(np.uint32) for b in tab[:, 7]])
-    assert np.array_equal(rbits(rew), want_bits)           # incl. -0.0 and the stale 'S' reward
+    assert np.array_equal(u32(rew), reward_f32_bits(tab[:, 7]))           # incl. -0.0 and the stale 'S' reward
     assert np.array_equal(done.cpu().numpy().astype(np.int64), tab[:, 8])
     assert np.array_equal(out[:, 6] - 3, tab[:, 9])        # goalCount delta
     assert np.array_equal(out[:, 4], tab[:, 10])           # stepCount
     assert torch.equal(info["action"].cpu(), torch.as_tensor(tab[:, 2]))
     # obs of each row = the reference render of its new position
     pos_index = {tuple(p): i for i, p in enumerate(z["positions"])}
-    renders = torch.from_numpy(np.stack([unpack(b, (4, 84, 84)) for b in z["renders"]])).cuda()
+    renders = torch.from_numpy(unpack(z["renders"], (4, 84, 84))).cuda()
     idx = torch.as_tensor([pos_index[(int(a), int(b))] for a, b in zip(tab[:, 5], tab[:, 6])]).cuda()
     assert torch.equal(obs, renders[idx])
     env.close()
@@ -84,8 +65,7 @@ def test_v3_golden_table(lmz, golden_dir):
     out = env.get_state().cpu().numpy()
     assert np.array_equal(out[:, 0], tab[:, 6]) and np.array_equal(out[:, 1], tab[:, 7])
     assert np.array_equal(out[:, 2:4], tab[:, 2:4])
-    want_bits = np.array([np.float32(np.int64(b).view(np.float64)).view(np.uint32) for b in tab[:, 8]])
-    assert np.array_equal(rbits(rew), want_bits)
+    assert np.array_equal(u32(rew), reward_f32_bits(tab[:, 8]))
     assert np.array_equal(done.cpu().numpy().astype(np.int64), tab[:, 9])
     assert np.array_equal(out[:, 4], tab[:, 10])
     # renders: set each (ball, goal) key and render without stepping
@@ -95,7 +75,7 @@ def test_v3_golden_table(lmz, golden_dir):
     st2[:, 0:4] = keys
     env2.set_state(st2)
     got = env2.render_obs()
-    want = torch.from_numpy(np.stack([unpack(b, (3, 72, 72)) for b in z["renders"]])).cuda()
+    want = torch.from_numpy(unpack(z["renders"], (3, 72, 72))).cuda()
     assert torch.equal(got, want)
     env.close(); env2.close()
 
@@ -104,33 +84,26 @@ def test_v3_golden_table(lmz, golden_dir):
 @pytest.mark.parametrize("render_mode", ["tma", "st128"])
 def test_golden_traces(lmz, golden_dir, variant, render_mode):
     """Recorded reference episodes (scripted spawns, invalid actions, timeouts, goals)."""
-    z = np.load(os.path.join(golden_dir, variant + "_traces.npz"))
-    ne = int(z["n_envs"])
+    tr = Traces(golden_dir, variant)
     shape = (4, 84, 84) if variant == "v0" else (3, 72, 72)
-    env = lmz.LmazeVecCuda(ne, variant, autoreset=True, render_mode=render_mode)
-    sp0 = np.stack([z["e%d_spawn0" % e] for e in range(ne)])
+    env = lmz.LmazeVecCuda(tr.n_envs, variant, autoreset=True, render_mode=render_mode)
+    sp0 = tr.per_env("spawn0")
     if variant == "v0":
         sp0 = np.concatenate([sp0, -np.ones_like(sp0)], 1)
     env.reset(spawn=sp0)
-    T = len(z["e0_actions"])
-    n_done = 0
-    for t in range(T):
-        acts = np.array([z["e%d_actions" % e][t] for e in range(ne)])
-        spawn = np.stack([z["e%d_spawn" % e][t] for e in range(ne)])
+    acts, spawns, dref = tr.per_step("actions"), tr.per_step("spawn"), tr.per_step("done")
+    want_r, obs_bits = reward_f32_bits(tr.per_step("reward_bits")), tr.per_step("obs")
+    for t in range(tr.T):
+        spawn = spawns[t]
         if variant == "v0":
             spawn = np.concatenate([spawn, -np.ones_like(spawn)], 1)
-        dref = np.array([z["e%d_done" % e][t] for e in range(ne)])
-        spawn = np.where(dref[:, None] > 0, spawn, 1)
-        obs, rew, done, _ = env.step(torch.as_tensor(acts), spawn=spawn)
-        want_r = np.array([np.float32(np.int64(z["e%d_reward_bits" % e][t]).view(np.float64)).view(np.uint32)
-                           for e in range(ne)])
-        assert np.array_equal(rbits(rew), want_r), t
-        assert np.array_equal(done.cpu().numpy().astype(np.uint8), dref), t
-        want_o = np.stack([unpack(z["e%d_obs" % e][t], shape) for e in range(ne)])
-        assert np.array_equal(obs.cpu().numpy(), want_o), t
-        n_done += int(dref.sum())
+        spawn = np.where(dref[t][:, None] > 0, spawn, 1)
+        obs, rew, done, _ = env.step(torch.as_tensor(acts[t]), spawn=spawn)
+        assert np.array_equal(u32(rew), want_r[t]), t
+        assert np.array_equal(done.cpu().numpy().astype(np.uint8), dref[t]), t
+        assert np.array_equal(obs.cpu().numpy(), unpack(obs_bits[t], shape)), t
     s = env.stats()
-    assert s["episodes"] == n_done and s["steps"] == T * ne
+    assert s["episodes"] == int(dref.sum()) and s["steps"] == tr.T * tr.n_envs
     env.close()
 
 
@@ -141,8 +114,7 @@ def test_v0_real_mt_trace(lmz, golden_dir):
     for t in range(len(z["mt_actions"])):
         sp = z["mt_spawn"][t] if z["mt_done"][t] else (1, 1)
         obs, rew, done, _ = env.step(torch.as_tensor([z["mt_actions"][t]]), spawn=[[sp[0], sp[1]]])
-        want = np.float32(np.int64(z["mt_reward_bits"][t]).view(np.float64)).view(np.uint32)
-        assert rbits(rew)[0] == want and bool(done[0]) == bool(z["mt_done"][t]), t
+        assert u32(rew)[0] == reward_f32_bits(z["mt_reward_bits"][t]) and bool(done[0]) == bool(z["mt_done"][t]), t
         if not z["mt_done"][t]:
             assert tuple(env.get_state()[0, :2].tolist()) == tuple(z["mt_pos"][t])
     env.close()
@@ -196,7 +168,7 @@ def test_config2_4096_envs_per_step_parity(lmz, oracle_mod, variant, render_mode
         _, r_ref, d_ref = ora.step(a.numpy(), spawn=sp, obs_out=obs_buf)
         obs, rew, done, _ = env.step(a.to(torch.uint8) if t % 3 == 0 else (a.to(torch.int32) if t % 3 == 1 else a),
                                      spawn=sp)
-        assert np.array_equal(rbits(rew), r_ref.view(np.uint32)), t
+        assert np.array_equal(u32(rew), r_ref.view(np.uint32)), t
         assert np.array_equal(done.cpu().numpy().view(np.uint8), d_ref), t
         assert torch.equal(obs, pinned.cuda()), t
         if t % 16 == 0 or t == T - 1:
@@ -225,7 +197,7 @@ def test_device_rng_spawn_matches_spec(lmz, oracle_mod, variant):
         a = torch.randint(0, 4, (N,), generator=gen)
         _, r_ref, d_ref = ora.step(a.numpy(), want_obs=False)
         _, rew, done, _ = env.step(a, )
-        assert np.array_equal(rbits(rew), r_ref.view(np.uint32)) and np.array_equal(done.cpu().numpy().view(np.uint8), d_ref), t
+        assert np.array_equal(u32(rew), r_ref.view(np.uint32)) and np.array_equal(done.cpu().numpy().view(np.uint8), d_ref), t
     st = env.get_state().cpu().numpy()
     pos, sc, gc, _ = ora.export()
     assert np.array_equal(st[:, 0:2], pos[:, 0:2]) and np.array_equal(st[:, 4], sc)
@@ -250,7 +222,7 @@ def test_rollout_kernel_parity(lmz, oracle_mod, variant):
         acts = np.array([[oracle_mod.rng_action(seed, id0 + i, t_global + t) for i in range(N)] for t in range(Tk)])
         for t in range(Tk):
             _, r_ref, d_ref = ora.step(acts[t], want_obs=False)
-            assert np.array_equal(rbits(rew[t]), r_ref.view(np.uint32)), (Tk, t)
+            assert np.array_equal(u32(rew[t]), r_ref.view(np.uint32)), (Tk, t)
             assert np.array_equal(done[t].cpu().numpy().view(np.uint8), d_ref), (Tk, t)
         t_global += Tk
     # (b) caller-supplied action buffer [T, N]
@@ -259,7 +231,7 @@ def test_rollout_kernel_parity(lmz, oracle_mod, variant):
     rew, done = env.rollout(T, actions=a.to(torch.uint8))
     for t in range(T):
         _, r_ref, d_ref = ora.step(a[t].numpy(), want_obs=False)
-        assert np.array_equal(rbits(rew[t]), r_ref.view(np.uint32)) and \
+        assert np.array_equal(u32(rew[t]), r_ref.view(np.uint32)) and \
             np.array_equal(done[t].cpu().numpy().view(np.uint8), d_ref), t
     st = env.get_state().cpu().numpy()
     pos, sc, gc, _ = ora.export()
@@ -300,11 +272,11 @@ def test_no_autoreset_matches_reference_semantics(lmz, oracle_mod):
         a = torch.randint(0, 4, (N,), generator=gen)
         o_ref, r_ref, d_ref = ora.step(a.numpy())
         obs, rew, done, _ = env.step(a)
-        assert np.array_equal(rbits(rew), r_ref.view(np.uint32)) and np.array_equal(done.cpu().numpy().view(np.uint8), d_ref)
+        assert np.array_equal(u32(rew), r_ref.view(np.uint32)) and np.array_equal(done.cpu().numpy().view(np.uint8), d_ref)
         assert torch.equal(obs.cpu(), torch.from_numpy(o_ref))
         if t == 100:
             seen_101 = True
-            goal = rbits(rew) == 0x42C80000
+            goal = u32(rew) == 0x42C80000
             assert not done.cpu().numpy()[~goal].any()
     assert seen_101
     # masked reset only touches the selected envs (state and obs)
@@ -376,20 +348,14 @@ def test_v3_string_actions(lmz, oracle_mod):
     env.reset(spawn=sp); ora.reset(spawn=sp)
     obs, rew, done, _ = env.step(["left", "1", "up", "noop"])
     o_ref, r_ref, d_ref = ora.step(np.array([0, 1, 2, INVALID]))
-    assert np.array_equal(rbits(rew), r_ref.view(np.uint32)) and torch.equal(obs.cpu(), torch.from_numpy(o_ref))
+    assert np.array_equal(u32(rew), r_ref.view(np.uint32)) and torch.equal(obs.cpu(), torch.from_numpy(o_ref))
     env.close()
 
 
 # ---------------------------------------------------------------- BASELINE config 3 scale: 2^20 envs, size-independent properties
 def test_one_million_envs_properties(lmz, oracle_mod):
     N = 1 << 20
-    import gc
-    gc.collect()
-    torch.cuda.empty_cache()             # earlier tests' tensors sit in torch's caching allocator
-    free_b = torch.cuda.mem_get_info()[0]
-    need = N * 112896 + (4 << 30)
-    if free_b < need:
-        pytest.fail("B200 expected: %d GiB free, need %d GiB" % (free_b >> 30, need >> 30))
+    need_free(N * 112896 + (4 << 30))
     env = lmz.LmazeVecCuda(N, "v0", seed=2026)
     obs = env.reset()
     gen = torch.Generator(device="cuda").manual_seed(1)
@@ -400,7 +366,7 @@ def test_one_million_envs_properties(lmz, oracle_mod):
     after = env.get_state()
     # every reward is one of the reference's four bit patterns
     rb = rew.view(torch.int32)
-    allowed = torch.as_tensor(RC_F32_BITS.view(np.int32)).cuda()
+    allowed = torch.as_tensor(REWARD_BITS.view(np.int32)).cuda()
     assert torch.isin(rb, allowed).all()
     # per-env channel sums [49, 3528, 49, 3430] and ball block where the state says (chunked: obs is 118 GB)
     want = torch.tensor([49.0, 3528.0, 49.0, 3430.0], device="cuda")
@@ -417,9 +383,9 @@ def test_one_million_envs_properties(lmz, oracle_mod):
     b = before[idx.cuda()].cpu().numpy()
     ora = oracle_mod.OracleVec(oracle_mod.V0, len(idx), autoreset=False)
     for i, row in enumerate(b):
-        ora.force(i, int(row[0]), int(row[1]), step_count=int(row[4]), reward=RC_VALUE[row[5]], goal_count=int(row[6]))
+        ora.force(i, int(row[0]), int(row[1]), step_count=int(row[4]), reward=float(REWARD_F32[row[5]]), goal_count=int(row[6]))
     _, r_ref, d_ref = ora.step(a[idx.cuda()].cpu().numpy().astype(np.int64), want_obs=False)
-    assert np.array_equal(rbits(rew[idx.cuda()]), r_ref.view(np.uint32))
+    assert np.array_equal(u32(rew[idx.cuda()]), r_ref.view(np.uint32))
     assert np.array_equal(done[idx.cuda()].cpu().numpy().view(np.uint8), d_ref)
     nd = d_ref == 0                                 # envs that did not reset: position must match, obs must match
     pos = ora.export()[0]
@@ -447,7 +413,7 @@ def test_compact_obs_reconstructs_reference_image(lmz, oracle_mod, variant):
         a = torch.randint(0, 5, (N,), generator=gen)
         o_ref, r_ref, d_ref = ora.step(a.numpy())
         obs, rew, done, _ = env.step(a)
-        assert np.array_equal(rbits(rew), r_ref.view(np.uint32)) and np.array_equal(done.cpu().numpy().view(np.uint8), d_ref)
+        assert np.array_equal(u32(rew), r_ref.view(np.uint32)) and np.array_equal(done.cpu().numpy().view(np.uint8), d_ref)
         assert torch.equal(env.expand(obs).cpu(), torch.from_numpy(o_ref)), t
     s = env.stats()
     assert [s[k] for k in oracle_mod.STAT_NAMES] == ora.stats.tolist()
@@ -476,7 +442,7 @@ def test_render_window(lmz, oracle_mod, render_mode, obs_mode):
         env.set_window(lo)
         env.obs.fill_(7)                                   # sentinel: rows must be fully rewritten
         obs, rew, done, _ = env.step(a)
-        assert np.array_equal(rbits(rew), r_ref.view(np.uint32))          # all N envs stepped
+        assert np.array_equal(u32(rew), r_ref.view(np.uint32))          # all N envs stepped
         assert torch.equal(env.expand(obs).cpu(), torch.from_numpy(o_ref[lo:lo + W])), t
         # walk the rest of the batch window by window without stepping
         for lo2 in (0, N - W, 350):
@@ -498,7 +464,7 @@ def test_transition_only_mode(lmz, oracle_mod):
         a = torch.randint(0, 4, (N,), generator=gen)
         _, r_ref, d_ref = ora.step(a.numpy(), want_obs=False)
         obs, rew, done, _ = env.step(a)
-        assert obs is None and np.array_equal(rbits(rew), r_ref.view(np.uint32)) and \
+        assert obs is None and np.array_equal(u32(rew), r_ref.view(np.uint32)) and \
             np.array_equal(done.cpu().numpy().view(np.uint8), d_ref)
     assert [env.stats()[k] for k in oracle_mod.STAT_NAMES] == ora.stats.tolist()
     env.close()
@@ -521,11 +487,10 @@ def test_v2_golden_table(lmz, golden_dir):
     obs, rew, done, info = env.step(torch.as_tensor(tab[:, 7]))
     out = env.get_state().cpu().numpy()
     assert np.array_equal(out[:, 0], tab[:, 9]) and np.array_equal(out[:, 1], tab[:, 10])
-    want_bits = np.array([np.float32(np.int64(b).view(np.float64)).view(np.uint32) for b in tab[:, 11]])
-    assert np.array_equal(rbits(rew), want_bits)
+    assert np.array_equal(u32(rew), reward_f32_bits(tab[:, 11]))
     assert np.array_equal(done.cpu().numpy().astype(np.int64), tab[:, 12])
     assert np.array_equal(out[:, 4], tab[:, 13])
-    want = torch.from_numpy(np.stack([unpack(b, (5, 35, 35)) for b in z["obs"]]))
+    want = torch.from_numpy(unpack(z["obs"], (5, 35, 35)))
     # the device state has no room for an UNREACHABLE history (previous crop taken somewhere other than
     # the ball's cell), which half of the fixture rows use on purpose: compare their channels 0-2 only
     reachable = torch.from_numpy((tab[:, 1] == tab[:, 5]) & (tab[:, 2] == tab[:, 6]))
@@ -541,29 +506,21 @@ def test_v2_golden_table(lmz, golden_dir):
 
 
 def test_v2_golden_traces(lmz, golden_dir):
-    z = np.load(os.path.join(golden_dir, "v2_traces.npz"))
-    ne = int(z["n_envs"])
-    env = lmz.LmazeVecCuda(ne, "v2", autoreset=True)
-    init = np.stack([z["e%d_init" % e] for e in range(ne)])        # bx, by, gx, gy, layout, layout-before
+    tr = Traces(golden_dir, "v2")
+    env = lmz.LmazeVecCuda(tr.n_envs, "v2", autoreset=True)
+    init = tr.per_env("init")                                      # bx, by, gx, gy, layout, layout-before
     st = np.array([_v2_state_rows(r[5], 4, 4, 8, 8, 4, 4, 0) for r in init], np.int32)
     env.set_state(st)                                              # the maze the constructor rolled
     obs = env.reset(spawn=init[:, :5])
-    want = np.stack([unpack(z["e%d_first_obs" % e], (5, 35, 35)) for e in range(ne)])
-    assert np.array_equal(obs.cpu().numpy(), want)
-    T = len(z["e0_actions"])
-    for t in range(T):
-        acts = np.array([z["e%d_actions" % e][t] for e in range(ne)])
-        s5 = np.stack([z["e%d_spawn" % e][t] for e in range(ne)])
-        dref = np.array([z["e%d_done" % e][t] for e in range(ne)])
-        s5 = np.where(dref[:, None] > 0, s5, 0)
-        obs, rew, done, _ = env.step(torch.as_tensor(acts), spawn=s5)
-        want_r = np.array([np.float32(np.int64(z["e%d_reward_bits" % e][t]).view(np.float64)).view(np.uint32)
-                           for e in range(ne)])
-        assert np.array_equal(rbits(rew), want_r), t
-        assert np.array_equal(done.cpu().numpy().astype(np.uint8), dref), t
-        want_o = np.stack([unpack(z["e%d_obs" % e][t], (5, 35, 35)) for e in range(ne)])
-        assert np.array_equal(obs.cpu().numpy(), want_o), t
-    assert env.stats()["episodes"] == sum(int(z["e%d_done" % e].sum()) for e in range(ne))
+    assert np.array_equal(obs.cpu().numpy(), unpack(tr.per_env("first_obs"), (5, 35, 35)))
+    acts, s5, dref = tr.per_step("actions"), tr.per_step("spawn"), tr.per_step("done")
+    want_r, obs_bits = reward_f32_bits(tr.per_step("reward_bits")), tr.per_step("obs")
+    for t in range(tr.T):
+        obs, rew, done, _ = env.step(torch.as_tensor(acts[t]), spawn=np.where(dref[t][:, None] > 0, s5[t], 0))
+        assert np.array_equal(u32(rew), want_r[t]), t
+        assert np.array_equal(done.cpu().numpy().astype(np.uint8), dref[t]), t
+        assert np.array_equal(obs.cpu().numpy(), unpack(obs_bits[t], (5, 35, 35))), t
+    assert env.stats()["episodes"] == int(dref.sum())
     env.close()
 
 
@@ -593,11 +550,9 @@ def test_v2_4096_envs_vs_oracle(lmz, oracle_mod, inject):
             out[i] = (b[0], b[1], g[0], g[1], rng.randint(1, 6))
         return out
 
-    def packed(s5):
-        return np.stack([s5[:, 0], s5[:, 1], s5[:, 2], s5[:, 3] | (s5[:, 4] << 5)], 1)
     if inject:
         s5 = draw_spawn(np.ones(N, int))
-        o_ref = ora.reset(spawn=packed(s5)); o_gpu = env.reset(spawn=s5)
+        o_ref = ora.reset(spawn=pack_v2_spawn(s5)); o_gpu = env.reset(spawn=s5)
     else:
         o_ref = ora.reset(); o_gpu = env.reset()
     assert torch.equal(o_gpu.cpu(), torch.from_numpy(o_ref))
@@ -607,12 +562,12 @@ def test_v2_4096_envs_vs_oracle(lmz, oracle_mod, inject):
         a = torch.randint(0, 25, (N,), generator=gen)
         if inject:
             s5 = draw_spawn(ora.export_aux()[:, 0])
-            _, r_ref, d_ref = ora.step(a.numpy(), spawn=packed(s5), obs_out=obs_buf)
+            _, r_ref, d_ref = ora.step(a.numpy(), spawn=pack_v2_spawn(s5), obs_out=obs_buf)
             obs, rew, done, _ = env.step(a, spawn=s5)
         else:
             _, r_ref, d_ref = ora.step(a.numpy(), obs_out=obs_buf)
             obs, rew, done, _ = env.step(a)
-        assert np.array_equal(rbits(rew), r_ref.view(np.uint32)), t
+        assert np.array_equal(u32(rew), r_ref.view(np.uint32)), t
         assert np.array_equal(done.cpu().numpy().view(np.uint8), d_ref), t
         assert torch.equal(obs.cpu(), torch.from_numpy(obs_buf)), t
     st = env.get_state().cpu().numpy()
@@ -642,7 +597,7 @@ def test_v2_windows_and_masks(lmz, oracle_mod):
         env.set_window(lo)
         env.obs.fill_(5)
         obs, rew, done, _ = env.step(a)
-        assert np.array_equal(rbits(rew), r_ref.view(np.uint32))
+        assert np.array_equal(u32(rew), r_ref.view(np.uint32))
         assert torch.equal(obs.cpu(), torch.from_numpy(o_ref[lo:lo + W])), t
         assert torch.equal(env.render_window(N - W).cpu(), torch.from_numpy(o_ref[N - W:]))
     rew, done = env.rollout(4)                      # (round 2: the foveal variants have a rollout kernel too)
@@ -658,12 +613,6 @@ def test_v2_windows_and_masks(lmz, oracle_mod):
 
 
 # ---------------------------------------------------------------- lmaze-v4 (v2 + float visit layer)
-def _v4_obs(bits, visit):
-    b = np.unpackbits(bits)[:125].reshape(5, 5, 5).astype(np.float32)
-    small = np.stack([b[0], b[1], visit[0], b[2], b[3], b[4], visit[1]])
-    return np.repeat(np.repeat(small, 7, 1), 7, 2)
-
-
 def test_v4_golden_table(lmz, golden_dir):
     """Reference outputs incl. the float visit layer, compared as f32 BIT patterns."""
     z = np.load(os.path.join(golden_dir, "v4_table.npz"))
@@ -677,39 +626,28 @@ def test_v4_golden_table(lmz, golden_dir):
     obs, rew, done, _ = env.step(torch.as_tensor(tab[:, 5]))
     out = env.get_state().cpu().numpy()
     assert np.array_equal(out[:, 0], tab[:, 7]) and np.array_equal(out[:, 1], tab[:, 8])
-    want_bits = np.array([np.float32(np.int64(b).view(np.float64)).view(np.uint32) for b in tab[:, 9]])
-    assert np.array_equal(rbits(rew), want_bits)
+    assert np.array_equal(u32(rew), reward_f32_bits(tab[:, 9]))
     assert np.array_equal(done.cpu().numpy().astype(np.int64), tab[:, 10]) and np.array_equal(out[:, 4], tab[:, 11])
     assert np.array_equal(env.get_visit().cpu().numpy().view(np.uint32), z["post_visit"].view(np.uint32))
-    want = np.stack([_v4_obs(z["obs_bits"][k], z["obs_visit"][k]) for k in range(n)])
+    want = fov_image(z["obs_bits"], z["obs_visit"])
     assert np.array_equal(obs.cpu().numpy().view(np.uint32), want.view(np.uint32))
     env.close()
 
 
 def test_v4_golden_traces(lmz, golden_dir):
-    z = np.load(os.path.join(golden_dir, "v4_traces.npz"))
-    ne = int(z["n_envs"])
-    env = lmz.LmazeVecCuda(ne, "v4", autoreset=True)
-    init = np.stack([z["e%d_init" % e] for e in range(ne)])        # bx, by, gx, gy, layout
-    obs = env.reset(spawn=init)
-    want = np.stack([_v4_obs(z["e%d_first_bits" % e], z["e%d_first_visit" % e]) for e in range(ne)])
-    assert np.array_equal(obs.cpu().numpy(), want)
-    T = len(z["e0_actions"])
-    for t in range(T):
-        acts = np.array([z["e%d_actions" % e][t] for e in range(ne)])
-        s5 = np.stack([z["e%d_spawn" % e][t] for e in range(ne)])
-        dref = np.array([z["e%d_done" % e][t] for e in range(ne)])
-        s5 = np.where(dref[:, None] > 0, s5, 0)
-        obs, rew, done, _ = env.step(torch.as_tensor(acts), spawn=s5)
-        want_r = np.array([np.float32(np.int64(z["e%d_reward_bits" % e][t]).view(np.float64)).view(np.uint32)
-                           for e in range(ne)])
-        assert np.array_equal(rbits(rew), want_r), t
-        assert np.array_equal(done.cpu().numpy().astype(np.uint8), dref), t
-        want_o = np.stack([_v4_obs(z["e%d_obs_bits" % e][t], z["e%d_obs_visit" % e][t]) for e in range(ne)])
-        assert np.array_equal(obs.cpu().numpy().view(np.uint32), want_o.view(np.uint32)), t
-    vis = env.get_visit().cpu().numpy()
-    for e in range(ne):
-        assert np.array_equal(vis[e].view(np.uint32), z["e%d_final_visit" % e].view(np.uint32))
+    tr = Traces(golden_dir, "v4")
+    env = lmz.LmazeVecCuda(tr.n_envs, "v4", autoreset=True)
+    obs = env.reset(spawn=tr.per_env("init"))                      # bx, by, gx, gy, layout
+    assert np.array_equal(obs.cpu().numpy(), fov_image(tr.per_env("first_bits"), tr.per_env("first_visit")))
+    acts, s5, dref = tr.per_step("actions"), tr.per_step("spawn"), tr.per_step("done")
+    want_r = reward_f32_bits(tr.per_step("reward_bits"))
+    obs_bits, obs_visit = tr.per_step("obs_bits"), tr.per_step("obs_visit")
+    for t in range(tr.T):
+        obs, rew, done, _ = env.step(torch.as_tensor(acts[t]), spawn=np.where(dref[t][:, None] > 0, s5[t], 0))
+        assert np.array_equal(u32(rew), want_r[t]), t
+        assert np.array_equal(done.cpu().numpy().astype(np.uint8), dref[t]), t
+        assert np.array_equal(u32(obs), u32(fov_image(obs_bits[t], obs_visit[t]))), t
+    assert np.array_equal(u32(env.get_visit()), u32(tr.per_env("final_visit")))
     env.close()
 
 
@@ -725,7 +663,7 @@ def test_v4_4096_envs_vs_oracle(lmz, oracle_mod):
         a = torch.randint(0, 25, (N,), generator=gen)
         _, r_ref, d_ref = ora.step(a.numpy(), obs_out=obs_buf)
         obs, rew, done, _ = env.step(a)
-        assert np.array_equal(rbits(rew), r_ref.view(np.uint32)), t
+        assert np.array_equal(u32(rew), r_ref.view(np.uint32)), t
         assert np.array_equal(done.cpu().numpy().view(np.uint8), d_ref), t
         assert torch.equal(obs.cpu().view(torch.int32), torch.from_numpy(obs_buf).view(torch.int32)), t
         if t % 25 == 0:
@@ -759,7 +697,7 @@ def test_cuda_graph_replay(lmz, oracle_mod, variant, render_mode):
         abuf.copy_(a.to(torch.uint8))
         replay()
         o_ref, r_ref, d_ref = ora.step(a.numpy(), want_obs=(t % 30 == 0))
-        assert np.array_equal(rbits(env.reward), r_ref.view(np.uint32)), t
+        assert np.array_equal(u32(env.reward), r_ref.view(np.uint32)), t
         assert np.array_equal(env.done.cpu().numpy().view(np.uint8), d_ref), t
         if t % 30 == 0:
             assert torch.equal(env.obs.cpu(), torch.from_numpy(o_ref)), t
@@ -783,7 +721,7 @@ def test_fixed_ball_and_goal_switches(lmz, oracle_mod, variant, random_ball, ran
         a = torch.randint(0, 4, (N,), generator=gen)
         o_ref, r_ref, d_ref = ora.step(a.numpy(), want_obs=(t % 20 == 0))
         obs, rew, done, _ = env.step(a)
-        assert np.array_equal(rbits(rew), r_ref.view(np.uint32)) and np.array_equal(done.cpu().numpy().view(np.uint8), d_ref), t
+        assert np.array_equal(u32(rew), r_ref.view(np.uint32)) and np.array_equal(done.cpu().numpy().view(np.uint8), d_ref), t
         if t % 20 == 0:
             assert torch.equal(obs.cpu(), torch.from_numpy(o_ref)), t
     st = env.get_state().cpu().numpy()
@@ -825,7 +763,7 @@ def test_incremental_render_stays_bit_identical(lmz, oracle_mod, variant):
         want_obs = t % 7 == 0 or t > T - 4
         _, r_ref, d_ref = ora.step(a.numpy(), obs_out=obs_buf if want_obs else None, want_obs=want_obs)
         obs, rew, done, _ = env.step(a)
-        assert np.array_equal(rbits(rew), r_ref.view(np.uint32)) and np.array_equal(done.cpu().numpy().view(np.uint8), d_ref), t
+        assert np.array_equal(u32(rew), r_ref.view(np.uint32)) and np.array_equal(done.cpu().numpy().view(np.uint8), d_ref), t
         if want_obs:
             assert torch.equal(obs.cpu(), torch.from_numpy(obs_buf)), t
         if t == 100:                              # move envs behind the tensor's back: must resync with a full render
@@ -833,7 +771,7 @@ def test_incremental_render_stays_bit_identical(lmz, oracle_mod, variant):
             env.set_state(st.roll(1, 0))
             for i, row in enumerate(st.roll(1, 0).cpu().numpy()):
                 ora.force(i, int(row[0]), int(row[1]), int(row[2]), int(row[3]), step_count=int(row[4]),
-                          reward=RC_VALUE[row[5]], goal_count=int(row[6]))
+                          reward=float(REWARD_F32[row[5]]), goal_count=int(row[6]))
             ora.episode[:] = st.roll(1, 0).cpu().numpy()[:, 7]
         if t == 150:                              # masked reset in the middle (full render of the masked rows only)
             mask = torch.rand(N, generator=gen) < 0.3

@@ -7,31 +7,11 @@ import numpy as np
 import pytest
 import torch
 
+from golden_io import unpack
+from gpu_helpers import REWARD_BITS, lmz, u32
+from philox_np import _rng_actions
+
 pytestmark = pytest.mark.gpu
-
-RC_VALUE = [-0.0, -1.0, -0.01, 100.0]
-
-
-@pytest.fixture(scope="module")
-def lmz():
-    import gym_lmaze_b200 as g
-    from gym_lmaze_b200 import _abi
-    _abi.load()                      # must be the in-tree CUDA library; raises if missing
-    assert torch.cuda.is_available()
-    return g
-
-
-def rbits(t):
-    return t.detach().cpu().numpy().view(np.uint32)
-
-
-def unpack(bits, shape):
-    n = int(np.prod(shape))
-    return np.unpackbits(bits)[:n].reshape(shape).astype(np.float32)
-
-
-def _rng_actions(O, seed, n, t):
-    return np.array([O.rng_action(seed, i, t) for i in range(n)], dtype=np.int64)
 
 
 # ---------------------------------------------------------------- ADVICE r1 (high): incremental render + rollout
@@ -52,12 +32,12 @@ def test_incremental_render_resyncs_after_rollout(lmz, oracle_mod, variant):
             a = torch.randint(0, 5, (N,), generator=gen)
             o_ref, r_ref, d_ref = ora.step(a.numpy())
             obs, rew, done, _ = env.step(a)
-            assert np.array_equal(rbits(rew), r_ref.view(np.uint32))
+            assert np.array_equal(u32(rew), r_ref.view(np.uint32))
             assert torch.equal(obs.cpu(), torch.from_numpy(o_ref)), it
         rew, done = env.rollout(T)                             # no obs written
         for t in range(T):
-            _, r_ref, d_ref = ora.step(_rng_actions(oracle_mod, seed, N, t_roll + t), want_obs=False)
-            assert np.array_equal(rbits(rew[t]), r_ref.view(np.uint32)), (it, t)
+            _, r_ref, d_ref = ora.step(_rng_actions(seed, np.arange(N), t_roll + t), want_obs=False)
+            assert np.array_equal(u32(rew[t]), r_ref.view(np.uint32)), (it, t)
         t_roll += T
     a = torch.randint(0, 4, (N,), generator=gen)
     o_ref, _, _ = ora.step(a.numpy())
@@ -184,7 +164,7 @@ def test_bits_obs_reconstructs_reference_image(lmz, oracle_mod, variant):
         want = t % 5 == 0 or t > T - 3
         o_ref, r_ref, d_ref = ora.step(a.numpy(), want_obs=want)
         obs, rew, done, _ = env.step(a)
-        assert np.array_equal(rbits(rew), r_ref.view(np.uint32)) and np.array_equal(done.cpu().numpy().view(np.uint8), d_ref), t
+        assert np.array_equal(u32(rew), r_ref.view(np.uint32)) and np.array_equal(done.cpu().numpy().view(np.uint8), d_ref), t
         if want:
             assert torch.equal(env.expand(obs).cpu(), torch.from_numpy(o_ref)), t
         if variant == "v3":
@@ -224,7 +204,7 @@ def test_rollout_reward_codes(lmz, variant):
     b = lmz.LmazeVecCuda(N, variant, seed=5, with_obs=False)
     a.reset(); b.reset()
     table = a.reward_table("cuda")
-    assert rbits(table).tolist() == [0x80000000, 0xBF800000, 0xBC23D70A, 0x42C80000]
+    assert u32(table).tolist() == REWARD_BITS.tolist()
     for it in range(2):
         rew, done_a = a.rollout(T)
         codes, done_b = b.rollout(T, reward_codes=True)
@@ -285,10 +265,6 @@ def test_host_pipeline_matches_oracle(lmz, oracle_mod, variant, obs_mode):
 
 
 # ---------------------------------------------------------------- the visit layer kept as its HISTORY (v4 / v5), edge cases
-def u32(t):
-    return (t.detach().cpu().numpy() if torch.is_tensor(t) else t).view(np.uint32)
-
-
 @pytest.mark.parametrize("obs_mode", ["full", "compact"])
 def test_v4_visit_layer_long_episode_without_reset(lmz, oracle_mod, obs_mode):
     """autoreset off and no reset for 330 steps: the layer is averaged 330 times in a row, far past the 64 entries
@@ -307,7 +283,7 @@ def test_v4_visit_layer_long_episode_without_reset(lmz, oracle_mod, obs_mode):
         a[N // 2:] = 12
         o_ref, r_ref, d_ref = ora.step(a.numpy())
         obs, rew, done, _ = env.step(a)
-        assert np.array_equal(rbits(rew), r_ref.view(np.uint32)) and np.array_equal(done.cpu().numpy().view(np.uint8), d_ref), t
+        assert np.array_equal(u32(rew), r_ref.view(np.uint32)) and np.array_equal(done.cpu().numpy().view(np.uint8), d_ref), t
         assert np.array_equal(u32(env.expand(obs)), u32(o_ref)), t
         if t % 20 == 19 or t in (61, 62, 63, 64, 65, 66, 148, 149, 150, 151):
             vref = ora.export_visit()
@@ -408,7 +384,7 @@ def test_foveal_rollout_kernel_parity(lmz, oracle_mod, variant):
         t_glob += T
         for t in range(T):
             _, r_ref, d_ref = ora.step(acts[t], want_obs=False)
-            assert np.array_equal(rbits(rew[t]), r_ref.view(np.uint32)), (rnd, t)
+            assert np.array_equal(u32(rew[t]), r_ref.view(np.uint32)), (rnd, t)
             assert np.array_equal(done[t].cpu().numpy().view(np.uint8), d_ref), (rnd, t)
         st = env.get_state().cpu().numpy()
         pos, sc, _, _ = ora.export()
@@ -424,7 +400,7 @@ def test_foveal_rollout_kernel_parity(lmz, oracle_mod, variant):
         t_glob += T_short
         for t in range(T_short):
             _, r_ref, d_ref = ora.step(acts[t], want_obs=False)
-            assert np.array_equal(rbits(rew[t]), r_ref.view(np.uint32)) and np.array_equal(done[t].cpu().numpy().view(np.uint8), d_ref)
+            assert np.array_equal(u32(rew[t]), r_ref.view(np.uint32)) and np.array_equal(done[t].cpu().numpy().view(np.uint8), d_ref)
     if variant == "v4":
         assert np.array_equal(u32(env.get_visit()), u32(ora.export_visit()))
     s = env.stats(check_errors=False)
@@ -433,7 +409,7 @@ def test_foveal_rollout_kernel_parity(lmz, oracle_mod, variant):
     a = np.random.RandomState(9).randint(0, 25, size=N)
     o_ref, r_ref, _ = ora.step(a)
     obs, rew, _, _ = env.step(a)
-    assert np.array_equal(u32(obs), u32(o_ref)) and np.array_equal(rbits(rew), r_ref.view(np.uint32))
+    assert np.array_equal(u32(obs), u32(o_ref)) and np.array_equal(u32(rew), r_ref.view(np.uint32))
     env.close()
 
 
@@ -462,7 +438,7 @@ def test_hier_rollout_kernel_parity(lmz, oracle_mod, philox):
             if need.any():
                 ora.planner_step(goals[t], mask=need)
             _, _, gr_ref, lr_ref, gd_ref, ld_ref, _ = ora.step(acts[t])
-            assert np.array_equal(rbits(gr[t]), gr_ref.view(np.uint32)) and np.array_equal(rbits(lr[t]), lr_ref.view(np.uint32)), (rnd, t)
+            assert np.array_equal(u32(gr[t]), gr_ref.view(np.uint32)) and np.array_equal(u32(lr[t]), lr_ref.view(np.uint32)), (rnd, t)
             assert np.array_equal(gd[t].cpu().numpy(), gd_ref.astype(bool)) and np.array_equal(ld[t].cpu().numpy(), ld_ref.astype(bool)), (rnd, t)
             if gd_ref.any():
                 ora.reset(mask=gd_ref, want_obs=False)
@@ -484,7 +460,7 @@ def test_hier_rollout_kernel_parity(lmz, oracle_mod, philox):
                 if need.any():
                     ora.planner_step(ga[t, :, 0], mask=need)
                 _, _, gr_ref, lr_ref, gd_ref, ld_ref, _ = ora.step(ga[t, :, 1])
-                assert np.array_equal(rbits(gr6[t]), gr_ref.view(np.uint32)) and np.array_equal(ld6[t].cpu().numpy(), ld_ref.astype(bool)), t
+                assert np.array_equal(u32(gr6[t]), gr_ref.view(np.uint32)) and np.array_equal(ld6[t].cpu().numpy(), ld_ref.astype(bool)), t
                 if gd_ref.any():
                     ora.reset(mask=gd_ref, want_obs=False)
             assert np.array_equal(u32(env.get_visit()), u32(ora.export_visit()))

@@ -7,37 +7,15 @@ import numpy as np
 import pytest
 import torch
 
+from gpu_helpers import REWARD_BITS, lmz, need_free, u32
+
 pytestmark = pytest.mark.gpu
-
-RC_BITS = np.array([0x80000000, 0xBF800000, 0xBC23D70A, 0x42C80000], dtype=np.uint32).view(np.int32)
-
-
-@pytest.fixture(scope="module")
-def lmz():
-    import gym_lmaze_b200 as g
-    from gym_lmaze_b200 import _abi
-    _abi.load()
-    assert torch.cuda.is_available()
-    return g
-
-
-def u32(t):
-    return (t.detach().cpu().numpy() if torch.is_tensor(t) else t).view(np.uint32)
-
-
-def _need(nbytes):
-    import gc
-    gc.collect()
-    torch.cuda.empty_cache()             # earlier tests' tensors sit in torch's caching allocator
-    free_b = torch.cuda.mem_get_info()[0]
-    if free_b < nbytes:
-        pytest.fail("B200 expected: %d GiB free, need %d GiB" % (free_b >> 30, nbytes >> 30))
 
 
 def test_one_million_envs_st128_render(lmz, oracle_mod):
     """configs[2] size on the 128-bit vector-store render path (LMZ_RENDER_ST128): 2^20 envs x 112,896 B."""
     N, B, LO, seed = 1 << 20, 1024, 555_555, 77
-    _need(N * 112896 + (4 << 30))
+    need_free(N * 112896 + (4 << 30))
     env = lmz.LmazeVecCuda(N, "v0", seed=seed, render_mode="st128")
     ora = oracle_mod.OracleVec(oracle_mod.V0, B, seed=seed, env_id0=LO)
     obs = env.reset()
@@ -51,7 +29,7 @@ def test_one_million_envs_st128_render(lmz, oracle_mod):
         assert np.array_equal(done[LO:LO + B].cpu().numpy().view(np.uint8), d_ref), t
         assert np.array_equal(u32(obs[LO:LO + B]), u32(o_ref)), t
     st = env.get_state()
-    assert torch.isin(rew.view(torch.int32), torch.as_tensor(RC_BITS).cuda()).all()
+    assert torch.isin(rew.view(torch.int32), torch.as_tensor(REWARD_BITS.view(np.int32)).cuda()).all()
     want = torch.tensor([49.0, 3528.0, 49.0, 3430.0], device="cuda")          # per-env channel sums (SURVEY 8a, a10)
     CH = 1 << 14
     for lo in range(0, N, CH):
@@ -70,7 +48,7 @@ def test_v3_eight_million_envs_through_a_window(lmz, oracle_mod):
     """BASELINE configs[3] on ONE GPU: 8 M lmaze-v3 envs (498 GB of observations) consumed through a 1 M-env render
     window -- a step advances every env and renders window 0, lmz_render re-renders the other seven."""
     N, W, B, LO, seed = 1 << 23, 1 << 20, 1024, 5 * (1 << 20) + 333_333, 5
-    _need(W * 62208 + (4 << 30))
+    need_free(W * 62208 + (4 << 30))
     env = lmz.LmazeVecCuda(N, "v3", seed=seed, obs_window=W)
     ora = oracle_mod.OracleVec(oracle_mod.V3, B, seed=seed, env_id0=LO)
     env.reset()
@@ -84,7 +62,7 @@ def test_v3_eight_million_envs_through_a_window(lmz, oracle_mod):
         assert np.array_equal(u32(rew[LO:LO + B]), r_ref.view(np.uint32)), t
         assert np.array_equal(done[LO:LO + B].cpu().numpy().view(np.uint8), d_ref), t
     st = env.get_state()
-    assert torch.isin(rew.view(torch.int32), torch.as_tensor(RC_BITS[[1, 2, 3]]).cuda()).all()    # v3 never returns -0.0
+    assert torch.isin(rew.view(torch.int32), torch.as_tensor(REWARD_BITS[[1, 2, 3]].view(np.int32)).cuda()).all()    # v3 never returns -0.0
     free = 73 * 16.0                                        # 73 free cells x 4 x 4 (lmaze_env_v3.py:166)
     want = torch.tensor([free, 16.0, 16.0], device="cuda")
     total_ball = 0.0
@@ -112,7 +90,7 @@ def test_v5_one_million_envs_auto_planner(lmz, oracle_mod):
     """lmaze-v5 at 2^20 envs on its default CTA configuration: plannerStep with the device-side "waiting for the
     planner" mask + step + same-step auto-reset, both observation tensors."""
     N, B, LO, seed = 1 << 20, 1024, 700_001, 9
-    _need(N * (34300 + 19600 + 1296) + (4 << 30))
+    need_free(N * (34300 + 19600 + 1296) + (4 << 30))
     env = lmz.LmazeHierCuda(N, "v5", seed=seed, autoreset=True)
     ora = oracle_mod.OracleHier(B, seed=seed, env_id0=LO)
     fov = env.reset()
@@ -143,7 +121,7 @@ def test_v5_one_million_envs_auto_planner(lmz, oracle_mod):
     assert np.array_equal(u32(env.get_visit()[LO:LO + B]), u32(ora.export_visit()))
     # properties of every row: the fovealGoal plane (ch 3) is one 7x7 block; the free-cell crop (ch 0) shows the ball's
     # own cell; binary channels are binary; the visit crops (ch 2, 6) lie in [0, 1]; IndexError rows of loc are zero
-    allowed = torch.as_tensor(RC_BITS).cuda()
+    allowed = torch.as_tensor(REWARD_BITS.view(np.int32)).cuda()
     assert torch.isin(gr.view(torch.int32), allowed).all() and torch.isin(lr.view(torch.int32), allowed).all()
     CH = 1 << 14
     for lo in range(0, N, CH):

@@ -6,16 +6,7 @@ import os
 import numpy as np
 import pytest
 
-INVALID = 7
-
-
-def f64(bits):
-    return np.int64(bits).view(np.float64)
-
-
-def unpack(bits, shape):
-    n = int(np.prod(shape))
-    return np.unpackbits(bits)[:n].reshape(shape).astype(np.float32)
+from golden_io import Traces, f64, fov_image, loc_image, pack_v2_spawn, reward_f32_bits, unpack
 
 
 def test_layouts_match_reference(oracle_mod, golden_dir):
@@ -76,34 +67,31 @@ def test_v0_reset_semantics(oracle_mod, golden_dir):
 def test_traces(oracle_mod, golden_dir, variant_name):
     variant = oracle_mod.V0 if variant_name == "v0" else oracle_mod.V3
     shape = oracle_mod.OBS_SHAPE[variant]
-    z = np.load(os.path.join(golden_dir, variant_name + "_traces.npz"))
-    ne = int(z["n_envs"])
-    o = oracle_mod.OracleVec(variant, ne, autoreset=True)
-    sp0 = np.stack([z["e%d_spawn0" % e] for e in range(ne)])
+    tr = Traces(golden_dir, variant_name)
+    o = oracle_mod.OracleVec(variant, tr.n_envs, autoreset=True)
+    sp0 = tr.per_env("spawn0")
     if variant == oracle_mod.V0:
         sp0 = np.concatenate([sp0, -np.ones_like(sp0)], axis=1)
     o.reset(spawn=sp0)
-    T = len(z["e0_actions"])
-    for t in range(T):
-        acts = np.array([z["e%d_actions" % e][t] for e in range(ne)])
-        spawn = np.stack([z["e%d_spawn" % e][t] for e in range(ne)])
+    acts, spawns, dones_ref = tr.per_step("actions"), tr.per_step("spawn"), tr.per_step("done")
+    want_r, obs_bits = reward_f32_bits(tr.per_step("reward_bits")), tr.per_step("obs")
+    pos_ref, sc_ref = tr.per_step("pos"), tr.per_step("step_count")
+    for t in range(tr.T):
+        spawn = spawns[t]
         if variant == oracle_mod.V0:
             spawn = np.concatenate([spawn, -np.ones_like(spawn)], axis=1)
-        dones_ref = np.array([z["e%d_done" % e][t] for e in range(ne)])
-        spawn = np.where(dones_ref[:, None] > 0, spawn, 1)      # unused rows: any value
+        spawn = np.where(dones_ref[t][:, None] > 0, spawn, 1)      # unused rows: any value
         # pre-reset positions are checked through a non-resetting twin below; here: outputs
-        obs, rew, done = o.step(acts, spawn=spawn)
-        for e in range(ne):
-            ref_r = np.float32(f64(z["e%d_reward_bits" % e][t]))
-            assert rew[e].view(np.uint32) == ref_r.view(np.uint32), (t, e)
-            assert done[e] == dones_ref[e], (t, e)
-            assert np.array_equal(obs[e], unpack(z["e%d_obs" % e][t], shape)), (t, e)
-            if not done[e]:
-                pos = o.export()[0][e]
-                assert tuple(pos[:z["e%d_pos" % e].shape[1]]) == tuple(z["e%d_pos" % e][t]), (t, e)
-                assert o.export()[1][e] == z["e%d_step_count" % e][t]
-    assert o.stats[1] == sum(int(z["e%d_done" % e].sum()) for e in range(ne))
-    assert o.stats[1] >= 2 * ne       # every env finished at least two episodes
+        obs, rew, done = o.step(acts[t], spawn=spawn)
+        assert np.array_equal(rew.view(np.uint32), want_r[t]), t
+        assert np.array_equal(done, dones_ref[t]), t
+        assert np.array_equal(obs, unpack(obs_bits[t], shape)), t
+        pos, sc = o.export()[:2]
+        live = done == 0
+        assert np.array_equal(pos[live, :pos_ref.shape[2]], pos_ref[t][live]), t
+        assert np.array_equal(sc[live], sc_ref[t][live]), t
+    assert o.stats[1] == int(dones_ref.sum())
+    assert o.stats[1] >= 2 * tr.n_envs       # every env finished at least two episodes
 
 
 def test_v0_real_mt_trace(oracle_mod, golden_dir):
@@ -116,7 +104,7 @@ def test_v0_real_mt_trace(oracle_mod, golden_dir):
         sp = z["mt_spawn"][t]
         spawn = [[sp[0], sp[1], -1, -1]] if z["mt_done"][t] else [[1, 1, -1, -1]]
         _, rew, done = o.step([z["mt_actions"][t]], spawn=spawn, want_obs=False)
-        assert rew.view(np.uint32)[0] == np.float32(f64(z["mt_reward_bits"][t])).view(np.uint32)
+        assert rew.view(np.uint32)[0] == reward_f32_bits(z["mt_reward_bits"][t])
         assert done[0] == z["mt_done"][t]
         if not done[0]:
             assert tuple(o.export()[0][0][:2]) == tuple(z["mt_pos"][t])
@@ -237,29 +225,22 @@ def test_v2_transition_table(oracle_mod, golden_dir):
 
 
 def test_v2_traces(oracle_mod, golden_dir):
-    z = np.load(os.path.join(golden_dir, "v2_traces.npz"))
-    ne = int(z["n_envs"])
-    o = oracle_mod.OracleVec(oracle_mod.V2, ne, autoreset=True)
-    init = np.stack([z["e%d_init" % e] for e in range(ne)])        # bx, by, gx, gy, layout, layout-before
-    for e in range(ne):                                            # the maze the constructor rolled
+    tr = Traces(golden_dir, "v2")
+    o = oracle_mod.OracleVec(oracle_mod.V2, tr.n_envs, autoreset=True)
+    init = tr.per_env("init")                                      # bx, by, gx, gy, layout, layout-before
+    for e in range(tr.n_envs):                                     # the maze the constructor rolled
         oracle_mod.lib().lmzo_layout_v2(int(init[e, 5]), ctypes_grid(o, e))
-    sp = np.stack([init[:, 0], init[:, 1], init[:, 2], init[:, 3] | (init[:, 4] << 5)], axis=1)
-    obs = o.reset(spawn=sp)
-    for e in range(ne):
-        assert np.array_equal(obs[e], unpack(z["e%d_first_obs" % e], (5, 35, 35)))
-    T = len(z["e0_actions"])
-    for t in range(T):
-        acts = np.array([z["e%d_actions" % e][t] for e in range(ne)])
-        s5 = np.stack([z["e%d_spawn" % e][t] for e in range(ne)])
-        dref = np.array([z["e%d_done" % e][t] for e in range(ne)])
-        spawn = np.stack([s5[:, 0], s5[:, 1], s5[:, 2], s5[:, 3] | (s5[:, 4] << 5)], axis=1)
-        spawn = np.where(dref[:, None] > 0, spawn, 0)
-        obs, rew, done = o.step(acts, spawn=spawn)
-        for e in range(ne):
-            assert rew[e].view(np.uint32) == np.float32(f64(z["e%d_reward_bits" % e][t])).view(np.uint32), (t, e)
-            assert done[e] == dref[e], (t, e)
-            assert np.array_equal(obs[e], unpack(z["e%d_obs" % e][t], (5, 35, 35))), (t, e)
-    assert o.stats[1] == sum(int(z["e%d_done" % e].sum()) for e in range(ne)) >= 16
+    obs = o.reset(spawn=pack_v2_spawn(init))
+    assert np.array_equal(obs, unpack(tr.per_env("first_obs"), (5, 35, 35)))
+    acts, s5, dref = tr.per_step("actions"), tr.per_step("spawn"), tr.per_step("done")
+    want_r, obs_bits = reward_f32_bits(tr.per_step("reward_bits")), tr.per_step("obs")
+    for t in range(tr.T):
+        spawn = np.where(dref[t][:, None] > 0, pack_v2_spawn(s5[t]), 0)
+        obs, rew, done = o.step(acts[t], spawn=spawn)
+        assert np.array_equal(rew.view(np.uint32), want_r[t]), t
+        assert np.array_equal(done, dref[t]), t
+        assert np.array_equal(obs, unpack(obs_bits[t], (5, 35, 35))), t
+    assert o.stats[1] == int(dref.sum()) >= 16
 
 
 def ctypes_grid(o, i):
@@ -269,13 +250,6 @@ def ctypes_grid(o, i):
 
 
 # ---------------------------------------------------------------- v4 (v2 + float visit layer)
-def v4_obs(bits, visit):
-    """Rebuild the reference's (7,35,35) obs from the fixture's packed binary channels + 5x5 visit crops."""
-    b = np.unpackbits(bits)[:125].reshape(5, 5, 5).astype(np.float32)
-    small = np.stack([b[0], b[1], visit[0], b[2], b[3], b[4], visit[1]])
-    return np.repeat(np.repeat(small, 7, 1), 7, 2)
-
-
 def test_v4_transition_table(oracle_mod, golden_dir):
     z = np.load(os.path.join(golden_dir, "v4_table.npz"))
     o = oracle_mod.OracleVec(oracle_mod.V4, 1, autoreset=False)
@@ -288,79 +262,66 @@ def test_v4_transition_table(oracle_mod, golden_dir):
         assert tuple(pos[0]) == (nx, ny, gx, gy) and rw.view(np.int64)[0] == rb and dd == d and sc[0] == sa
         assert np.array_equal(o.export_visit()[0].view(np.uint32), z["post_visit"][k].view(np.uint32))   # bit-exact f32
         got = o.render_one(0)
-        assert np.array_equal(got.view(np.uint32), v4_obs(z["obs_bits"][k], z["obs_visit"][k]).view(np.uint32))
+        assert np.array_equal(got.view(np.uint32), fov_image(z["obs_bits"][k], z["obs_visit"][k]).view(np.uint32))
 
 
 def test_v4_traces(oracle_mod, golden_dir):
-    z = np.load(os.path.join(golden_dir, "v4_traces.npz"))
-    ne = int(z["n_envs"])
-    o = oracle_mod.OracleVec(oracle_mod.V4, ne, autoreset=True)
-    init = np.stack([z["e%d_init" % e] for e in range(ne)])        # bx, by, gx, gy, layout
-    obs = o.reset(spawn=np.stack([init[:, 0], init[:, 1], init[:, 2], init[:, 3] | (init[:, 4] << 5)], 1))
-    for e in range(ne):
-        assert np.array_equal(obs[e], v4_obs(z["e%d_first_bits" % e], z["e%d_first_visit" % e]))
-    T = len(z["e0_actions"])
-    for t in range(T):
-        acts = np.array([z["e%d_actions" % e][t] for e in range(ne)])
-        s5 = np.stack([z["e%d_spawn" % e][t] for e in range(ne)])
-        dref = np.array([z["e%d_done" % e][t] for e in range(ne)])
-        spawn = np.where(dref[:, None] > 0, np.stack([s5[:, 0], s5[:, 1], s5[:, 2], s5[:, 3] | (s5[:, 4] << 5)], 1), 0)
-        obs, rew, done = o.step(acts, spawn=spawn)
+    tr = Traces(golden_dir, "v4")
+    o = oracle_mod.OracleVec(oracle_mod.V4, tr.n_envs, autoreset=True)
+    obs = o.reset(spawn=pack_v2_spawn(tr.per_env("init")))          # bx, by, gx, gy, layout
+    assert np.array_equal(obs, fov_image(tr.per_env("first_bits"), tr.per_env("first_visit")))
+    acts, s5, dref = tr.per_step("actions"), tr.per_step("spawn"), tr.per_step("done")
+    want_r, visit_sum = reward_f32_bits(tr.per_step("reward_bits")), tr.per_step("visit_sum")
+    obs_bits, obs_visit = tr.per_step("obs_bits"), tr.per_step("obs_visit")
+    for t in range(tr.T):
+        spawn = np.where(dref[t][:, None] > 0, pack_v2_spawn(s5[t]), 0)
+        obs, rew, done = o.step(acts[t], spawn=spawn)
         vis = o.export_visit()
-        for e in range(ne):
-            assert rew[e].view(np.uint32) == np.float32(f64(z["e%d_reward_bits" % e][t])).view(np.uint32), (t, e)
-            assert done[e] == dref[e], (t, e)
-            want = v4_obs(z["e%d_obs_bits" % e][t], z["e%d_obs_visit" % e][t])
-            assert np.array_equal(obs[e].view(np.uint32), want.view(np.uint32)), (t, e)
-            assert float(vis[e].astype(np.float64).sum()) == z["e%d_visit_sum" % e][t]
-    for e in range(ne):
-        assert np.array_equal(vis[e].view(np.uint32), z["e%d_final_visit" % e].view(np.uint32))
+        assert np.array_equal(rew.view(np.uint32), want_r[t]), t
+        assert np.array_equal(done, dref[t]), t
+        assert np.array_equal(obs.view(np.uint32), fov_image(obs_bits[t], obs_visit[t]).view(np.uint32)), t
+        assert np.array_equal([float(v.astype(np.float64).sum()) for v in vis], visit_sum[t]), t
+    assert np.array_equal(vis.view(np.uint32), tr.per_env("final_visit").view(np.uint32))
 
 
 # ---------------------------------------------------------------- v5 / v6 (planner / actor protocol)
-def _loc_obs(bits):
-    small = np.unpackbits(bits)[:100].reshape(4, 5, 5).astype(np.float32)
-    return np.repeat(np.repeat(small, 7, 1), 7, 2)
-
-
 @pytest.mark.parametrize("variant", ["v5", "v6", "v5_edge"])
 def test_v5_traces(oracle_mod, golden_dir, variant):
     """Every value the reference returned from reset / plannerStep / step over 4 x ~730 events; "v5_edge": 21 scripted
     envs on the paths random traces never take (steps before any plannerStep, stepping on past globalDone, goal
     next to the ball, every planner cell, the 50-planner-step timeout) -- tests/golden/gen_golden_v5_edge.py."""
-    z = np.load(os.path.join(golden_dir, variant + "_traces.npz"))
+    tr = Traces(golden_dir, variant)
     n_events = 0
-    for e in range(int(z["n_envs"])):
+    for e in range(tr.n_envs):
         o = oracle_mod.OracleHier(1)
-        ev = z["e%d_events" % e]
-        for k, row in enumerate(ev):
+        z = tr.env(e)
+        for k, row in enumerate(z["events"]):
             kind, arg, grb, orb, gd, ld, bx, by = (int(v) for v in row[:8])
-            sp = row[8:13]
             if kind == 0:
-                fov = o.reset(spawn=[[sp[0], sp[1], sp[2], sp[3] | (sp[4] << 5)]])
-                assert np.array_equal(fov[0].view(np.uint32), v4_obs(z["e%d_fov_bits" % e][k], z["e%d_fov_visit" % e][k]).view(np.uint32)), (e, k)
+                fov = o.reset(spawn=[pack_v2_spawn(row[8:13])])
+                assert np.array_equal(fov[0].view(np.uint32), fov_image(z["fov_bits"][k], z["fov_visit"][k]).view(np.uint32)), (e, k)
             elif kind == 1:
                 loc, err = o.planner_step([arg])
-                assert not err[0] and np.array_equal(loc[0], _loc_obs(z["e%d_loc_bits" % e][k])), (e, k)
+                assert not err[0] and np.array_equal(loc[0], loc_image(z["loc_bits"][k])), (e, k)
             else:
                 fov, loc, gr, lr, gdo, ldo, err = o.step([arg])
                 assert not err[0]
-                assert gr.view(np.uint32)[0] == np.float32(f64(grb)).view(np.uint32), (e, k)
-                assert lr.view(np.uint32)[0] == np.float32(f64(orb)).view(np.uint32), (e, k)
+                assert gr.view(np.uint32)[0] == reward_f32_bits(grb), (e, k)
+                assert lr.view(np.uint32)[0] == reward_f32_bits(orb), (e, k)
                 assert (gdo[0], ldo[0]) == (gd, ld), (e, k)
-                assert np.array_equal(fov[0].view(np.uint32), v4_obs(z["e%d_fov_bits" % e][k], z["e%d_fov_visit" % e][k]).view(np.uint32)), (e, k)
-                assert np.array_equal(loc[0], _loc_obs(z["e%d_loc_bits" % e][k])), (e, k)
+                assert np.array_equal(fov[0].view(np.uint32), fov_image(z["fov_bits"][k], z["fov_visit"][k]).view(np.uint32)), (e, k)
+                assert np.array_equal(loc[0], loc_image(z["loc_bits"][k])), (e, k)
             st = o.export()[0]
             assert (st[0], st[1]) == (bx, by), (e, k)
-            assert float(o.export_visit()[0].astype(np.float64).sum()) == z["e%d_visit_sum" % e][k], (e, k)
+            assert float(o.export_visit()[0].astype(np.float64).sum()) == z["visit_sum"][k], (e, k)
             n_events += 1
     assert n_events > (400 if variant == "v5_edge" else 2500)
     if variant == "v6":       # safeFovealGoal(): re-draw until the window cell is not a wall (lmaze_env_v6.py:505-523)
         o = oracle_mod.OracleHier(1)
-        rows = [str(r) for r in z["safe_layout"]]
+        rows = [str(r) for r in tr["safe_layout"]]
         k = [i for i in range(1, 6) if oracle_mod.layout_v2(i) == rows][0]
-        draws, pos = z["safe_draws"], 0
-        for bx, by, want, used in z["safe_results"]:
+        draws, pos = tr["safe_draws"], 0
+        for bx, by, want, used in tr["safe_results"]:
             o.reset(spawn=[[4, 4, 8, 8 | (k << 5)]], want_obs=False)
             oracle_mod.lib().lmzo_env_force_v2(o._env(0), k, int(bx), int(by), 8, 8, int(bx), int(by), 0)
             got, n_used = o.safe_goal(0, draws[pos:pos + 40])
